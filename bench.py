@@ -1,15 +1,16 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the batched RendezvousEnv step/reset hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo's CUDA path
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this repo's CUDA path
     python bench.py --impl reference [--steps K] [--warmup W]    # the reference algorithm on the host cores
 
 Workload (BASELINE.json configs[1]): 65,536 envs per GPU, default constructor parameters, uniform random
 actions, auto-reset on, fp64 state.  A "step" is one env step of every env of the batch.  Prints ONE JSON line
 (rank 0).  Keys:
 
-  value / ms_per_step   device-resident loop: K steps as fused rollouts (rdv_rollout, --steps-per-launch steps per
-                        launch), fp64 U(-1,1) actions drawn on the device (Philox), CUDA events, max over ranks
+  value / ms_per_step   device-resident loop: exactly K timed steps as fused rollouts (rdv_rollout, --steps-per-launch
+                        steps per launch), fp64 U(-1,1) actions drawn on the device (Philox), CUDA events, max over
+                        ranks
   step_api              the same workload through the one-launch-per-step entry point (rdv_step) with fp64 actions
                         from a pre-generated 64-step device ring (201 MB, larger than L2)
   e2e                   same metric through RendezvousVecEnv.step(numpy actions): pinned H2D of the actions and
@@ -37,6 +38,8 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 ENVS_PER_GPU = 65536
+WARMUP_MIN = 1000
+LEAD_IN_LAUNCHES = 10
 RING = 64
 METRIC = "env-steps/sec"
 UNIT = "env-steps/s"
@@ -183,6 +186,28 @@ def cpu_baseline_leg(args):
     }
 
 
+def dump_outputs(out_dir, env, stats, limit=64 << 20):
+    """Write what the timed rollout hands its caller after its last step, so that two builds can be compared output
+    for output (the inputs are a function of the arguments alone): obs.npy (float32 [envs, 17], the observation the
+    last step returned), state.npy (float64 [envs, 20], the env state it left) and stats.npy (float64 [16], the
+    statistics of the timed steps summed over ranks, _native.STAT_NAMES order).  When the rows do not fit in `limit`
+    bytes, a fixed seeded sample of envs is written instead, their indices in env_index.npy (float64)."""
+    import numpy as np
+    from reinforcement_learning_rendezvous_b200 import _native as N
+    arrays = {"obs": env.obs.cpu().numpy(), "state": env.get_state().cpu().numpy()}
+    n = env.num_envs
+    per_env = sum(a.itemsize * a.shape[1] for a in arrays.values())
+    budget = limit - 8 * N.NSTATS - 4096                   # 4 KB for the .npy headers
+    if n * per_env > budget:
+        rows = np.sort(np.random.default_rng(0).choice(n, budget // (per_env + 8), replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["env_index"] = rows.astype(np.float64)
+    arrays["stats"] = stats.cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_cuda(args):
     import numpy as np
     rank = int(os.environ.get("RANK", "0"))
@@ -233,10 +258,9 @@ def run_cuda(args):
         return ms
 
     # ---------------- device-resident leg: fused rollouts, KL steps per launch, Philox actions ----------------
-    # One "repeat" = one K-step rollout (launches of at most KL steps) followed by the per-rollout statistics
-    # reduction.  The timed region holds R repeats, R chosen so that it lasts >= ~60 ms whatever --steps is; the
-    # all-reduce of rollout r (NCCL, N > 1) is issued asynchronously on a snapshot of the statistics and waited for
-    # after rollout r + 1 has been enqueued, and one SM is left free for it (RdvRolloutIO.sm_reserve).
+    # The timed region is exactly K steps: one K-step rollout (launches of at most KL steps).  The statistics
+    # all-reduce (NCCL, N > 1) is issued asynchronously on the rollout's statistics row at its end and waited for
+    # after the region, and one SM is left free for it (RdvRolloutIO.sm_reserve).
     KL = max(1, min(args.steps_per_launch, K))
     launches = [KL] * (K // KL) + ([K % KL] if K % KL else [])
     env = BatchedRendezvousEnv(n, device=dev, seed=args.seed, env_offset=rank * n, auto_reset=True,
@@ -244,61 +268,54 @@ def run_cuda(args):
     env.sm_reserve = 1 if world > 1 else 0
     env.reset()
     done_steps = 0
-    W_eff = max(W, 3)
+    # at least WARMUP_MIN warm-up steps: every episode of the batch starts at the reset above, and until their ends
+    # have spread out, the resets come in bursts (profiles/bench_short_region.md)
+    W_eff = max(W, WARMUP_MIN)
     env.rollout(W_eff, action_seed=args.seed + 1, step_base=0)
     done_steps = W_eff
     red = OverlappedStatsReducer(dev, capacity=4096)
-    # calibration (untimed; doubles as warm-up of the K-step launch shape and of every torch op and the collective
-    # the timed loop issues): how long is one repeat?
-    c0, c1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    for warm in range(2):
-        barrier()
-        c0.record()
-        for rr in range(2):
-            env.stats = red.begin()
-            for kl in launches:
-                env.rollout(kl, action_seed=args.seed + 1, step_base=done_steps)
-                done_steps += kl
-            red.end()
-        red.finish()
-        c1.record()
-        torch.cuda.synchronize()
+    # one untimed pass of the timed launches: warms the K-step launch shapes and every torch op and the collective
+    # the timed region issues
+    env.stats = red.begin()
+    for kl in launches:
+        env.rollout(kl, action_seed=args.seed + 1, step_base=done_steps)
+        done_steps += kl
+    red.end()
     red.reset()
-    t_rep = max_over_ranks(c0.elapsed_time(c1)) / 2
     n_l = len(launches)
-    R = max(1, math.ceil(args.min_region_ms / max(t_rep, 1e-3)), math.ceil(25 / n_l))
-    R = min(R, 4000)
-    if world > 1:                                          # every rank must run the same number of repeats
-        rt = torch.tensor([R], dtype=torch.int64, device=dev)
-        dist.all_reduce(rt, op=dist.ReduceOp.MAX)
-        R = int(rt[0])
     sampler = ClockSampler(local_rank).start() if rank == 0 else None
-    ev = [torch.cuda.Event(enable_timing=True) for _ in range(R * n_l + 1)]
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    # region start and end are the first and last of the per-launch events: one event record between two launches,
+    # as between any two timed launches (every record costs the stream a few microseconds)
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(n_l + 1)]
     barrier()
-    e0.record()
+    # untimed lead-in launches queued ahead of the region: the first timed launch then starts as a launch inside a
+    # long stream of them does, not after the host's launch latency (one lead-in launch is not enough: see
+    # profiles/bench_short_region.md)
+    env.stats = None
+    for _ in range(LEAD_IN_LAUNCHES):
+        env.rollout(KL, action_seed=args.seed + 1, step_base=done_steps)
+        done_steps += KL
     ev[0].record()
-    j = 0
-    for r in range(R):
-        env.stats = red.begin()
-        for kl in launches:
-            env.rollout(kl, action_seed=args.seed + 1, step_base=done_steps)
-            done_steps += kl
-            j += 1
-            ev[j].record()
-        red.end()          # issues this rollout's all-reduce (async, in place on its row); nothing waits for it here
+    first_timed_step = done_steps
+    env.stats = red.begin()
+    for j, kl in enumerate(launches):
+        env.rollout(kl, action_seed=args.seed + 1, step_base=done_steps)
+        done_steps += kl
+        ev[j + 1].record()
+    red.end()
     total_stats = red.finish()
-    e1.record()
     barrier()
-    ms = max_over_ranks(e0.elapsed_time(e1))
+    ms = max_over_ranks(ev[0].elapsed_time(ev[-1]))
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env, total_stats)
     stats = dict(zip(N.STAT_NAMES, total_stats.cpu().tolist()))
     total_steps = stats["steps"]
-    assert total_steps == world * n * K * R, (total_steps, world, n, K, R)
-    value = world * n * K * R / (ms * 1e-3)
+    assert total_steps == world * n * K, (total_steps, world, n, K)
+    value = world * n * K / (ms * 1e-3)
     rk_mean = stats["rk_accepted"] / (2.0 * max(total_steps, 1.0))
     # dominant kernel: rollout_kernel, per-launch durations of the full-size launches inside the timed region
-    full = [ev[q].elapsed_time(ev[q + 1]) for q in range(R * n_l) if launches[q % n_l] == KL]
+    full = [ev[q].elapsed_time(ev[q + 1]) for q in range(n_l) if launches[q] == KL]
     t_launch = sum(full) / len(full)
     t_step = t_launch / KL
     env.stats = torch.zeros(N.NSTATS, dtype=torch.float64, device=dev)
@@ -482,6 +499,7 @@ def run_cuda(args):
         venv.step(host_ring[k % RING])
     checksum = 0.0
     d2h_before = venv.d2h_bytes_total
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     t0 = time.perf_counter()
     e0.record()
@@ -518,18 +536,19 @@ def run_cuda(args):
         return 0
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
-        "ms_per_step": ms / (K * R), "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+        "ms_per_step": ms / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f64", "data": "synthetic",
         "config": {"workload": f"batched RendezvousEnv, {n:,} envs per GPU, random actions, fp64 step/reset "
                                "(BASELINE.json configs[1])",
                    "envs_per_gpu": n, "total_envs": world * n, "auto_reset": True, "integrator": args.integrator,
                    "actions": "fp64 U(-1,1) drawn on the device every step from the Philox4x32-10 stream "
                               "(action seed; global env id, step index)",
-                   "steps_per_launch": KL, "repeats": R, "steps_timed": K * R, "timed_region_ms": ms,
-                   "timing": "the timed region is `repeats` x (one `steps`-step rollout + its statistics reduction), "
-                             "sized to last >= %g ms whatever --steps is" % args.min_region_ms,
+                   "steps_per_launch": KL, "steps_timed": K, "timed_region_ms": ms,
+                   "warmup_steps": W_eff, "first_timed_step": first_timed_step,
+                   "timing": "the timed region is one `steps`-step rollout, queued behind %d untimed launches"
+                             % LEAD_IN_LAUNCHES,
                    "stats_all_reduce": ("one 16-double NCCL all-reduce per rollout, issued asynchronously in place on the "
-                                        "rollout's own statistics row and waited for once at the end of the region; "
+                                        "rollout's own statistics row at the end of the region and waited for after it; "
                                         "the rollout leaves 1 SM free for it" if world > 1 else "no-op at N = 1"),
                    "l2": "state lives in registers for the steps of a launch and is re-read from memory once per "
                          "launch; ms_per_step_l2_flushed repeats the launches with a 256 MB L2 flush before each; "
@@ -539,7 +558,7 @@ def run_cuda(args):
                    "ms_per_step_no_auto_reset": ms_no_reset,
                    "parallelism": f"{world} x independent env shards, no data-path collective; one "
                                   "16-double statistics all-reduce per rollout"},
-        "clocks": clocks, "e2e": e2e, "gpu_launches": R * len(launches),
+        "clocks": clocks, "e2e": e2e, "gpu_launches": n_l,
         "roofline": roofline, "cpu_baseline": cpu_baseline, "step_api": step_api,
         "policy_rollout": policy_rollout, "policy_rollout_1m": policy_rollout_1m,
         "episode_stats": {"episodes": stats["episodes"], "mean_length": stats["length_sum"] / max(stats["episodes"], 1),
@@ -569,7 +588,10 @@ def main():
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--integrator", choices=("rk45", "closed_form"), default="rk45")
     ap.add_argument("--e2e-steps", type=int, default=1000)
-    ap.add_argument("--min-region-ms", type=float, default=80.0, help="minimum length of a timed region")
+    ap.add_argument("--min-region-ms", type=float, default=80.0,
+                    help="minimum length of a timed region of the policy_rollout legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what they computed as DIR/<name>.npy (see dump_outputs)")
     ap.add_argument("--ref-min-seconds", type=float, default=8.0, help="time floor of the reference arm")
     ap.add_argument("--steps-per-launch", type=int, default=250, help="env steps fused into one rollout launch")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)

@@ -306,3 +306,29 @@ def test_bench_cpu_baseline_leg_runs_in_a_child():
     c = json.loads(lines[0])
     assert c["kind"] == "port" and c["cores"] >= 1 and c["value"] > 0 and c["unit"] == "env-steps/s"
     assert "sample" in c and c["single_process_value"] > 0 and c["c_port_value"] > 0
+
+
+def test_bench_dump_outputs_samples_within_the_limit(tmp_path):
+    """bench.py --dump-outputs: rows that do not fit the size limit are replaced by a fixed seeded sample of envs,
+    the same one on every run, with the arrays kept in float32 / float64."""
+    import types
+    import torch
+    import bench
+    n = 5000
+    obs, state = torch.rand(n, 17), torch.rand(n, 20, dtype=torch.float64)
+    env = types.SimpleNamespace(num_envs=n, obs=obs, get_state=lambda: state)
+    stats = torch.arange(16, dtype=torch.float64)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), env, stats, limit=300_000)
+        assert sum(os.path.getsize(tmp_path / d / f) for f in os.listdir(tmp_path / d)) <= 300_000
+    got = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in ("obs", "state", "stats", "env_index")}
+    idx = got["env_index"]
+    assert got["env_index"].dtype == np.float64 and 0 < len(idx) < n and np.all(np.diff(idx) > 0)
+    np.testing.assert_array_equal(idx, np.load(tmp_path / "b" / "env_index.npy"))
+    rows = idx.astype(np.int64)
+    np.testing.assert_array_equal(got["obs"], obs.numpy()[rows])
+    np.testing.assert_array_equal(got["state"], state.numpy()[rows])
+    np.testing.assert_array_equal(got["stats"], stats.numpy())
+    bench.dump_outputs(str(tmp_path / "c"), env, stats)             # fits the default 64 MB: every env, no index
+    assert sorted(os.listdir(tmp_path / "c")) == ["obs.npy", "state.npy", "stats.npy"]
+    np.testing.assert_array_equal(np.load(tmp_path / "c" / "obs.npy"), obs.numpy())
