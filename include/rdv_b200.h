@@ -294,7 +294,8 @@ int rdv_tune(int key, int value);
 
 /* Test hook: y[i] = f(x[i]) for the device math helpers the step is built from.  op 0: 1/sqrt(x), 1: 1/x,
  * 2: sqrt(x), 3: x^-0.1 (fp64 controller), 4: x^-0.1 (float32 controller), 5: acos(round(x, 5))
- * (angle_between_vectors, utils/general.py:163-181). */
+ * (angle_between_vectors, utils/general.py:163-181); at x = s^2 > 0, one attempted step of the plane attitude solver:
+ * 6-9: P, Q, R, I of rdv_plane_poly.h, 10-13: the same four from the stagewise attempt. */
 int rdv_math_probe(const double *x, double *y, int64_t n, int op, void *cuda_stream);
 
 /* Measured-peak helper for the roofline: runs `iters` dependent-chain-free DFMA per thread on

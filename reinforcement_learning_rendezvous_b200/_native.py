@@ -25,7 +25,7 @@ LIB_PATH = os.environ.get("RDV_B200_LIB") or os.path.join(CSRC_DIR, "librdv_b200
 HOST_SRC = os.path.join(CSRC_DIR, "rdv_host.c")                 # CPython helper of RendezvousVecEnv (gcc, no CUDA)
 HOST_LIB = os.path.join(PKG_DIR, "_rdv_host" + (sysconfig.get_config_var("EXT_SUFFIX") or ".so"))
 SOURCES = ("rdv_b200.cu",)
-HEADERS = ("rdv_math.cuh", "rdv_env.cuh", "rdv_step.cuh", "rdv_policy.cuh", "rdv_policy_tc.cuh")
+HEADERS = ("rdv_math.cuh", "rdv_plane_poly.h", "rdv_env.cuh", "rdv_step.cuh", "rdv_policy.cuh", "rdv_policy_tc.cuh")
 
 ABI_VERSION = 15
 OBS_DIM, ACT_DIM, N_UNIFORMS = 17, 6, 24

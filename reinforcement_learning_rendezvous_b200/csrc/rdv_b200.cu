@@ -1187,7 +1187,22 @@ __global__ void math_probe_kernel(const double *x, double *y, int64_t n, int op)
         case 2: r = fast_sqrt(v); break;
         case 3: r = pow_neg_tenth(v); break;
         case 4: r = (double)pow_neg_tenth_f32((float)v); break;
-        default: r = rounded_angle_from(v, 1.0, 1.0); break;      // acos(round(v, 5))
+        case 5: r = rounded_angle_from(v, 1.0, 1.0); break;       // acos(round(v, 5))
+        default: {
+            // the attempted plane step at x = v = s^2 > 0: P, Q, R, I of rdv_plane_poly.h (ops 6-9), and the same
+            // four quantities from the stagewise attempt at (a, b, g, om2, h) = (1, 0, 1, 1, sqrt(x)) (ops 10-13)
+            double P, Q, R, I;
+            if (op < 10) {
+                plane_poly(v, P, Q, R, I);
+            } else {
+                const double h = sqrt(v);
+                plane_attempt<false>(1.0, 0.0, 1.0, 1.0, h, P, Q, R, I);
+                Q /= h; R /= v * v * v; I /= h * v * v;
+            }
+            const int k = (op - 6) & 3;
+            r = k == 0 ? P : k == 1 ? Q : k == 2 ? R : I;
+            break;
+        }
     }
     y[i] = r;
 }
@@ -1711,7 +1726,7 @@ int rdv_policy_forward_ffma(const RdvPolicy *pi, const float *obs, float *action
 int rdv_math_probe(const double *x, double *y, int64_t n, int op, void *cuda_stream)
 {
     if (!x || !y) return RDV_ERR_NULL;
-    if (n < 0 || op < 0 || op > 5) return RDV_ERR_SIZE;
+    if (n < 0 || op < 0 || op > 13) return RDV_ERR_SIZE;
     if (n == 0) return RDV_OK;
     if (!ensure_tables((cudaStream_t)cuda_stream)) return RDV_ERR_CUDA;
     math_probe_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)cuda_stream>>>(x, y, n, op);

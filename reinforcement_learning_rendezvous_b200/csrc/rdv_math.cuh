@@ -12,6 +12,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "rdv_b200.h"
+#include "rdv_plane_poly.h"
 
 #define RDV_DEV __device__ __forceinline__
 
@@ -567,6 +568,110 @@ RDV_DEV void rhs_plane(const double a, const double b, const double om2, double 
     ka = -(t * g);
     kb = a * g;
 }
+// g = |q0| / |y| at y = a q0 + b p, formed exactly as inside rhs_plane: a point carries g instead of its slope, which is
+// (-(om2 b) g, a g) bit for bit.
+RDV_DEV double plane_g(const double a, const double b, const double om2) { return fast_rsqrt(fma(om2 * b, b, a * a)); }
+
+// ---------------------------------------------------------------------------------
+// One attempted step in closed form (RDV_PLANE_POLY).
+//
+// With z = a + i w b, w^2 = om2, the plane equation is z' = i w z / |z|: rotation-equivariant and homogeneous of
+// degree 0.  Every stage of one Dormand-Prince attempt from z with step h is therefore z times a function of
+// s = h w / |z| alone, and so are the 5th-order point and the error estimate:  z_new = z S(s), (K^T E) h = z E(s).
+// S and E satisfy f(-s) = conj f(s); with x = s^2 = h^2 om2 g^2 (g = 1 / |z|)
+//
+//     Re S = 1 + x P1(x),   Im S = s (1 + x Q1(x)),   Re E = x^3 R(x),   Im E = s x^2 I(x),
+//
+// polynomials fitted at 50 digits by tools/gen_plane_poly.py (rdv_plane_poly.h; 6-7 coefficients each on
+// x <= X_MAX = 1/32, P and Q to < 0.01 ulp, R and I to < 1e-14).  Back in plane coordinates, with u = h g a and
+// v = h g om2 b (no division by w; w = 0 gives x = 0, P = 1 and a_new = a exactly):
+//
+//     a_new = a P - v Q,   b_new = b P + u Q,   ea = a x^3 R - v x^2 I,   eb = b x^3 R + u x^2 I.
+//
+// That is ~40 fp64 operations and no MUFU per attempt against ~130 operations and 7 RSQ for the six slopes of the
+// stagewise form, and the critical path is one Horner chain instead of six dependent slope chains.  The results
+// agree with the stagewise attempt to its rounding (~1e-16 on the state; the stagewise error estimate carries
+// ~1e-16 h of cancellation noise that the polynomial does not).
+//
+// Where it applies: h <= dt and g = 1 at the start of a solve, and |z| moves by at most DRIFT_PER_S s per accepted
+// step (4e-10 s), i.e. by < 1e-10 over a whole solve (sum of s <= sqrt(om2) dt).  So om2 dt^2 (1 + 2^-20) <= X_MAX
+// keeps every attempt of the solve inside the fitted range; the 2^-20 also covers the rounding of om2 and x.  Faster
+// spins (om2 dt^2 > X_MAX ~ |w| dt > 0.35 rad) take the stagewise attempt for the whole solve, out of line.
+// ---------------------------------------------------------------------------------
+#ifndef RDV_PLANE_POLY
+#define RDV_PLANE_POLY 1         /* measured (B200): 9.72 -> 9.30 us per step (20-step launches), 8.86 -> 8.65 (250-step) */
+#endif
+constexpr int PP_P1 = 0, PP_Q1 = PP_P1 + RDV_PP_N_P1, PP_R = PP_Q1 + RDV_PP_N_Q1, PP_I = PP_R + RDV_PP_N_R;
+__constant__ double c_pp[PP_I + RDV_PP_N_I] = {RDV_PP_P1, RDV_PP_Q1, RDV_PP_R, RDV_PP_I};
+
+template <int OFF, int N>
+RDV_DEV double pp_horner(const double x)
+{
+    double r = c_pp[OFF + N - 1];
+#pragma unroll
+    for (int k = N - 2; k >= 0; --k) r = fma(r, x, c_pp[OFF + k]);
+    return r;
+}
+// Re S, Im S / s, Re E / x^3, Im E / (s x^2) at x = s^2
+RDV_DEV void plane_poly(const double x, double &P, double &Q, double &R, double &I)
+{
+    P = fma(x, pp_horner<PP_P1, RDV_PP_N_P1>(x), 1.0);
+    Q = fma(x, pp_horner<PP_Q1, RDV_PP_N_Q1>(x), 1.0);
+    R = pp_horner<PP_R, RDV_PP_N_R>(x);
+    I = pp_horner<PP_I, RDV_PP_N_I>(x);
+}
+// whether every attempt of the solve from y over dt stays inside the polynomials' range (see above); false for a
+// non-finite rate.  0.25 |w|^2 / |q0|^2 is om2 of plane_basis to a few ulp.
+RDV_DEV bool plane_poly_covers(const double (&y)[7], const double dt)
+{
+    const double w2 = fma(y[6], y[6], fma(y[5], y[5], y[4] * y[4]));
+    const double q2 = fma(y[3], y[3], fma(y[2], y[2], fma(y[1], y[1], y[0] * y[0])));
+    return 0.25 * w2 * (dt * dt) <= (RDV_PP_X_MAX * (1.0 - 0x1p-20)) * q2;
+}
+
+// One attempted step of rk_step (scipy rk.py:14-69) in plane coordinates from y = a q0 + b p (g = |q0| / |y|) with
+// step h: the candidate (a_new, b_new) and the error estimate (K^T E) h = ea q0 + eb p.  POLY: the closed form above;
+// otherwise the six stages and the slope at the new point, the first slope (FSAL) rebuilt from g bit for bit.  Both
+// solvers and every launch shape call this one function, so they give identical bits.
+template <bool POLY>
+RDV_DEV void plane_attempt(const double a, const double b, const double g, const double om2, const double h,
+                           double &a_new, double &b_new, double &ea, double &eb)
+{
+    if (POLY) {
+        const double hg = h * g, t = hg * om2;
+        const double u = hg * a, v = t * b, x = t * hg;
+        double P, Q, R, I;
+        plane_poly(x, P, Q, R, I);
+        a_new = fma(a, P, -(v * Q));
+        b_new = fma(b, P, u * Q);
+        const double x2 = x * x, xr = x * R;
+        ea = x2 * fma(a, xr, -(v * I));
+        eb = x2 * fma(b, xr, u * I);
+    } else {
+        double ka[7], kb[7], as, bs;
+        ka[0] = -((om2 * b) * g); kb[0] = a * g;
+        as = fma(ka[0] * RK_A21, h, a);
+        bs = fma(kb[0] * RK_A21, h, b);
+        rhs_plane(as, bs, om2, ka[1], kb[1]);
+        as = fma(fma(ka[1], RK_A32, ka[0] * RK_A31), h, a);
+        bs = fma(fma(kb[1], RK_A32, kb[0] * RK_A31), h, b);
+        rhs_plane(as, bs, om2, ka[2], kb[2]);
+        as = fma(fma(ka[2], RK_A43, fma(ka[1], RK_A42, ka[0] * RK_A41)), h, a);
+        bs = fma(fma(kb[2], RK_A43, fma(kb[1], RK_A42, kb[0] * RK_A41)), h, b);
+        rhs_plane(as, bs, om2, ka[3], kb[3]);
+        as = fma(fma(ka[3], RK_A54, fma(ka[2], RK_A53, fma(ka[1], RK_A52, ka[0] * RK_A51))), h, a);
+        bs = fma(fma(kb[3], RK_A54, fma(kb[2], RK_A53, fma(kb[1], RK_A52, kb[0] * RK_A51))), h, b);
+        rhs_plane(as, bs, om2, ka[4], kb[4]);
+        as = fma(fma(ka[4], RK_A65, fma(ka[3], RK_A64, fma(ka[2], RK_A63, fma(ka[1], RK_A62, ka[0] * RK_A61)))), h, a);
+        bs = fma(fma(kb[4], RK_A65, fma(kb[3], RK_A64, fma(kb[2], RK_A63, fma(kb[1], RK_A62, kb[0] * RK_A61)))), h, b);
+        rhs_plane(as, bs, om2, ka[5], kb[5]);
+        a_new = fma(h, fma(ka[5], RK_B6, fma(ka[4], RK_B5, fma(ka[3], RK_B4, fma(ka[2], RK_B3, ka[0] * RK_B1)))), a);
+        b_new = fma(h, fma(kb[5], RK_B6, fma(kb[4], RK_B5, fma(kb[3], RK_B4, fma(kb[2], RK_B3, kb[0] * RK_B1)))), b);
+        rhs_plane(a_new, b_new, om2, ka[6], kb[6]);
+        ea = h * fma(ka[6], RK_E7, fma(ka[5], RK_E6, fma(ka[4], RK_E5, fma(ka[3], RK_E4, fma(ka[2], RK_E3, ka[0] * RK_E1)))));
+        eb = h * fma(kb[6], RK_E7, fma(kb[5], RK_E6, fma(kb[4], RK_E5, fma(kb[3], RK_E4, fma(kb[2], RK_E3, kb[0] * RK_E1)))));
+    }
+}
 
 // What the controller sees of one attempted step, in float32 (RDV_CTRL_F32 rationale above): the candidate state
 // y_new = a_new q0 + b_new p and the error estimate e = ea q0 + eb p in quaternion components, and
@@ -746,9 +851,10 @@ RDV_DEV void plane_basis(const double (&y)[7], double (&q0)[4], double (&p)[4], 
     om2 = fma(hw[2], hw[2], fma(hw[1], hw[1], hw[0] * hw[0]));
 }
 
-// One point of the solution in plane coordinates, with what the next step needs from it: the slope (FSAL) and the
-// float32 quaternion components the controller's scale vector uses.
-struct PlanePoint { double a, b, ka, kb, t; float yf[4]; };
+// One point of the solution in plane coordinates, with what the next step needs from it: g = |q0| / |y| (which also
+// gives the FSAL slope of the stagewise attempt) and the float32 quaternion components the controller's scale vector
+// uses.
+struct PlanePoint { double a, b, g, t; float yf[4]; };
 
 // One solver.step() of scipy's RungeKutta._step_impl (rk.py:111-179): attempts from `s` until one is accepted; the
 // accepted point goes to `n` (`s` is left untouched, so the caller alternates two points and no copy is made).
@@ -784,6 +890,7 @@ struct PlanePoint { double a, b, ka, kb, t; float yf[4]; };
 #ifndef RDV_LAST_SHORTCUT
 #define RDV_LAST_SHORTCUT 1     /* measured: 9.76 -> 9.74 us per step (20-step launches), 8.94 -> 8.91 (250-step) */
 #endif
+template <bool POLY>
 RDV_DEV int plane_step(const PlanePoint &s, PlanePoint &n, double &h_abs, int &n_rejected, const double om2, const double dt,
                         const double (&q0)[4], const double (&p)[4], const float (&q0f)[4], const float (&pf)[4])
 {
@@ -813,32 +920,9 @@ RDV_DEV int plane_step(const PlanePoint &s, PlanePoint &n, double &h_abs, int &n
 #endif
         const double h = t_new - t;
         h_abs = fabs(h);
-        // ---- rk_step: six stages, FSAL row ----
-        double ka[7], kb[7], as, bs;
-        ka[0] = s.ka; kb[0] = s.kb;
-        as = fma(ka[0] * RK_A21, h, a);
-        bs = fma(kb[0] * RK_A21, h, b);
-        rhs_plane(as, bs, om2, ka[1], kb[1]);
-        as = fma(fma(ka[1], RK_A32, ka[0] * RK_A31), h, a);
-        bs = fma(fma(kb[1], RK_A32, kb[0] * RK_A31), h, b);
-        rhs_plane(as, bs, om2, ka[2], kb[2]);
-        as = fma(fma(ka[2], RK_A43, fma(ka[1], RK_A42, ka[0] * RK_A41)), h, a);
-        bs = fma(fma(kb[2], RK_A43, fma(kb[1], RK_A42, kb[0] * RK_A41)), h, b);
-        rhs_plane(as, bs, om2, ka[3], kb[3]);
-        as = fma(fma(ka[3], RK_A54, fma(ka[2], RK_A53, fma(ka[1], RK_A52, ka[0] * RK_A51))), h, a);
-        bs = fma(fma(kb[3], RK_A54, fma(kb[2], RK_A53, fma(kb[1], RK_A52, kb[0] * RK_A51))), h, b);
-        rhs_plane(as, bs, om2, ka[4], kb[4]);
-        as = fma(fma(ka[4], RK_A65, fma(ka[3], RK_A64, fma(ka[2], RK_A63, fma(ka[1], RK_A62, ka[0] * RK_A61)))), h, a);
-        bs = fma(fma(kb[4], RK_A65, fma(kb[3], RK_A64, fma(kb[2], RK_A63, fma(kb[1], RK_A62, kb[0] * RK_A61)))), h, b);
-        rhs_plane(as, bs, om2, ka[5], kb[5]);
-        const double a_new = fma(h, fma(ka[5], RK_B6, fma(ka[4], RK_B5, fma(ka[3], RK_B4, fma(ka[2], RK_B3, ka[0] * RK_B1)))), a);
-        const double b_new = fma(h, fma(kb[5], RK_B6, fma(kb[4], RK_B5, fma(kb[3], RK_B4, fma(kb[2], RK_B3, kb[0] * RK_B1)))), b);
-        rhs_plane(a_new, b_new, om2, ka[6], kb[6]);
-        // ---- error estimate (K^T E) h in the plane; the controller's norm in quaternion components ----
-        const double ea = h * fma(ka[6], RK_E7, fma(ka[5], RK_E6, fma(ka[4], RK_E5, fma(ka[3], RK_E4,
-                              fma(ka[2], RK_E3, ka[0] * RK_E1)))));
-        const double eb = h * fma(kb[6], RK_E7, fma(kb[5], RK_E6, fma(kb[4], RK_E5, fma(kb[3], RK_E4,
-                              fma(kb[2], RK_E3, kb[0] * RK_E1)))));
+        // ---- rk_step and the error estimate (K^T E) h in the plane; the controller's norm in quaternion components ----
+        double a_new, b_new, ea, eb;
+        plane_attempt<POLY>(a, b, s.g, om2, h, a_new, b_new, ea, eb);
 #if RDV_LAST_SHORTCUT
         if (last) {
             const float eaf = (float)ea, ebf = (float)eb;
@@ -847,7 +931,7 @@ RDV_DEV int plane_step(const PlanePoint &s, PlanePoint &n, double &h_abs, int &n
             for (int i = 0; i < 4; ++i) { nq = fmaf(q0f[i], q0f[i], nq); np = fmaf(pf[i], pf[i], np); }
             const float ub = fmaf(eaf * eaf, nq, ebf * ebf * np) * (2.0f / 7.0f * 1.0e12f);   // atol^-2 = 1e12
             if (ub < 0.99f) {
-                n.a = a_new; n.b = b_new; n.ka = ka[6]; n.kb = kb[6]; n.t = t_new;
+                n.a = a_new; n.b = b_new; n.t = t_new;          // the solve ends here: g is not needed
                 return 2;
             }
         }
@@ -873,7 +957,7 @@ RDV_DEV int plane_step(const PlanePoint &s, PlanePoint &n, double &h_abs, int &n
             float factor = fminf(10.0f, pw);
             if (rejected) factor = fminf(1.0f, factor);
             h_abs *= (double)factor;
-            n.a = a_new; n.b = b_new; n.ka = ka[6]; n.kb = kb[6]; n.t = t_new;
+            n.a = a_new; n.b = b_new; n.g = plane_g(a_new, b_new, om2); n.t = t_new;
 #if RDV_LAST_FLAG || RDV_LAST_SHORTCUT
             return last ? 2 : 1;
 #else
@@ -905,7 +989,8 @@ RDV_DEV int plane_step(const PlanePoint &s, PlanePoint &n, double &h_abs, int &n
 #else
 #define RDV_KEEP_F32(x)
 #endif
-RDV_RK_FN int rk45_iso_plane(double (&y)[7], const double dt, int &n_rejected)
+template <bool POLY>
+RDV_DEV int rk45_iso_plane_solve(double (&y)[7], const double dt, int &n_rejected)
 {
     double q0[4], p[4], om2;
     plane_basis(y, q0, p, om2);
@@ -917,22 +1002,22 @@ RDV_RK_FN int rk45_iso_plane(double (&y)[7], const double dt, int &n_rejected)
         RDV_KEEP_F32(q0f[i]); RDV_KEEP_F32(pf[i]);
         X.yf[i] = q0f[i];
     }
-    X.a = 1.0; X.b = 0.0; X.ka = 0.0; X.kb = 1.0; X.t = 0.0;     // y = a q0 + b p; slope there = p
+    X.a = 1.0; X.b = 0.0; X.g = 1.0; X.t = 0.0;                 // y = a q0 + b p; slope there = p
     double h_abs = plane_initial_step(y, q0f, pf, om2, dt);
     int accepted = 0;
 #if RDV_RK_PINGPONG
     // two copies of the step that read one point and write the other: the accepted candidate is never copied
     for (;;) {
-        if (!plane_step(X, Y, h_abs, n_rejected, om2, dt, q0, p, q0f, pf)) return -1;
+        if (!plane_step<POLY>(X, Y, h_abs, n_rejected, om2, dt, q0, p, q0f, pf)) return -1;
         ++accepted;
         if (Y.t - dt >= 0.0) { X.a = Y.a; X.b = Y.b; break; }
-        if (!plane_step(Y, X, h_abs, n_rejected, om2, dt, q0, p, q0f, pf)) return -1;
+        if (!plane_step<POLY>(Y, X, h_abs, n_rejected, om2, dt, q0, p, q0f, pf)) return -1;
         ++accepted;
         if (X.t - dt >= 0.0) break;
     }
 #else
     for (;;) {
-        const int r = plane_step(X, Y, h_abs, n_rejected, om2, dt, q0, p, q0f, pf);
+        const int r = plane_step<POLY>(X, Y, h_abs, n_rejected, om2, dt, q0, p, q0f, pf);
         if (!r) return -1;
         ++accepted;
         X = Y;
@@ -947,6 +1032,20 @@ RDV_RK_FN int rk45_iso_plane(double (&y)[7], const double dt, int &n_rejected)
     for (int i = 0; i < 4; ++i) y[i] = fma(X.b, p[i], X.a * q0[i]);
     return accepted;
 }
+// the stagewise solve for rates outside the polynomials' range, out of line: the hot loop holds one form only
+__device__ __noinline__ int rk45_iso_plane_stagewise(double (&y)[7], const double dt, int &n_rejected)
+{
+    return rk45_iso_plane_solve<false>(y, dt, n_rejected);
+}
+RDV_RK_FN int rk45_iso_plane(double (&y)[7], const double dt, int &n_rejected)
+{
+#if RDV_PLANE_POLY
+    if (!plane_poly_covers(y, dt)) return rk45_iso_plane_stagewise(y, dt, n_rejected);
+    return rk45_iso_plane_solve<true>(y, dt, n_rejected);
+#else
+    return rk45_iso_plane_solve<false>(y, dt, n_rejected);
+#endif
+}
 
 // Lock-step form of rk45_iso_plane for TWO bodies in one thread (chaser and target of one env): the control flow of
 // scipy's _step_impl (accept / reject, the factor clamps, the rejected-step rule, TOO_SMALL_STEP) is written as
@@ -954,9 +1053,10 @@ RDV_RK_FN int rk45_iso_plane(double (&y)[7], const double dt, int &n_rejected)
 // the two bodies are interleaved stage by stage in the source, so that two independent slope chains (norm ->
 // rsqrt -> scale) sit next to each other in every basic block.  Arithmetic per body is that of rk45_iso_plane,
 // operation for operation (tests/test_gpu_rollout.py compares the bits).
-RDV_DEV int rk45_iso_plane_pair(double (&ya)[7], double (&yb)[7], const double dt, int &n_rejected)
+template <bool POLY>
+RDV_DEV int rk45_iso_plane_pair_solve(double (&ya)[7], double (&yb)[7], const double dt, int &n_rejected)
 {
-    double q0[2][4], p[2][4], om2[2], a[2], b[2], ka0[2], kb0[2], h_abs[2], t[2];
+    double q0[2][4], p[2][4], om2[2], a[2], b[2], g[2], h_abs[2], t[2];
     float q0f[2][4], pf[2][4], ycf[2][4];
     int accepted[2] = {0, 0};
     bool done[2] = {false, false}, rejected[2] = {false, false}, failed[2] = {false, false};
@@ -964,7 +1064,7 @@ RDV_DEV int rk45_iso_plane_pair(double (&ya)[7], double (&yb)[7], const double d
     plane_basis(yb, q0[1], p[1], om2[1]);
 #pragma unroll
     for (int c = 0; c < 2; ++c) {
-        a[c] = 1.0; b[c] = 0.0; ka0[c] = 0.0; kb0[c] = 1.0;
+        a[c] = 1.0; b[c] = 0.0; g[c] = 1.0;
 #pragma unroll
         for (int i = 0; i < 4; ++i) { q0f[c][i] = (float)q0[c][i]; pf[c][i] = (float)p[c][i]; ycf[c][i] = q0f[c][i]; }
     }
@@ -973,9 +1073,8 @@ RDV_DEV int rk45_iso_plane_pair(double (&ya)[7], double (&yb)[7], const double d
     t[0] = t[1] = 0.0;
     // ---- attempted steps, both bodies per pass, predicated commit ----
     while (!((done[0] || failed[0]) && (done[1] || failed[1]))) {
-        double h[2], t_new[2], ha[2], as[2], bs[2];
+        double h[2], t_new[2], ha[2], as[2], bs[2], ea[2], eb[2];
         bool fail_now[2];
-        double ka1[2], kb1[2], ka2[2], kb2[2], ka3[2], kb3[2], ka4[2], kb4[2], ka5[2], kb5[2], ka6[2], kb6[2];
 #pragma unroll
         for (int c = 0; c < 2; ++c) {
             const double min_step = 10.0 * (__longlong_as_double(__double_as_longlong(t[c]) + 1) - t[c]);
@@ -986,42 +1085,18 @@ RDV_DEV int rk45_iso_plane_pair(double (&ya)[7], double (&yb)[7], const double d
             h[c] = t_new[c] - t[c];
             ha[c] = fabs(h[c]);
         }
-#define RDV_PSTAGE(KA, KB, EA, EB)                                                       \
-        _Pragma("unroll") for (int c = 0; c < 2; ++c) { as[c] = (EA); bs[c] = (EB); }    \
-        _Pragma("unroll") for (int c = 0; c < 2; ++c) rhs_plane(as[c], bs[c], om2[c], KA[c], KB[c]);
-        RDV_PSTAGE(ka1, kb1, fma(ka0[c] * RK_A21, h[c], a[c]), fma(kb0[c] * RK_A21, h[c], b[c]))
-        RDV_PSTAGE(ka2, kb2, fma(fma(ka1[c], RK_A32, ka0[c] * RK_A31), h[c], a[c]),
-                   fma(fma(kb1[c], RK_A32, kb0[c] * RK_A31), h[c], b[c]))
-        RDV_PSTAGE(ka3, kb3, fma(fma(ka2[c], RK_A43, fma(ka1[c], RK_A42, ka0[c] * RK_A41)), h[c], a[c]),
-                   fma(fma(kb2[c], RK_A43, fma(kb1[c], RK_A42, kb0[c] * RK_A41)), h[c], b[c]))
-        RDV_PSTAGE(ka4, kb4,
-                   fma(fma(ka3[c], RK_A54, fma(ka2[c], RK_A53, fma(ka1[c], RK_A52, ka0[c] * RK_A51))), h[c], a[c]),
-                   fma(fma(kb3[c], RK_A54, fma(kb2[c], RK_A53, fma(kb1[c], RK_A52, kb0[c] * RK_A51))), h[c], b[c]))
-        RDV_PSTAGE(ka5, kb5,
-                   fma(fma(ka4[c], RK_A65, fma(ka3[c], RK_A64, fma(ka2[c], RK_A63, fma(ka1[c], RK_A62, ka0[c] * RK_A61)))),
-                       h[c], a[c]),
-                   fma(fma(kb4[c], RK_A65, fma(kb3[c], RK_A64, fma(kb2[c], RK_A63, fma(kb1[c], RK_A62, kb0[c] * RK_A61)))),
-                       h[c], b[c]))
-        RDV_PSTAGE(ka6, kb6,
-                   fma(h[c], fma(ka5[c], RK_B6, fma(ka4[c], RK_B5, fma(ka3[c], RK_B4, fma(ka2[c], RK_B3, ka0[c] * RK_B1)))),
-                       a[c]),
-                   fma(h[c], fma(kb5[c], RK_B6, fma(kb4[c], RK_B5, fma(kb3[c], RK_B4, fma(kb2[c], RK_B3, kb0[c] * RK_B1)))),
-                       b[c]))
-#undef RDV_PSTAGE
+#pragma unroll
+        for (int c = 0; c < 2; ++c) plane_attempt<POLY>(a[c], b[c], g[c], om2[c], h[c], as[c], bs[c], ea[c], eb[c]);
 #pragma unroll
         for (int c = 0; c < 2; ++c) {
             // as / bs hold (a_new, b_new) of the attempted step
-            const double ea = h[c] * fma(ka6[c], RK_E7, fma(ka5[c], RK_E6, fma(ka4[c], RK_E5, fma(ka3[c], RK_E4,
-                                     fma(ka2[c], RK_E3, ka0[c] * RK_E1)))));
-            const double eb = h[c] * fma(kb6[c], RK_E7, fma(kb5[c], RK_E6, fma(kb4[c], RK_E5, fma(kb3[c], RK_E4,
-                                     fma(kb2[c], RK_E3, kb0[c] * RK_E1)))));
             float ynf[4];
-            const float esf = plane_err2_f32(ea, eb, as[c], bs[c], q0f[c], pf[c], ycf[c], ynf);
+            const float esf = plane_err2_f32(ea[c], eb[c], as[c], bs[c], q0f[c], pf[c], ycf[c], ynf);
             const bool live = !done[c] && !failed[c];
             const bool bad = fail_now[c] || !(esf < 1.0e30f);
             bool accept = esf < 1.0f;
             if (fabsf(esf - 1.0f) < 1.0e-3f)           // threshold region: decide with the fp64 norm
-                accept = plane_err2_f64(ea, eb, a[c], b[c], as[c], bs[c], q0[c], p[c]) < 1.0;
+                accept = plane_err2_f64(ea[c], eb[c], a[c], b[c], as[c], bs[c], q0[c], p[c]) < 1.0;
             const float pw = 0.9f * pow_neg_tenth_f32(fminf(fmaxf(esf, 1e-12f), 1e8f));
             float factor = accept ? fminf(10.0f, pw) : fmaxf(0.2f, pw);
             if (accept && rejected[c]) factor = fminf(1.0f, factor);
@@ -1033,7 +1108,7 @@ RDV_DEV int rk45_iso_plane_pair(double (&ya)[7], double (&yb)[7], const double d
                 n_rejected += (!bad && !accept) ? 1 : 0;
             }
             if (commit) {
-                a[c] = as[c]; b[c] = bs[c]; ka0[c] = ka6[c]; kb0[c] = kb6[c];
+                a[c] = as[c]; b[c] = bs[c]; g[c] = plane_g(as[c], bs[c], om2[c]);
 #pragma unroll
                 for (int i = 0; i < 4; ++i) ycf[c][i] = ynf[i];
                 t[c] = t_new[c];
@@ -1048,6 +1123,23 @@ RDV_DEV int rk45_iso_plane_pair(double (&ya)[7], double (&yb)[7], const double d
         yb[i] = fma(b[1], p[1][i], a[1] * q0[1][i]);
     }
     return (failed[0] || failed[1]) ? -1 : accepted[0] + accepted[1];
+}
+// a pair with a body outside the polynomials' range: the two solves one after the other, each in its own form (the
+// same bits as in the lock-step form), out of line
+__device__ __noinline__ int rk45_iso_plane_pair_mixed(double (&ya)[7], double (&yb)[7], const double dt, int &n_rejected)
+{
+    const int ka = rk45_iso_plane(ya, dt, n_rejected);
+    const int kb = rk45_iso_plane(yb, dt, n_rejected);
+    return (ka < 0 || kb < 0) ? -1 : ka + kb;
+}
+RDV_DEV int rk45_iso_plane_pair(double (&ya)[7], double (&yb)[7], const double dt, int &n_rejected)
+{
+#if RDV_PLANE_POLY
+    if (!(plane_poly_covers(ya, dt) && plane_poly_covers(yb, dt))) return rk45_iso_plane_pair_mixed(ya, yb, dt, n_rejected);
+    return rk45_iso_plane_pair_solve<true>(ya, yb, dt, n_rejected);
+#else
+    return rk45_iso_plane_pair_solve<false>(ya, yb, dt, n_rejected);
+#endif
 }
 
 // Closed-form alternative (opt-in, RDV_INTEGRATOR_CLOSED_FORM; only valid for ISO bodies):
