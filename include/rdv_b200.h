@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define RDV_ABI_VERSION 15
+#define RDV_ABI_VERSION 16
 #define RDV_OBS_DIM 17          /* rendezvous_env.py:133-137 Box(-1, 1, (17,), float32) */
 #define RDV_ACT_DIM 6           /* rendezvous_env.py:140-144 Box(-1, 1, (6,),  float32) */
 #define RDV_N_UNIFORMS 24       /* draws consumed by one reset(): rendezvous_env.py:229-250 */
@@ -232,6 +232,19 @@ typedef struct RdvRolloutIO {
      * results accumulated in registers from the state at launch (sample 0) to the env's first done; finished envs
      * stop stepping.  NULL: off. */
     double  *mc_out;
+    /* Policy tables (many actors in one launch, e.g. one model per parameter set of a sweep): a device array of
+     * RdvPolicy entries and, for every tile of 128 consecutive envs, the index of the entry its envs use.  NULL: every
+     * env uses `policy`, exactly as without the fields.  With a table `policy` is not read (its weights may be NULL);
+     * needs a policy action source (RDV_ACTIONS_POLICY / _SAMPLE, every entry with log_std for sampling) and the
+     * reference's isotropic bodies with the RK45 integrator; combines with the evaluator mode, auto-reset, reset_rows
+     * and RdvState.param_table.  Every entry must have hidden = 64 and non-NULL weights and biases, and, for
+     * RDV_ACTIONS_POLICY_SAMPLE, a non-NULL log_std; the library does not read the table on the host, so the kernel
+     * checks each entry when a group stages it.  A tile whose index lies outside [0, policy_count), or whose entry
+     * fails that check, takes zero actions, and each of its env-steps counts in RDV_S_FAILURES. */
+    const RdvPolicy *policy_table;    /* nullable, device, [policy_count]                                  */
+    const int32_t *policy_tile;       /* device, [ceil(n / 128)]: entry of envs 128 t .. 128 t + 127        */
+    int32_t  policy_count;
+    int32_t  reserved3;
 } RdvRolloutIO;
 #define RDV_RESET_ROWS 23
 /* Columns of RdvRolloutIO.mc_out: the workbook columns of monte_carlo.py:190-203 (errors in rad / rad/s, the host

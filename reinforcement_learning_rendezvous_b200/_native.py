@@ -27,7 +27,7 @@ HOST_LIB = os.path.join(PKG_DIR, "_rdv_host" + (sysconfig.get_config_var("EXT_SU
 SOURCES = ("rdv_b200.cu",)
 HEADERS = ("rdv_math.cuh", "rdv_plane_poly.h", "rdv_env.cuh", "rdv_step.cuh", "rdv_policy.cuh", "rdv_policy_tc.cuh")
 
-ABI_VERSION = 15
+ABI_VERSION = 16
 OBS_DIM, ACT_DIM, N_UNIFORMS = 17, 6, 24
 
 # rows of RdvState.f64 / RdvState.i32, statistics slots, episode-record columns (rdv_b200.h)
@@ -113,10 +113,13 @@ class RdvRolloutIO(C.Structure):
         ("actions_out", C.c_void_p), ("obs", C.c_void_p), ("rewards", C.c_void_p), ("dones", C.c_void_p),
         ("obs_steps", C.c_void_p), ("stats", C.c_void_p), ("policy", RdvPolicy),
         ("reset_rows", C.c_void_p), ("sm_reserve", C.c_int32), ("reserved2", C.c_int32), ("mc_out", C.c_void_p),
+        ("policy_table", C.c_void_p), ("policy_tile", C.c_void_p), ("policy_count", C.c_int32),
+        ("reserved3", C.c_int32),
     ]
 
 
 RESET_ROWS = 23
+POLICY_TILE = 128               # envs per entry of RdvRolloutIO.policy_tile
 (MC_EP_LEN, MC_NUM_COLLISIONS, MC_COLLIDED, MC_TOTAL_REWARD, MC_TOTAL_DELTA_V, MC_NUM_SUCCESSES, MC_SUCCEEDED,
  MC_MIN_KOZ, MC_POS_ERR, MC_VEL_ERR, MC_ATT_ERR, MC_ROT_ERR, MC_LEVEL, MC_TAIL_COUNT, MC_END_REASON,
  MC_TOTAL_DELTA_W, MC_NCOL) = range(17)

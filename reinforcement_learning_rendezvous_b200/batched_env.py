@@ -30,6 +30,25 @@ def _stream_ptr(device) -> C.c_void_p:
     return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
+def policy_tile_indices(policy_tiles, num_envs: int, count: int) -> np.ndarray:
+    """Host-side check of a policy-table tile map: one int per tile of 128 envs (``ceil(num_envs / 128)``), each in
+    ``[0, count)``.  Returns it as int32 (``RdvRolloutIO.policy_tile``)."""
+    if policy_tiles is None:
+        raise ValueError("a PolicyTable needs policy_tiles (one entry index per tile of 128 envs)")
+    if isinstance(policy_tiles, torch.Tensor):
+        policy_tiles = policy_tiles.detach().cpu().numpy()
+    tiles = np.asarray(policy_tiles)
+    if tiles.dtype.kind not in "iu":
+        raise ValueError("policy_tiles must hold integers")
+    tiles = tiles.reshape(-1).astype(np.int64)
+    want = (int(num_envs) + N.POLICY_TILE - 1) // N.POLICY_TILE
+    if tiles.size != want:
+        raise ValueError(f"policy_tiles has {tiles.size} entries, expected {want} (one per {N.POLICY_TILE} envs)")
+    if tiles.size and (tiles.min() < 0 or tiles.max() >= count):
+        raise ValueError(f"policy_tiles holds an index outside [0, {count})")
+    return tiles.astype(np.int32)
+
+
 class ParamGroup:
     """A contiguous env range [lo, hi) sharing one RdvParams block."""
 
@@ -73,6 +92,7 @@ class BatchedRendezvousEnv:
         self._seed, self.env_offset, self.auto_reset = int(seed), int(env_offset), bool(auto_reset)
         self.ctor_kwargs = dict(ctor_kwargs)
         self.reset_rows = None          # prefetched reset rows carried from rollout to rollout (allocated on first use)
+        self._tile_map = None           # (bytes, device int32 tensor): the last policy-table tile map uploaded
         self.sm_reserve = 0             # SMs a rollout launch leaves free (distributed.py: overlapped stats all-reduce)
 
         if param_batches:
@@ -226,7 +246,8 @@ class BatchedRendezvousEnv:
     def rollout(self, steps: int, actions: Optional[torch.Tensor] = None, action_seed: Optional[int] = None,
                 step_base: int = 0, record_rewards: bool = False, record_dones: bool = False,
                 record_obs: bool = False, record_actions: bool = False, policy=None,
-                stochastic: bool = False, carry_reset_rows: bool = True, monte_carlo: bool = False) -> dict:
+                stochastic: bool = False, carry_reset_rows: bool = True, monte_carlo: bool = False,
+                policy_tiles=None) -> dict:
         """``steps`` consecutive env steps in ONE kernel launch (state stays in registers, finished envs restart
         in place when ``auto_reset``).  Actions come from ``actions`` ([steps, N, 6] float32/float64 on the device) or,
         when it is None, from the device Philox stream ``(action_seed; global env id, step_base + k)`` as U(-1,1) fp64
@@ -240,11 +261,16 @@ class BatchedRendezvousEnv:
         state in a device scratch between launches (short launches then run at the rate of long ones).
         ``monte_carlo`` (needs ``auto_reset=False``): evaluator mode -- an env stops at its first done and the launch
         returns ``mc`` f64 [N, MC_NCOL], the per-episode columns of monte_carlo.py:190-203 accumulated on the device.
-        Asynchronous on the current stream."""
+        ``policy`` may also be a :class:`~.policy.PolicyTable`: then ``policy_tiles`` (ints or an int tensor, one per
+        tile of 128 envs) names the entry that acts for envs ``128 t .. 128 t + 127``, all in the same launch; every
+        tile gives the bits a separate env of its envs (same seed, ``env_offset`` = tile start) rolled with that entry
+        would give.  Asynchronous on the current stream (the tile map is checked on the host: a device tensor given as
+        ``policy_tiles`` is read back for that, which waits for the stream; a host sequence does not)."""
         steps = int(steps)
         n, dev = self.num_envs, self.device
         if steps < 0:
             raise ValueError("steps must be >= 0")
+        table = None                    # policy tables: the tile map on the device
         if actions is not None:
             if actions.device != dev or actions.dtype not in (torch.float32, torch.float64):
                 raise ValueError("actions must be a float32/float64 tensor on the env's device")
@@ -254,15 +280,26 @@ class BatchedRendezvousEnv:
             source = N.ACTIONS_F64 if actions.dtype == torch.float64 else N.ACTIONS_F32
             esz = 8 if actions.dtype == torch.float64 else 4
         elif policy is not None:
+            from .policy import PolicyTable
             if policy.device != dev:
                 raise ValueError("policy and env live on different devices")
-            if stochastic and (policy.log_std is None or action_seed is None):
+            if isinstance(policy, PolicyTable):
+                tiles = policy_tile_indices(policy_tiles, n, len(policy))
+                if stochastic and (not policy.stochastic_ready or action_seed is None):
+                    raise ValueError("stochastic policy-table rollouts need log_std in every entry and an action_seed")
+                if len(self._units) > 1:
+                    raise NotImplementedError("policy tables with param_batches of general-inertia or closed-form "
+                                              "groups (one launch per group)")
+                table = self._policy_tile_map(tiles)
+            elif stochastic and (policy.log_std is None or action_seed is None):
                 raise ValueError("stochastic policy rollouts need policy.log_std and an action_seed")
             source, esz = (N.ACTIONS_POLICY_SAMPLE if stochastic else N.ACTIONS_POLICY), 0
         else:
             if action_seed is None:
                 raise ValueError("give an actions tensor, an action_seed (device-generated actions) or a policy")
             source, esz = N.ACTIONS_PHILOX, 0
+        if policy_tiles is not None and table is None:
+            raise ValueError("policy_tiles needs a PolicyTable policy")
         out = {"obs": self.obs}
         rew = torch.empty((steps, n), dtype=torch.float64, device=dev) if record_rewards else None
         don = torch.empty((steps, n), dtype=torch.uint8, device=dev) if record_dones else None
@@ -290,13 +327,15 @@ class BatchedRendezvousEnv:
                     rew.data_ptr() if rew is not None else None, don.data_ptr() if don is not None else None,
                     obs_steps.data_ptr() if obs_steps is not None else None,
                     self.stats.data_ptr() if self.stats is not None else None,
-                    policy._c if policy is not None else N.RdvPolicy(),
+                    policy._c if policy is not None and table is None else N.RdvPolicy(),
                     self._reset_rows_ptr(g) if carry_reset_rows else None, int(self.sm_reserve), 0,
-                    mc_out.data_ptr() + g.lo * N.MC_NCOL * 8 if mc_out is not None else None)
+                    mc_out.data_ptr() + g.lo * N.MC_NCOL * 8 if mc_out is not None else None,
+                    policy.table.data_ptr() if table is not None else None,
+                    table.data_ptr() if table is not None else None, len(policy) if table is not None else 0, 0)
                 st = self._state_of(g)
                 N.check(self.lib.rdv_rollout(C.byref(g.params), C.byref(st), C.byref(io), g.n, self.seed,
                                              self.env_offset + g.lo, stream), "rdv_rollout")
-        self._keepalive = (actions, policy)
+        self._keepalive = (actions, policy, table)
         if rew is not None:
             out["rewards"] = rew
         if don is not None:
@@ -308,6 +347,17 @@ class BatchedRendezvousEnv:
         if mc_out is not None:
             out["mc"] = mc_out
         return out
+
+    def _policy_tile_map(self, tiles: np.ndarray) -> torch.Tensor:
+        """The checked tile map on the device.  The last one is kept, so repeated rollouts with the same map upload
+        nothing; a new one goes through pinned memory with a non-blocking copy, so the call does not wait for the
+        stream."""
+        key = tiles.tobytes()
+        if self._tile_map is None or self._tile_map[0] != key:
+            dev_map = torch.empty(tiles.shape, dtype=torch.int32, device=self.device)
+            dev_map.copy_(torch.from_numpy(tiles).pin_memory(), non_blocking=True)
+            self._tile_map = (key, dev_map)
+        return self._tile_map[1]
 
     def reset(self, mask: Optional[torch.Tensor] = None, uniforms: Optional[torch.Tensor] = None,
               bump_episode: bool = True) -> torch.Tensor:

@@ -17,6 +17,7 @@
 #include <stdlib.h>
 #include <atomic>
 #include <mutex>
+#include <type_traits>
 #include "rdv_step.cuh"
 #include "rdv_policy.cuh"
 #include "rdv_policy_tc.cuh"
@@ -455,6 +456,10 @@ __global__ void __launch_bounds__(TPB, RDV_STEP_MIN_CTAS) step_kernel(const __gr
 // POLICY: the action of every step is the output of the SB3 MlpPolicy actor, evaluated on the tensor cores
 // (tcgen05 / TMEM, rdv_policy_tc.cuh: groups of 128 threads = 128 envs = one UMMA tile) from the observation the
 // previous step produced.
+// PTAB (policy tables, with POLICY): every 128-env tile of the launch has its own actor, an entry of
+// RdvRolloutIO.policy_table chosen by policy_tile.  Slices are cut at multiples of 128 envs and passes are 256 envs,
+// so each group's tile is 128 envs starting at a multiple of 128 from env 0 of the launch; each group stages its
+// entry's weights into its own weight set (TableSmem) when the entry differs from the one it holds.
 #ifndef RDV_SYNC_PERIOD
 #define RDV_SYNC_PERIOD 8             /* steps between the CTA barriers that keep the warps in one code region */
 #endif
@@ -497,18 +502,22 @@ RDV_DEV void take_reset_row(const double *rw, const int64_t rs, EnvRegs &e, EnvC
 // the trajectory off the workers: recomputing the reset rows that were used.  Workers post (lane, episode) requests in
 // shared memory and never wait -- a row that is not ready when its lane finishes is computed on the spot, as before.
 template <bool ISO, bool CLOSED, int TPB_, bool POLICY = false, bool MC = false, bool TABLE = false, bool OBS = POLICY,
-          bool HELP = false>
+          bool HELP = false, bool PTAB = false>
 __global__ void __launch_bounds__(TPB_ + (HELP ? 64 : 0), 1)
 rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __grid_constant__ RdvRolloutIO io,
                const int64_t n, const uint64_t seed, const int64_t env_offset)
 {
     static_assert(!HELP || (!POLICY && !MC && !TABLE && !OBS), "helper warps: plain variant only");
+    static_assert(!PTAB || (POLICY && TPB_ == 256), "policy tables: the fused actor with two 128-thread groups");
     constexpr int NW = TPB_ / 32;                       // worker warps
     constexpr int NWT = NW + (HELP ? 2 : 0);            // all warps of the CTA
     extern __shared__ __align__(128) unsigned char dyn_smem[];
-    tc::TileSmem *ts = reinterpret_cast<tc::TileSmem *>(dyn_smem);
+    typedef typename std::conditional<PTAB, tc::TableSmem, tc::TileSmem>::type TS;
+    TS *ts = reinterpret_cast<TS *>(dyn_smem);
     uint32_t tmem_all = 0, mma_phase = 0;
-    if (POLICY) {
+    if constexpr (PTAB) {
+        tmem_all = tc::tile_cta_setup(*ts);             // the weights are staged per group, at the start of a pass
+    } else if (POLICY) {
         // the actor's weights may have been written by the previous kernel of the stream (an optimiser step), so the
         // dependency wait of a programmatic launch (below) comes before they are read
         asm volatile("griddepcontrol.wait;" ::: "memory");
@@ -582,13 +591,18 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
                   "staging rows + team rows must fit the group's activation tile");
     constexpr bool want_obs = POLICY || OBS;
     // this CTA's slice [lo, hi) and its passes; with a parameter table the slices are cut at multiples of 32 envs so
-    // that a warp never straddles two parameter blocks
-    const int64_t units = TABLE ? (n + 31) / 32 : n, unit = TABLE ? 32 : 1;
+    // that a warp never straddles two parameter blocks, with a policy table at multiples of 128 so that a group's tile
+    // never straddles two policy tiles (the results do not depend on the slicing)
+    const int64_t units = PTAB ? (n + 127) / 128 : TABLE ? (n + 31) / 32 : n, unit = PTAB ? 128 : TABLE ? 32 : 1;
     const int64_t lo = unit * (units * (int64_t)blockIdx.x / gridDim.x);
     const int64_t hi_raw = unit * (units * ((int64_t)blockIdx.x + 1) / gridDim.x), hi = hi_raw < n ? hi_raw : n;
     const int64_t span = hi - lo;
     const int passes = (int)((span + TPB_ - 1) / TPB_);
-    const int64_t chunk = TABLE ? TPB_ : (passes > 0 ? (span + passes - 1) / passes : 0);
+    const int64_t chunk = (TABLE || PTAB) ? TPB_ : (passes > 0 ? (span + passes - 1) / passes : 0);
+    // policy tables: the entry whose weights this thread's group holds (-1: none yet; uniform within the group), and
+    // whether the group's tile of the current pass has an index outside the table
+    int ptab_staged = -1;
+    bool ptab_bad = false;
     StepStats st = {};
     // Programmatic dependent launch: when rdv_rollout launches with the stream-serialisation attribute, this grid may
     // become resident while the previous kernel of the stream is still draining (its CTAs finish at different times),
@@ -652,6 +666,29 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
         const int64_t env_id = env_offset + i;
         const int rows_w = (int)((c_hi - warp_base) < 32 ? ((c_hi - warp_base) > 0 ? (c_hi - warp_base) : 0) : 32);
         const RdvParams &P = params_of<TABLE>(Pc, S, i);
+        if constexpr (PTAB) {
+            // The group's tile: idle lanes shadow the slice's last env, which lies in the tile of the group's active
+            // envs (or, for a group with none, is the same env for all 128 threads), so `want` is group-uniform.
+            const int g = threadIdx.x >> 7;
+            const int32_t want = io.policy_tile[i >> 7];
+            ptab_bad = want < 0 || want >= io.policy_count;         // never read outside the table: zero actions
+            if (!ptab_bad) {
+                // an entry the actor cannot run is treated the same way: another width (the staging reads 64-wide
+                // matrices), a missing weight, or no Gaussian head when sampling
+                const RdvPolicy &pe = io.policy_table[want];
+                ptab_bad = pe.hidden != tc::H || !pe.w0 || !pe.b0 || !pe.w1 || !pe.b1 || !pe.w2 || !pe.b2 ||
+                           (src == RDV_ACTIONS_POLICY_SAMPLE && !pe.log_std);
+            }
+            if (!ptab_bad && want != ptab_staged) {
+                // the group's MMAs of its previous tile have completed (every thread waited for them), but a thread may
+                // still read the previous biases / std: wait for the group, restage, publish to the async proxy
+                tc::group_sync(g, tc::TM);
+                tc::stage_weights<tc::TM>(io.policy_table[want], ts->w[g], threadIdx.x & (tc::TM - 1));
+                tc::fence_async_smem();
+                tc::group_sync(g, tc::TM);
+                ptab_staged = want;
+            }
+        }
 
         EnvRegs e;
         EnvCounters c;
@@ -735,14 +772,23 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
             // through the actor on the tensor cores: thread = row = TMEM lane
             float a[RDV_ACT_DIM];
             const int g = threadIdx.x >> 7;
-            tc::tile_forward(*ts, g, threadIdx.x & 127, TPB_ - 128 * g < 128 ? TPB_ - 128 * g : 128, ov,
-                             tmem_all + (uint32_t)g * tc::GROUP_COLS, mma_phase, a, [] {});
+            if (PTAB && ptab_bad) {
+                // tile index outside the policy table, or an entry the actor cannot run: zero actions, one failure
+                // per env-step
+#pragma unroll
+                for (int j = 0; j < RDV_ACT_DIM; ++j) a[j] = 0.0f;
+                if (active && (!MC || alive)) st.fail += 1;
+            } else {
+                tc::tile_forward(ts->al[g], &ts->mma_bar[g], ts->w[PTAB ? g : 0], g, threadIdx.x & 127,
+                                 TPB_ - 128 * g < 128 ? TPB_ - 128 * g : 128, ov, tmem_all + (uint32_t)g * tc::GROUP_COLS,
+                                 mma_phase, a, [] {});
+            }
             const bool sample = src == RDV_ACTIONS_POLICY_SAMPLE;
-            if (sample) {                                     // a ~ N(mean, exp(log_std)^2)
+            if (sample && !(PTAB && ptab_bad)) {              // a ~ N(mean, exp(log_std)^2)
                 float z[RDV_ACT_DIM];
                 philox_normals(io.action_seed, env_id, io.step_base + k, z);
 #pragma unroll
-                for (int j = 0; j < RDV_ACT_DIM; ++j) a[j] = fmaf(ts->std[j], z[j], a[j]);
+                for (int j = 0; j < RDV_ACT_DIM; ++j) a[j] = fmaf(ts->w[PTAB ? g : 0].std[j], z[j], a[j]);
             }
             float ac[RDV_ACT_DIM];
 #pragma unroll
@@ -1516,7 +1562,15 @@ int rdv_rollout(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, i
     if (io->steps < 0 || io->action_source < 0 || io->action_source > RDV_ACTIONS_POLICY_SAMPLE) return RDV_ERR_SIZE;
     if (io->auto_reset != 0 && io->auto_reset != 1) return RDV_ERR_SIZE;
     const bool policy = io->action_source == RDV_ACTIONS_POLICY || io->action_source == RDV_ACTIONS_POLICY_SAMPLE;
-    if (policy) {
+    const bool ptab = io->policy_table != nullptr;
+    if (ptab) {
+        // policy tables: the fused actor only; entries are checked by the caller (hidden = 64, log_std for sampling)
+        if (!policy) return RDV_ERR_SIZE;
+        if (!io->policy_tile) return RDV_ERR_NULL;
+        if (io->policy_count < 1) return RDV_ERR_SIZE;
+        if (((uintptr_t)io->policy_table & 7) || ((uintptr_t)io->policy_tile & 3)) return RDV_ERR_ALIGN;
+        if (!(p->iso_c && p->iso_t) || p->integrator == RDV_INTEGRATOR_CLOSED_FORM) return RDV_ERR_UNSUPPORTED;
+    } else if (policy) {
         const RdvPolicy *pi = &io->policy;
         if (io->action_source == RDV_ACTIONS_POLICY_SAMPLE && !pi->log_std) return RDV_ERR_NULL;
         if (!pi->w0 || !pi->b0 || !pi->w1 || !pi->b1 || !pi->w2 || !pi->b2) return RDV_ERR_NULL;
@@ -1542,7 +1596,7 @@ int rdv_rollout(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, i
     if ((uintptr_t)io->reset_rows & 7) return RDV_ERR_ALIGN;
     // development / test override of the CTA size (rdv_tune): 256 | 384 | 448 | 512; the evaluator mode has one size
     const bool table = s->param_table != nullptr;
-    const int force_tpb = (mc || table) ? 256 : g_tune_tpb.load(std::memory_order_relaxed);
+    const int force_tpb = (mc || table || ptab) ? 256 : g_tune_tpb.load(std::memory_order_relaxed);
     const int64_t max_tpb = force_tpb > 0 ? force_tpb : 512;
     const int64_t passes = (per_cta + max_tpb - 1) / max_tpb;
     const int64_t chunk = force_tpb > 0 ? force_tpb : (per_cta + passes - 1) / passes;
@@ -1587,30 +1641,42 @@ int rdv_rollout(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, i
     else if (chunk <= 448) { if (helpers && ISO_ && !CL_) RDV_LAUNCH_H(true, false) else RDV_LAUNCH_R(ISO_, CL_, 448) } \
     else RDV_LAUNCH_R(ISO_, CL_, 512)
 #define RDV_LAUNCH_P(T_) RDV_LAUNCH_K((rollout_kernel<true, false, T_, true, false>), T_, sizeof(tc::TileSmem))
-    if (table) {
-        if (!iso || closed) return RDV_ERR_UNSUPPORTED;      // parameter tables: the reference's bodies, RK45
-        if (mc && policy) RDV_LAUNCH_K((rollout_kernel<true, false, 256, true, true, true>), 256, sizeof(tc::TileSmem))
-        else if (mc) RDV_LAUNCH_K((rollout_kernel<true, false, 256, false, true, true, true>), 256, RDV_ROWS_SMEM(256))
-        else if (policy) RDV_LAUNCH_K((rollout_kernel<true, false, 256, true, false, true>), 256, sizeof(tc::TileSmem))
-        else RDV_LAUNCH_K((rollout_kernel<true, false, 256, false, false, true, true>), 256, RDV_ROWS_SMEM(256))
+#define RDV_LAUNCH_PT(MC_, TABLE_) \
+    RDV_LAUNCH_K((rollout_kernel<true, false, 256, true, MC_, TABLE_, true, false, true>), 256, sizeof(tc::TableSmem))
+    // the policy-table variants are instantiated after all others: ptxas handles a module's kernels in that order, and
+    // with them first the register allocation of an existing variant (POLICY + TABLE) came out differently
+    if (!ptab) {
+        if (table) {
+            if (!iso || closed) return RDV_ERR_UNSUPPORTED;      // parameter tables: the reference's bodies, RK45
+            if (mc && policy) RDV_LAUNCH_K((rollout_kernel<true, false, 256, true, true, true>), 256, sizeof(tc::TileSmem))
+            else if (mc) RDV_LAUNCH_K((rollout_kernel<true, false, 256, false, true, true, true>), 256, RDV_ROWS_SMEM(256))
+            else if (policy) RDV_LAUNCH_K((rollout_kernel<true, false, 256, true, false, true>), 256, sizeof(tc::TileSmem))
+            else RDV_LAUNCH_K((rollout_kernel<true, false, 256, false, false, true, true>), 256, RDV_ROWS_SMEM(256))
+        }
+        else if (mc) {
+            if (!iso || closed) return RDV_ERR_UNSUPPORTED;      // the evaluator mode is built for the reference's env
+            if (policy) RDV_LAUNCH_K((rollout_kernel<true, false, 256, true, true>), 256, sizeof(tc::TileSmem))
+            else RDV_LAUNCH_K((rollout_kernel<true, false, 256, false, true, false, true>), 256, RDV_ROWS_SMEM(256))
+        }
+        else if (policy) {
+            if (!iso || closed) return RDV_ERR_UNSUPPORTED;      // the fused policy is built for the reference's env
+            if (chunk <= 256) RDV_LAUNCH_P(256)
+            else if (chunk <= 384) RDV_LAUNCH_P(384)
+            else if (chunk <= 448) RDV_LAUNCH_P(448)
+            else RDV_LAUNCH_P(512)
+        }
+        else if (closed) { RDV_PICK_R(true, true) }
+        else if (iso) { RDV_PICK_R(true, false) }
+        else RDV_LAUNCH_OBS(false, false)                          // general inertia / held torque: one shape
+    } else {                                                    // (bodies and integrator checked above)
+        if (mc && table) RDV_LAUNCH_PT(true, true)
+        else if (mc) RDV_LAUNCH_PT(true, false)
+        else if (table) RDV_LAUNCH_PT(false, true)
+        else RDV_LAUNCH_PT(false, false)
     }
-    else if (mc) {
-        if (!iso || closed) return RDV_ERR_UNSUPPORTED;      // the evaluator mode is built for the reference's env
-        if (policy) RDV_LAUNCH_K((rollout_kernel<true, false, 256, true, true>), 256, sizeof(tc::TileSmem))
-        else RDV_LAUNCH_K((rollout_kernel<true, false, 256, false, true, false, true>), 256, RDV_ROWS_SMEM(256))
-    }
-    else if (policy) {
-        if (!iso || closed) return RDV_ERR_UNSUPPORTED;      // the fused policy is built for the reference's env
-        if (chunk <= 256) RDV_LAUNCH_P(256)
-        else if (chunk <= 384) RDV_LAUNCH_P(384)
-        else if (chunk <= 448) RDV_LAUNCH_P(448)
-        else RDV_LAUNCH_P(512)
-    }
-    else if (closed) { RDV_PICK_R(true, true) }
-    else if (iso) { RDV_PICK_R(true, false) }
-    else RDV_LAUNCH_OBS(false, false)                          // general inertia / held torque: one shape
 #undef RDV_LAUNCH_OBS
 #undef RDV_LAUNCH_P
+#undef RDV_LAUNCH_PT
 #undef RDV_PICK_R
 #undef RDV_LAUNCH_H
 #undef RDV_LAUNCH_R

@@ -2,7 +2,9 @@
 // 5th-generation tensor cores: tcgen05.mma with TMEM accumulators AND TMEM-resident A operands.  tile_setup /
 // tile_forward / tile_teardown are used by two kernels: policy_tc_kernel below (rdv_policy_forward, stand-alone,
 // observations from HBM) and rollout_kernel in rdv_b200.cu (the actor of every step of a fused rollout,
-// observations from the env state in registers).
+// observations from the env state in registers).  The set-up is split: the CTA-wide part (mbarriers, TMEM) and
+// stage_weights, which any set of threads can run into any WeightSet -- the policy-table rollout has one weight set per
+// group and restages it when the group's tile uses another actor.
 //
 // A group of 128 threads owns tiles of 128 environments (UMMA M = 128, one env per thread / TMEM lane):
 //
@@ -70,16 +72,24 @@ constexpr uint32_t A_COL = 64;
 constexpr int OBS_TILE = TM * RDV_OBS_DIM;              // floats of one observation tile (8704 B, 16 B multiple)
 constexpr float TANH_SCALE = 2.8853900817779268f;       // 2 log2(e)
 
-// what a tile forward needs: lo activations per group, split weights, biases, MMA mbarriers, the TMEM base
-struct TileSmem {
-    alignas(16) elem_t al[GROUPS][H * TM];                       // lo part of the activations, [group][chunk][row][CHUNK]
+// one actor's weights as the MMAs read them: split hi / lo, tanh factor folded in (28.3 KiB)
+struct WeightSet {
     alignas(16) elem_t w0h[K0 * H], w0l[K0 * H];                 // [chunk][n][CHUNK]
     alignas(16) elem_t w1h[H * H], w1l[H * H];
     alignas(16) elem_t w2h[H * N3], w2l[H * N3];
     float b1[H], b2[N3], std[8];                                 // std = exp(log_std) (0 without a Gaussian head)
+};
+static_assert(sizeof(WeightSet) % 16 == 0, "weight sets must stay 16-byte aligned");
+// what a tile forward needs: lo activations per group (NA tiles), NW weight sets, MMA mbarriers, the TMEM base
+template <int NA, int NW>
+struct TileSmemT {
+    alignas(16) elem_t al[NA][H * TM];                           // lo part of the activations, [group][chunk][row][CHUNK]
+    WeightSet w[NW];
     uint64_t mma_bar[GROUPS];
     uint32_t tmem_base, pad[3];
 };
+typedef TileSmemT<GROUPS, 1> TileSmem;  // one weight set shared by every group of the CTA
+typedef TileSmemT<2, 2> TableSmem;      // policy tables: two groups of 128 threads, each with its own weight set
 // the stand-alone kernel adds the bulk-copy landing zone of the next observation tile
 struct Smem {
     TileSmem t;
@@ -204,11 +214,12 @@ template <int NT, int N_VALID, int K_VALID, int N_PAD, int K_PAD>
 struct WeightTile {
     static constexpr int PER = (N_PAD * K_PAD + NT - 1) / NT;
     float x[PER];
-    __device__ __forceinline__ void fetch(const float *__restrict__ w, const float *__restrict__ bias_col)
+    // t: the calling thread's index among the NT staging threads
+    __device__ __forceinline__ void fetch(const float *__restrict__ w, const float *__restrict__ bias_col, int t)
     {
 #pragma unroll
         for (int i = 0; i < PER; ++i) {
-            const int idx = threadIdx.x + i * NT;
+            const int idx = t + i * NT;
             const int nn = idx / K_PAD, k = idx % K_PAD;
             x[i] = 0.0f;
             if (idx < N_PAD * K_PAD && nn < N_VALID) {
@@ -217,11 +228,11 @@ struct WeightTile {
             }
         }
     }
-    __device__ __forceinline__ void store(float scale, elem_t *wh, elem_t *wl) const
+    __device__ __forceinline__ void store(float scale, elem_t *wh, elem_t *wl, int t) const
     {
 #pragma unroll
         for (int i = 0; i < PER; ++i) {
-            const int idx = threadIdx.x + i * NT;
+            const int idx = t + i * NT;
             if (idx < N_PAD * K_PAD) {
                 const int nn = idx / K_PAD, k = idx % K_PAD;
                 const int o = ((k / CHUNK) * N_PAD + nn) * CHUNK + (k % CHUNK);
@@ -339,10 +350,30 @@ __device__ __forceinline__ void hidden_epilogue(uint32_t lane_addr, const float 
     tmem_st_wait();
 }
 
-// Whole CTA of NT threads, once per launch: weights (hi / lo, tanh factor folded in), biases, the groups' MMA
-// mbarriers, 512 TMEM columns.  Ends with a __syncthreads; returns the TMEM base address.
+// NT threads (t = 0 .. NT-1 among them) split the weights of pi into w: hi / lo, tanh factor folded in, biases and
+// std.  The caller orders the stores before the MMAs that read w (fence.proxy.async, then a barrier of the NT threads).
 template <int NT>
-__device__ __forceinline__ uint32_t tile_setup(const RdvPolicy &pi, TileSmem &s)
+__device__ __forceinline__ void stage_weights(const RdvPolicy &pi, WeightSet &w, int t)
+{
+    WeightTile<NT, H, RDV_OBS_DIM, H, K0> t0;
+    WeightTile<NT, H, H, H, H> t1;
+    WeightTile<NT, RDV_ACT_DIM, H, N3, H> t2;
+    t0.fetch(pi.w0, pi.b0, t);
+    t1.fetch(pi.w1, nullptr, t);
+    t2.fetch(pi.w2, nullptr, t);
+    const float bias1 = t < H ? __ldg(pi.b1 + t) : 0.0f;
+    const float bias2 = t < RDV_ACT_DIM ? __ldg(pi.b2 + t) : 0.0f;
+    const float lstd = (t < RDV_ACT_DIM && pi.log_std) ? __ldg(pi.log_std + t) : 0.0f;
+    t0.store(TANH_SCALE, w.w0h, w.w0l, t);
+    t1.store(TANH_SCALE, w.w1h, w.w1l, t);
+    t2.store(1.0f, w.w2h, w.w2l, t);
+    if (t < H) w.b1[t] = bias1 * TANH_SCALE;
+    if (t < N3) w.b2[t] = bias2;
+    if (t < 8) w.std[t] = (t < RDV_ACT_DIM && pi.log_std) ? expf(lstd) : 0.0f;
+}
+// The CTA-wide part of the set-up, in two halves: the groups' MMA mbarriers (thread 0) ...
+template <class S>
+__device__ __forceinline__ void tile_init_barriers(S &s)
 {
     if (threadIdx.x == 0) {
 #pragma unroll
@@ -350,23 +381,12 @@ __device__ __forceinline__ uint32_t tile_setup(const RdvPolicy &pi, TileSmem &s)
             asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(smem_u32(&s.mma_bar[g])) : "memory");
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    {
-        WeightTile<NT, H, RDV_OBS_DIM, H, K0> t0;
-        WeightTile<NT, H, H, H, H> t1;
-        WeightTile<NT, RDV_ACT_DIM, H, N3, H> t2;
-        t0.fetch(pi.w0, pi.b0);
-        t1.fetch(pi.w1, nullptr);
-        t2.fetch(pi.w2, nullptr);
-        const float bias1 = threadIdx.x < H ? __ldg(pi.b1 + threadIdx.x) : 0.0f;
-        const float bias2 = threadIdx.x < RDV_ACT_DIM ? __ldg(pi.b2 + threadIdx.x) : 0.0f;
-        const float lstd = (threadIdx.x < RDV_ACT_DIM && pi.log_std) ? __ldg(pi.log_std + threadIdx.x) : 0.0f;
-        t0.store(TANH_SCALE, s.w0h, s.w0l);
-        t1.store(TANH_SCALE, s.w1h, s.w1l);
-        t2.store(1.0f, s.w2h, s.w2l);
-        if (threadIdx.x < H) s.b1[threadIdx.x] = bias1 * TANH_SCALE;
-        if (threadIdx.x < N3) s.b2[threadIdx.x] = bias2;
-        if (threadIdx.x < 8) s.std[threadIdx.x] = (threadIdx.x < RDV_ACT_DIM && pi.log_std) ? expf(lstd) : 0.0f;
-    }
+}
+// ... and 512 TMEM columns (warp 0), then the fences and a __syncthreads that also publish any weights staged before
+// it.  Returns the TMEM base address.
+template <class S>
+__device__ __forceinline__ uint32_t tile_alloc(S &s)
+{
     if (threadIdx.x < 32) {
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
                      :: "r"(smem_u32(&s.tmem_base)), "r"(TMEM_COLS) : "memory");
@@ -378,6 +398,21 @@ __device__ __forceinline__ uint32_t tile_setup(const RdvPolicy &pi, TileSmem &s)
     tc_fence_after();
     return s.tmem_base;
 }
+// The CTA-wide part alone (mbarriers, TMEM): kernels whose groups stage their own weight sets.
+template <class S>
+__device__ __forceinline__ uint32_t tile_cta_setup(S &s)
+{
+    tile_init_barriers(s);
+    return tile_alloc(s);
+}
+// Whole CTA of NT threads, once per launch: the CTA-wide part around ONE weight set that every group uses.
+template <int NT>
+__device__ __forceinline__ uint32_t tile_setup(const RdvPolicy &pi, TileSmem &s)
+{
+    tile_init_barriers(s);
+    stage_weights<NT>(pi, s.w[0], threadIdx.x);
+    return tile_alloc(s);
+}
 // Whole CTA, after the last tile_forward.
 __device__ __forceinline__ void tile_teardown(uint32_t tmem_all)
 {
@@ -388,14 +423,14 @@ __device__ __forceinline__ void tile_teardown(uint32_t tmem_all)
 }
 
 // One tile through the actor, called by all `threads` threads of group g (thread r owns row r = its TMEM lane).
+// al / bar: the group's lo-activation tile and MMA mbarrier; w: the weight set the group applies.
 // x: the row's 17 observations; out: the actor's mean action, NOT clipped.  `after_issue` runs on the issuing
 // thread right after the layer-1 MMAs are queued (every thread of the group is past its use of shared staging).
 template <class F>
-__device__ __forceinline__ void tile_forward(TileSmem &s, int g, int r, int threads, const float (&x)[RDV_OBS_DIM],
-                                             uint32_t tmem, uint32_t &phase, float (&out)[RDV_ACT_DIM], F &&after_issue)
+__device__ __forceinline__ void tile_forward(elem_t *al, uint64_t *bar, const WeightSet &w, int g, int r, int threads,
+                                             const float (&x)[RDV_OBS_DIM], uint32_t tmem, uint32_t &phase,
+                                             float (&out)[RDV_ACT_DIM], F &&after_issue)
 {
-    elem_t *al = s.al[g];
-    uint64_t *bar = &s.mma_bar[g];
     const uint32_t lane_addr = tmem + ((uint32_t)(r & ~31) << 16);         // this warp's 32 TMEM lanes
     // ---- A0: the observation row and the constant 1 of the bias column, hi -> TMEM, lo -> shared ----
 #if RDV_ACTOR_F16
@@ -450,7 +485,7 @@ __device__ __forceinline__ void tile_forward(TileSmem &s, int g, int r, int thre
     // ---- layer 1 ----
     if (r == 0) {
         tc_fence_after();
-        issue_layer(tmem + A_COL, al, tmem, s.w0h, s.w0l, H, K0 / KSTEP, bar);
+        issue_layer(tmem + A_COL, al, tmem, w.w0h, w.w0l, H, K0 / KSTEP, bar);
         after_issue();
     }
     mbar_wait(bar, phase);
@@ -463,19 +498,19 @@ __device__ __forceinline__ void tile_forward(TileSmem &s, int g, int r, int thre
     // ---- layer 2 (D is reused: the layer-1 epilogue has drained it) ----
     if (r == 0) {
         tc_fence_after();
-        issue_layer(tmem + A_COL, al, tmem, s.w1h, s.w1l, H, H / KSTEP, bar);
+        issue_layer(tmem + A_COL, al, tmem, w.w1h, w.w1l, H, H / KSTEP, bar);
     }
     mbar_wait(bar, phase);
     phase ^= 1;
     tc_fence_after();
-    hidden_epilogue<true>(lane_addr, s.b1, al, r);
+    hidden_epilogue<true>(lane_addr, w.b1, al, r);
     fence_async_smem();
     tc_fence_before();
     group_sync(g, threads);
     // ---- layer 3 ----
     if (r == 0) {
         tc_fence_after();
-        issue_layer(tmem + A_COL, al, tmem, s.w2h, s.w2l, N3, H / KSTEP, bar);
+        issue_layer(tmem + A_COL, al, tmem, w.w2h, w.w2l, N3, H / KSTEP, bar);
     }
     mbar_wait(bar, phase);
     phase ^= 1;
@@ -485,7 +520,7 @@ __device__ __forceinline__ void tile_forward(TileSmem &s, int g, int r, int thre
         tmem_ld16_issue(lane_addr, v);
         tmem_ld_wait(v);
 #pragma unroll
-        for (int j = 0; j < RDV_ACT_DIM; ++j) out[j] = __uint_as_float(v[j]) + s.b2[j];
+        for (int j = 0; j < RDV_ACT_DIM; ++j) out[j] = __uint_as_float(v[j]) + w.b2[j];
     }
     // the next tile's A0 stores and layer-1 MMAs are ordered after these loads by the fences around its first
     // group_sync
@@ -529,7 +564,7 @@ __global__ void __launch_bounds__(GROUPS * TM, 1) policy_tc_kernel(const RdvPoli
 #pragma unroll
             for (int k = 0; k < RDV_OBS_DIM; ++k) x[k] = valid ? obs[env * RDV_OBS_DIM + k] : 0.0f;
         }
-        tile_forward(s.t, g, r, TM, x, tmem, mma_phase, a, [&] {
+        tile_forward(s.t.al[g], &s.t.mma_bar[g], s.t.w[0], g, r, TM, x, tmem, mma_phase, a, [&] {
             // bulk copy of this group's next tile: every thread has consumed the landing zone
             const int64_t next = tile + stride;
             if (bulk_ok && next < tiles && (next + 1) * TM <= n) bulk_load(s.obs[g], obs + next * OBS_TILE, OBS_TILE * 4, obs_bar);

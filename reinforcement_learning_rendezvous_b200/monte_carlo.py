@@ -11,8 +11,10 @@ from __future__ import annotations
 import numpy as np
 import torch
 
+from . import _native as N
 from .batched_env import BatchedRendezvousEnv
 from .environment_utils import config_to_kwargs
+from .policy import PolicyTable
 
 MC_COLS = ("ep_len", "num_collisions", "collided", "total_reward", "total_delta_v", "num_successes", "succeeded",
            "min_dist_from_koz", "pos_error", "vel_error", "att_error", "rot_error")
@@ -108,29 +110,46 @@ def evaluate_batch(policy, initial_states, config=None, reward_kwargs=None, devi
     ``dist_from_koz``, the return and the first-index terminal-error averages of monte_carlo.py:159-189 are
     accumulated in registers until the env's first done.  Returns a dict of length-M arrays with the columns of the
     reference's results workbook.  ``config`` defaults to the evaluator's ``dict(dt=1, t_max=60)`` with
-    ``stochastic=False`` (monte_carlo.py:26-27)."""
+    ``stochastic=False`` (monte_carlo.py:26-27).
+
+    ``policy`` may be a list or tuple of :class:`~.policy.MlpPolicy` (e.g. the checkpoints of a training run, or the models
+    of a sweep): every model then runs all M initial conditions in its own block of envs, padded to a multiple of 128
+    (one tile of the policy table; the padding rows are discarded), still in ONE launch with ONE read-back, and a list
+    with one result dict per model is returned.  Each dict equals what ``evaluate_batch(model, ...)`` returns."""
     ics = np.array(initial_states, dtype=np.float64, copy=True).reshape(-1, 20)
     if normalize_quaternions:                                   # monte_carlo.py:66-67
         ics[:, 6:10] /= np.linalg.norm(ics[:, 6:10], axis=1, keepdims=True)
         ics[:, 13:17] /= np.linalg.norm(ics[:, 13:17], axis=1, keepdims=True)
     m = ics.shape[0]
+    models = list(policy) if isinstance(policy, (list, tuple)) else None
+    block = m
+    if models is not None:
+        policy = PolicyTable(models)
+        block = (m + N.POLICY_TILE - 1) // N.POLICY_TILE * N.POLICY_TILE
+        # the reset state of the evaluator's config does not depend on the env id (zero ranges), so the last row
+        # repeated is a valid padding state
+        ics = np.tile(np.concatenate([ics, np.repeat(ics[-1:], block - m, axis=0)]), (len(models), 1))
     kw = config_to_kwargs(dict(dt=1, t_max=60) if config is None else config, stochastic=False)
-    env = BatchedRendezvousEnv(m, device=device, auto_reset=False, track_stats=False, reward_kwargs=reward_kwargs,
-                               **kw, **extra)
+    env = BatchedRendezvousEnv(ics.shape[0], device=device, auto_reset=False, track_stats=False,
+                               reward_kwargs=reward_kwargs, **kw, **extra)
     p = env.params
     env.reset()
     env.set_state(ics, reset_counters=False)        # flags stay as reset() left them (monte_carlo.py:106-112)
-    out = env.rollout(int(p.done_steps), policy=policy, monte_carlo=True)
-    mc = out["mc"].cpu().numpy()                    # the one read-back: [M, MC_NCOL]
-    res = mc_columns(mc, p.dt)
-    if return_raw:
-        res["raw"] = mc
-    return res
+    tiles = None if models is None else np.repeat(np.arange(len(models)), block // N.POLICY_TILE)
+    out = env.rollout(int(p.done_steps), policy=policy, monte_carlo=True, policy_tiles=tiles)
+    mc = out["mc"].cpu().numpy()                    # the one read-back: [M, MC_NCOL] (models x block with a list)
+    results = []
+    for b in range(1 if models is None else len(models)):
+        raw = mc[b * block:b * block + m]
+        res = mc_columns(raw, p.dt)
+        if return_raw:
+            res["raw"] = raw
+        results.append(res)
+    return results[0] if models is None else results
 
 
 def mc_columns(mc: np.ndarray, dt: float) -> dict:
     """[M, MC_NCOL] device results -> the workbook columns (monte_carlo.py:190-203): seconds and degrees."""
-    from . import _native as N
     return dict(
         ep_len=np.round(mc[:, N.MC_EP_LEN] * dt, 3), num_collisions=mc[:, N.MC_NUM_COLLISIONS].astype(np.int64),
         collided=mc[:, N.MC_COLLIDED].astype(np.int64), total_reward=mc[:, N.MC_TOTAL_REWARD].copy(),
@@ -164,15 +183,28 @@ def evaluate_sweep(policy, param_sets, episodes_per_set=1024, reward_kwargs=None
     first episode of every env is scored on the device).  With ``world_size`` > 1 the parameter sets are sharded over
     ranks by :func:`~.distributed.shard_range` (every rank returns its own sets; reset streams are keyed by the
     global env id, so a set's result does not depend on the sharding).  Returns one dict per set: mean return /
-    length, success and collision rates (the metrics of custom_callbacks.py:285-298)."""
-    from . import _native as N
+    length, success and collision rates (the metrics of custom_callbacks.py:285-298).
+
+    ``policy`` may be a list or tuple of :class:`~.policy.MlpPolicy`, as long as ``param_sets``: set i is then scored with
+    model i (sensitivity_analysis.py trains one model per set), all sets still in one launch through a policy table.
+    The list is global, sharded with the sets; ``episodes_per_set`` must then be a multiple of 128 (one table tile)."""
     from .distributed import shard_range
+    models = list(policy) if isinstance(policy, (list, tuple)) else None
+    if models is not None:
+        if len(models) != len(param_sets):
+            raise ValueError(f"{len(models)} policies for {len(param_sets)} parameter sets")
+        if episodes_per_set % N.POLICY_TILE:
+            raise ValueError(f"episodes_per_set must be a multiple of {N.POLICY_TILE} with one policy per set")
     if episodes_per_set % 32:
         raise ValueError("episodes_per_set must be a multiple of 32")
     lo_set, hi_set = shard_range(len(param_sets), world_size, rank)
     mine = list(param_sets[lo_set:hi_set])
     if not mine:
         return []
+    tiles = None
+    if models is not None:
+        policy = PolicyTable(models[lo_set:hi_set])
+        tiles = np.repeat(np.arange(len(mine)), episodes_per_set // N.POLICY_TILE)
     batches = []
     for ps in mine:
         kw = config_to_kwargs(dict(common, **ps), stochastic=True)
@@ -182,7 +214,7 @@ def evaluate_sweep(policy, param_sets, episodes_per_set=1024, reward_kwargs=None
                                track_stats=False, reward_kwargs=reward_kwargs, param_batches=batches)
     env.reset()
     steps = max(int(g.params.done_steps) for g in env.groups)
-    mc = env.rollout(steps, policy=policy, monte_carlo=True)["mc"]
+    mc = env.rollout(steps, policy=policy, monte_carlo=True, policy_tiles=tiles)["mc"]
     res = torch.stack([mc[:, N.MC_TOTAL_REWARD], mc[:, N.MC_EP_LEN], (env.success > 0).double(),
                        (env.collided > 0).double()], dim=1).cpu().numpy()        # flags are frozen at the first done
     out = []

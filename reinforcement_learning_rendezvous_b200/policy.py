@@ -99,3 +99,38 @@ class MlpPolicy:
         torch.cuda.current_stream(self.device).synchronize()
         act = self._h_act.numpy().copy()
         return (act[0] if single else act), state
+
+
+class PolicyTable:
+    """Several :class:`MlpPolicy` actors for ONE fused rollout (``BatchedRendezvousEnv.rollout(policy=table,
+    policy_tiles=...)``): entry ``e`` acts for every tile of 128 consecutive envs whose index in ``policy_tiles`` is
+    ``e`` (``RdvRolloutIO.policy_table``).  Holds the entries' ``RdvPolicy`` structs as a device ``uint8`` tensor and
+    keeps the policies (which own the weights the structs point to) alive.  Every entry must live on one device and
+    have the 64-wide actor the fused kernel is built for."""
+
+    def __init__(self, policies):
+        policies = list(policies)
+        if not policies:
+            raise ValueError("a policy table needs at least one policy")
+        if not all(isinstance(p, MlpPolicy) for p in policies):
+            raise TypeError("policy table entries must be MlpPolicy objects")
+        if any(p.device != policies[0].device for p in policies):
+            raise ValueError("policy table entries live on different devices")
+        if any(p.hidden != 64 for p in policies):
+            raise ValueError("the fused actor needs hidden width 64 for every entry")
+        self.policies = policies
+        self.device = policies[0].device
+        self.table = torch.frombuffer(bytearray(self.pack([p._c for p in policies])), dtype=torch.uint8).to(self.device)
+
+    @staticmethod
+    def pack(structs) -> bytes:
+        """``RdvPolicy`` structs -> the bytes of a C array ``RdvPolicy[len(structs)]``."""
+        return b"".join(bytes(s) for s in structs)
+
+    def __len__(self):
+        return len(self.policies)
+
+    @property
+    def stochastic_ready(self) -> bool:
+        """Every entry has the Gaussian head's ``log_std`` (needed for sampling rollouts)."""
+        return all(p.log_std is not None for p in self.policies)
