@@ -108,17 +108,12 @@ RDV_DEV int pair_swap(int v) { return __shfl_xor_sync(0xffffffffu, v, 1); }
 // ~20 doubles per step through warp shuffles.  Finished envs are appended to reset_list (count in
 // reset_list[0]) for the compacted reset kernel below, so the rare reset path never diverges a stepping warp.
 // ---------------------------------------------------------------------------------
-#ifndef RDV_STEP_MIN_CTAS
-#define RDV_STEP_MIN_CTAS 4          // 4 CTAs x 4 warps = 16 resident warps per SM at <= 128 registers
-#endif
-#ifndef RDV_EPB
-#define RDV_EPB 64
-#endif
-constexpr int EPB = RDV_EPB;        // environments per CTA
+constexpr int STEP_MIN_CTAS = 4;    // 4 CTAs x 4 warps = 16 resident warps per SM at <= 128 registers
+constexpr int EPB = 64;             // environments per CTA
 constexpr int TPB = 2 * EPB;        // threads per CTA
 
 template <bool ISO, bool ACT_F64, bool CLOSED, bool TABLE = false>
-__global__ void __launch_bounds__(TPB, RDV_STEP_MIN_CTAS) step_kernel(const __grid_constant__ RdvParams Pc, const RdvState S,
+__global__ void __launch_bounds__(TPB, STEP_MIN_CTAS) step_kernel(const __grid_constant__ RdvParams Pc, const RdvState S,
                                                       const RdvStepIO io, const int64_t n, const uint64_t seed,
                                                       const int64_t env_offset)
 {
@@ -449,7 +444,7 @@ __global__ void __launch_bounds__(TPB, RDV_STEP_MIN_CTAS) step_kernel(const __gr
 // ---------------------------------------------------------------------------------
 // Launch shape: ONE CTA per SM, every CTA owns an equal contiguous slice of the batch and walks it in
 // passes of at most TPB environments, all K steps of a pass before the next pass.  The CTA's warps re-converge
-// at a barrier every RDV_SYNC_PERIOD steps: the step is tens of KB of straight-line code, and warps that drift far
+// at a barrier every SYNC_PERIOD steps: the step is tens of KB of straight-line code, and warps that drift far
 // apart thrash the instruction cache (measured with the first, ~60 KB step: 58 % hit rate and 3.1 of 6.2 stall
 // cycles per instruction on "no instruction" with four independent 64-thread CTAs per SM; in-phase warps ran the
 // same workload 1.7x faster).
@@ -460,24 +455,10 @@ __global__ void __launch_bounds__(TPB, RDV_STEP_MIN_CTAS) step_kernel(const __gr
 // RdvRolloutIO.policy_table chosen by policy_tile.  Slices are cut at multiples of 128 envs and passes are 256 envs,
 // so each group's tile is 128 envs starting at a multiple of 128 from env 0 of the launch; each group stages its
 // entry's weights into its own weight set (TableSmem) when the entry differs from the one it holds.
-#ifndef RDV_SYNC_PERIOD
-#define RDV_SYNC_PERIOD 8             /* steps between the CTA barriers that keep the warps in one code region */
-#endif
-#ifndef RDV_HELP_POST_PERIOD
-#define RDV_HELP_POST_PERIOD 3        /* helper-warp variant: steps between the workers' request posts (1: 12 % slower, 2-4 alike) */
-#endif
-#ifndef RDV_HELP_IDLE_NS
-#define RDV_HELP_IDLE_NS 500          /* helper-warp variant: sleep of an idle helper between polls */
-#endif
-#ifndef RDV_TMEM_STASH
-#define RDV_TMEM_STASH 1              /* fused actor: park the cold per-env registers in tensor memory across the solves */
-#endif
-#ifndef RDV_TMEM_STASH_MAIN
-#define RDV_TMEM_STASH_MAIN 1         /* the same for the variants without the actor (they then allocate the TMEM) */
-#endif
-#ifndef RDV_LOCKSTEP_MAX_TPB
-#define RDV_LOCKSTEP_MAX_TPB 256      /* CTAs up to this size interleave the two attitude solves (rk45_iso_plane_pair) */
-#endif
+constexpr int SYNC_PERIOD = 8;            // steps between the CTA barriers that keep the warps in one code region
+constexpr int HELP_POST_PERIOD = 3;       // helper-warp variant: steps between the workers' request posts (1: 12 % slower, 2-4 alike)
+constexpr int HELP_IDLE_NS = 500;         // helper-warp variant: sleep of an idle helper between polls
+constexpr int LOCKSTEP_MAX_TPB = 256;     // CTAs up to this size interleave the two attitude solves (rk45_iso_plane_pair)
 constexpr int RDV_NEXT_ROW = 22;          // doubles per prefetched reset row: state[20], collided, success
 constexpr int RDV_ROW_TAG = 22;           // row of RdvRolloutIO.reset_rows holding the episode index a row belongs to
 
@@ -525,7 +506,7 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
     }
     // Without the actor the tensor memory (256 KB per SM) is entirely idle; the variant for the reference's bodies
     // allocates it as a parking area for cold registers (see the step phase): 128 columns for every thread.
-    constexpr bool main_stash = !POLICY && !MC && ISO && !CLOSED && (RDV_TMEM_STASH_MAIN != 0);
+    constexpr bool main_stash = !POLICY && !MC && ISO && !CLOSED;
     __shared__ uint32_t s_tmem_base;
     if constexpr (main_stash) {
         if (threadIdx.x < 32) {
@@ -652,7 +633,7 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
                     if (lane == 0) *(volatile int *)&s_inflight[h] = 0;
                 }
                 if (*(volatile int *)&s_ndone >= NW) break;
-                if (!worked) __nanosleep(RDV_HELP_IDLE_NS);
+                if (!worked) __nanosleep(HELP_IDLE_NS);
             }
         }
     }
@@ -697,7 +678,7 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
         float ov[RDV_OBS_DIM];
         if (want_obs) make_obs(e, obs_scale(P), ov);
         unsigned fresh = 0;                                    // lanes whose next reset row is ready
-        int countdown = HELP ? RDV_HELP_POST_PERIOD : refill;  // steps until the next refill of the rows (HELP: next post)
+        int countdown = HELP ? HELP_POST_PERIOD : refill;      // steps until the next refill of the rows (HELP: next post)
         // where this lane's row lives
         double *my_row = POLICY ? io.reset_rows + i : next_rows + lane * RDV_NEXT_ROW;
         const int64_t row_stride = POLICY ? ld : 1;
@@ -814,7 +795,7 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
                 // evaluator mode: an env stops at its first done (its lanes idle from then on)
                 r.rew = 0.0; r.done = 0; r.reason = -1;
                 if (alive) {
-                    env_advance<ISO, CLOSED, (TPB_ <= RDV_LOCKSTEP_MAX_TPB)>(P, e, t, rk_acc, rk_rej, fail);
+                    env_advance<ISO, CLOSED, (TPB_ <= LOCKSTEP_MAX_TPB)>(P, e, t, rk_acc, rk_rej, fail);
                     EvalDetail d;
                     r = env_evaluate<true, true>(P, e, t.fuel, c, ov, &d);
                     mc_sample(P, d, c.collided, mc);                          // monte_carlo.py:140-149
@@ -822,7 +803,7 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
                     mc.len += 1;
                     if (r.done) { alive = false; mc_reason = r.reason; }
                 }
-            } else if constexpr ((POLICY && RDV_TMEM_STASH) || main_stash) {
+            } else if constexpr (POLICY || main_stash) {
                 // The fused actor owns 196 KiB of shared memory, which leaves 60 KiB of L1 for 136 KB of register
                 // spills (local loads hit 58 %, and the misses cost an L2 round trip: 22 % of this variant's issue
                 // latency were long-scoreboard stalls).  During the env step the group's tensor memory is idle -- D and
@@ -855,7 +836,7 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
                     tc::tmem_st_wait();
                 }
                 // (parking, in addition, the body that is not being propagated around each solve measured no faster)
-                env_attitude<ISO, CLOSED, (TPB_ <= RDV_LOCKSTEP_MAX_TPB)>(P, e, t, rk_acc, rk_rej, fail);
+                env_attitude<ISO, CLOSED, (TPB_ <= LOCKSTEP_MAX_TPB)>(P, e, t, rk_acc, rk_rej, fail);
                 {
                     uint32_t w[48];
                     tc::tmem_ld16_issue(lane_addr, reinterpret_cast<uint32_t (&)[16]>(w[0]));
@@ -877,7 +858,7 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
                 }
                 r = env_evaluate<want_obs>(P, e, t.fuel, c, ov);
             } else {
-                env_advance<ISO, CLOSED, (TPB_ <= RDV_LOCKSTEP_MAX_TPB)>(P, e, t, rk_acc, rk_rej, fail);
+                env_advance<ISO, CLOSED, (TPB_ <= LOCKSTEP_MAX_TPB)>(P, e, t, rk_acc, rk_rej, fail);
                 r = env_evaluate<want_obs>(P, e, t.fuel, c, ov);
             }
             const bool done = r.done && active;
@@ -920,7 +901,7 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
                     }
                 }
                 if (--countdown <= 0) {
-                    countdown = RDV_HELP_POST_PERIOD;
+                    countdown = HELP_POST_PERIOD;
                     post_requests();
                 }
             } else if (!MC && io.auto_reset && refill) {
@@ -992,12 +973,10 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
                 // step a barrier every step was best (every 2 / 4 steps: 1 % / 8 % slower); the plane solver's step is
                 // smaller and tolerates drift: every step 12.06, every 4-8 steps 11.66, every 32 steps 11.77, never
                 // 12.1-12.2 us per step.
-#if RDV_SYNC_PERIOD >= 1
-                if ((k % RDV_SYNC_PERIOD) == 0) {
+                if ((k % SYNC_PERIOD) == 0) {
                     if constexpr (HELP) asm volatile("bar.sync 2, %0;" :: "n"(TPB_) : "memory");   // the workers only
                     else __syncthreads();
                 }
-#endif
                 // ---- action ----
                 const int64_t row = (int64_t)k * n + i;
                 if (src == RDV_ACTIONS_F32) {
@@ -1323,16 +1302,13 @@ static bool ensure_smem(K kernel, std::atomic<uint64_t> &mask, int dev, size_t b
 // The fill runs on the caller's stream and is waited for (once per device and process), so that launches on other
 // streams find it complete; a stream that is being captured into a graph cannot be waited for -- the first call on a
 // device has to come from outside a capture (any reset / step / rollout does).
-#if RDV_ACOS_TABLE
 __global__ void acos_table_kernel()
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i <= 2 * ACOS_TABLE_HALF) g_acos_table[i] = acos_of_rounded((double)(i - ACOS_TABLE_HALF));
 }
-#endif
 static bool ensure_tables(cudaStream_t st)
 {
-#if RDV_ACOS_TABLE
     static std::atomic<uint64_t> mask{0};
     static std::mutex mtx;
     int dev = 0;
@@ -1346,9 +1322,6 @@ static bool ensure_tables(cudaStream_t st)
     acos_table_kernel<<<(2 * ACOS_TABLE_HALF + 256) / 256, 256, 0, st>>>();
     if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) return false;
     mask.fetch_or(bit, std::memory_order_release);
-#else
-    (void)st;
-#endif
     return true;
 }
 

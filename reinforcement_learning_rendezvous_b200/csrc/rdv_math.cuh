@@ -112,23 +112,6 @@ RDV_DEV void rot_apply_T(const Rot &R, const double v[3], double o[3])          
     for (int i = 0; i < 3; ++i) o[i] = fma(R.m[6 + i], v[2], fma(R.m[3 + i], v[1], R.m[i] * v[0]));
 }
 
-// R(q / |q|) v for ONE vector without forming the matrix: v + 2 w (u x v) + 2 u x (u x v) with q / |q| = (w, u) --
-// 32 fp64 operations against 48 for quat2mat (including its re-normalisation) plus one matrix-vector product.
-// Same rotation as rot_apply(rot_from_quat(q), v) to rounding.
-#ifndef RDV_QUAT_ROTATE
-#define RDV_QUAT_ROTATE 0
-#endif
-RDV_DEV void quat_rotate(const double q[4], const double v[3], double o[3])
-{
-    const double r = fast_rsqrt(dot4(q, q));
-    const double w = q[0] * r, u[3] = {q[1] * r, q[2] * r, q[3] * r};
-    double c[3], d[3];
-    cross3(u, v, c);
-    cross3(u, c, d);
-#pragma unroll
-    for (int i = 0; i < 3; ++i) o[i] = fma(2.0, fma(w, c[i], d[i]), v[i]);
-}
-
 // sqrt(x) for x >= 0 (<= 1 ulp): x * rsqrt(x)
 RDV_DEV double fast_sqrt(double x) { return x > 0.0 ? x * fast_rsqrt(x) : 0.0; }
 
@@ -143,33 +126,14 @@ RDV_DEV double acos_of_rounded(double k)
 // The rounded cosine takes only 200,001 values, so the angle is a table look-up (1.6 MB, resident in the L2): one
 // load instead of the ~85 instructions of acos().  The table is filled by acos_table_kernel with acos_of_rounded
 // itself, once per device, before the first kernel that reads it (ensure_tables in rdv_b200.cu).
-#ifndef RDV_ACOS_TABLE
-#define RDV_ACOS_TABLE 1
-#endif
-#ifndef RDV_TABLE_INT_INDEX
-#define RDV_TABLE_INT_INDEX 0
-#endif
 constexpr int ACOS_TABLE_HALF = 100000;
-#if RDV_ACOS_TABLE
 __device__ double g_acos_table[2 * ACOS_TABLE_HALF + 1];
-#endif
 RDV_DEV double rounded_angle_from(double dot, double n1sq, double n2sq)
 {
     const double c = dot * fast_rsqrt(n1sq * n2sq);
-#if RDV_ACOS_TABLE && RDV_TABLE_INT_INDEX
-    // round-to-nearest-even conversion = rint for every value in range; huge values saturate outside the unsigned
-    // range test; NaN (a zero vector) converts to 0 and is sent to the library path by the second test
-    const int ki = __double2int_rn(c * 1e5);
-    if ((unsigned)(ki + ACOS_TABLE_HALF) <= 2u * ACOS_TABLE_HALF && (ki != 0 || c == c))
-        return g_acos_table[ki + ACOS_TABLE_HALF];
-    return acos_of_rounded(rint(c * 1e5));
-#else
     const double k = rint(c * 1e5);
-#if RDV_ACOS_TABLE
     if (fabs(k) <= (double)ACOS_TABLE_HALF) return g_acos_table[(int)k + ACOS_TABLE_HALF];
-#endif
     return acos_of_rounded(k);                       // NaN (a zero vector) or out of range: the library's answer
-#endif
 }
 
 // ---------------------------------------------------------------------------------
@@ -209,10 +173,6 @@ RDV_DEV void attitude_rhs(const double *y, const double *hw_iso, const BodyConst
 
 // Dormand-Prince tableau (scipy rk.py, class RK45).  Kept in the constant bank so that DFMA reads each
 // coefficient as a c[][] operand instead of materialising a 64-bit immediate with two moves per use.
-#ifndef RDV_RK_CONST_BANK
-#define RDV_RK_CONST_BANK 1
-#endif
-#if RDV_RK_CONST_BANK
 __constant__ double c_rk[26] = {
     1.0 / 5,
     3.0 / 40,
@@ -267,34 +227,6 @@ __constant__ double c_rk[26] = {
 #define RK_E5 c_rk[23]
 #define RK_E6 c_rk[24]
 #define RK_E7 c_rk[25]
-#else
-#define RK_A21 (1.0 / 5)
-#define RK_A31 (3.0 / 40)
-#define RK_A32 (9.0 / 40)
-#define RK_A41 (44.0 / 45)
-#define RK_A42 (-56.0 / 15)
-#define RK_A43 (32.0 / 9)
-#define RK_A51 (19372.0 / 6561)
-#define RK_A52 (-25360.0 / 2187)
-#define RK_A53 (64448.0 / 6561)
-#define RK_A54 (-212.0 / 729)
-#define RK_A61 (9017.0 / 3168)
-#define RK_A62 (-355.0 / 33)
-#define RK_A63 (46732.0 / 5247)
-#define RK_A64 (49.0 / 176)
-#define RK_A65 (-5103.0 / 18656)
-#define RK_B1 (35.0 / 384)
-#define RK_B3 (500.0 / 1113)
-#define RK_B4 (125.0 / 192)
-#define RK_B5 (-2187.0 / 6784)
-#define RK_B6 (11.0 / 84)
-#define RK_E1 (-71.0 / 57600)
-#define RK_E3 (71.0 / 16695)
-#define RK_E4 (-71.0 / 1920)
-#define RK_E5 (17253.0 / 339200)
-#define RK_E6 (-22.0 / 525)
-#define RK_E7 (1.0 / 40)
-#endif
 #define RK_RTOL 1e-7     /* rendezvous_env.py:567, :594 */
 #define RK_ATOL 1e-6     /* rendezvous_env.py:568, :595 */
 
@@ -304,11 +236,8 @@ __constant__ double c_rk[26] = {
 // branch (ivp.py:710-728) evaluates the dense-output polynomial at x == 1, which equals y_new
 // up to ~1 ulp; y_new is used.  Returns accepted steps, or -1 on TOO_SMALL_STEP / non-finite
 // error norm (the reference raises there); y is left at the last accepted state.
-#ifndef RDV_CTRL_F32
-#define RDV_CTRL_F32 1
-#endif
 // ---------------------------------------------------------------------------------
-// Step-size controller arithmetic in float32 (RDV_CTRL_F32).
+// Step-size controller arithmetic in float32.
 //
 // The error norm, the scale vector, the step factor 0.9 err^-0.2 and select_initial_step only steer the
 // step size; the propagated state never sees them except through h.  One accepted step changes by
@@ -326,16 +255,8 @@ RDV_DEV float lg2_f32(float x) { float r; asm("lg2.approx.ftz.f32 %0, %1;" : "=f
 RDV_DEV float ex2_f32(float x) { float r; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
 RDV_DEV float pow_neg_tenth_f32(float x) { return ex2_f32(-0.1f * lg2_f32(x)); }
 
-#ifndef RDV_RK_INLINE
-#define RDV_RK_INLINE 1
-#endif
-#if RDV_RK_INLINE
-#define RDV_RK_FN RDV_DEV
-#else
-#define RDV_RK_FN __device__ __noinline__
-#endif
 template <bool ISO>
-RDV_RK_FN int rk45_attitude(double (&y)[7], const double dt, const BodyConst &b, int &n_rejected)
+RDV_DEV int rk45_attitude(double (&y)[7], const double dt, const BodyConst &b, int &n_rejected)
 {
     constexpr int NA = ISO ? 4 : 7;         // components with a non-zero derivative
     double hw[3] = {0.5 * y[4], 0.5 * y[5], 0.5 * y[6]};
@@ -344,7 +265,6 @@ RDV_RK_FN int rk45_attitude(double (&y)[7], const double dt, const BodyConst &b,
 
     // ---- select_initial_step (order 4) ----
     double h_abs;
-#if RDV_CTRL_F32
     {
         float inv_sc[7], d0s = 0.0f, d1s = 0.0f;
 #pragma unroll
@@ -384,46 +304,6 @@ RDV_RK_FN int rk45_attitude(double (&y)[7], const double dt, const BodyConst &b,
         else h1 = pow_neg_tenth_f32(fminf(fmaxf(d1s, d2s), 1e30f) * 1e4f);   // (0.01/max(d1,d2))**(1/5)
         h_abs = fmin(fmin(100.0 * h0, (double)h1), dt);
     }
-#else
-    {
-        double inv_sc[7], d0s = 0.0, d1s = 0.0;
-#pragma unroll
-        for (int i = 0; i < 7; ++i) {
-            inv_sc[i] = fast_rcp(fma(fabs(y[i]), RK_RTOL, RK_ATOL));
-            double a = y[i] * inv_sc[i];
-            d0s = fma(a, a, d0s);
-        }
-#pragma unroll
-        for (int i = 0; i < NA; ++i) {
-            double a = K[0][i] * inv_sc[i];
-            d1s = fma(a, a, d1s);
-        }
-        d0s *= (1.0 / 7.0);
-        d1s *= (1.0 / 7.0);                                  // squares of the rms norms d0, d1
-        double h0;
-        if (d0s < 1e-10 || d1s < 1e-10) h0 = 1e-6;
-        else h0 = 0.01 * sqrt(d0s * fast_rcp(d1s));
-        h0 = fmin(h0, dt);
-        double y1[7], f1[NA];
-#pragma unroll
-        for (int i = 0; i < NA; ++i) y1[i] = fma(h0, K[0][i], y[i]);
-#pragma unroll
-        for (int i = NA; i < 7; ++i) y1[i] = y[i];
-        attitude_rhs<ISO>(y1, hw, b, f1);
-        double d2s = 0.0;
-#pragma unroll
-        for (int i = 0; i < NA; ++i) {
-            double a = (f1[i] - K[0][i]) * inv_sc[i];
-            d2s = fma(a, a, d2s);
-        }
-        double inv_h0 = fast_rcp(h0);
-        d2s = d2s * (1.0 / 7.0) * inv_h0 * inv_h0;
-        double h1;
-        if (d1s <= 1e-30 && d2s <= 1e-30) h1 = fmax(1e-6, h0 * 1e-3);
-        else h1 = pow_neg_tenth(fmax(d1s, d2s) * 1e4);        // (0.01/max(d1,d2))**(1/5)
-        h_abs = fmin(fmin(100.0 * h0, h1), dt);
-    }
-#endif
 
     double t = 0.0;
     int accepted = 0;
@@ -480,7 +360,6 @@ RDV_RK_FN int rk45_attitude(double (&y)[7], const double dt, const BodyConst &b,
                 eh[i] = h * fma(K[6][i], RK_E7,
                                 fma(K[5][i], RK_E6,
                                     fma(K[4][i], RK_E5, fma(K[3][i], RK_E4, fma(K[2][i], RK_E3, K[0][i] * RK_E1)))));
-#if RDV_CTRL_F32
             float esf = 0.0f;
 #pragma unroll
             for (int i = 0; i < NA; ++i) {
@@ -511,26 +390,6 @@ RDV_RK_FN int rk45_attitude(double (&y)[7], const double dt, const BodyConst &b,
             h_abs *= (double)fmaxf(0.2f, p);
             rejected = true;
             ++n_rejected;
-#else
-            double es = 0.0;
-#pragma unroll
-            for (int i = 0; i < NA; ++i) {
-                const double e = eh[i] * fast_rcp(fma(fmax(fabs(y[i]), fabs(y_new[i])), RK_RTOL, RK_ATOL));
-                es = fma(e, e, es);
-            }
-            es *= (1.0 / 7.0);                         // err_norm^2
-            if (!(es < 1.0e300)) return -1;            // NaN / inf: the reference shrinks h to failure
-            if (es < 1.0) {
-                // factor = min(10, 0.9 err^-0.2); err^-0.2 >= 10/0.9 whenever err^2 <= 3.5e-11
-                double factor = (es < 3.0e-11) ? 10.0 : fmin(10.0, 0.9 * pow_neg_tenth(es));
-                if (rejected) factor = fmin(1.0, factor);
-                h_abs *= factor;
-                break;
-            }
-            h_abs *= (es > 1.0e7) ? 0.2 : fmax(0.2, 0.9 * pow_neg_tenth(es));
-            rejected = true;
-            ++n_rejected;
-#endif
         }
         ++accepted;
         t = t_new;
@@ -573,7 +432,7 @@ RDV_DEV void rhs_plane(const double a, const double b, const double om2, double 
 RDV_DEV double plane_g(const double a, const double b, const double om2) { return fast_rsqrt(fma(om2 * b, b, a * a)); }
 
 // ---------------------------------------------------------------------------------
-// One attempted step in closed form (RDV_PLANE_POLY).
+// One attempted step in closed form.
 //
 // With z = a + i w b, w^2 = om2, the plane equation is z' = i w z / |z|: rotation-equivariant and homogeneous of
 // degree 0.  Every stage of one Dormand-Prince attempt from z with step h is therefore z times a function of
@@ -597,10 +456,8 @@ RDV_DEV double plane_g(const double a, const double b, const double om2) { retur
 // step (4e-10 s), i.e. by < 1e-10 over a whole solve (sum of s <= sqrt(om2) dt).  So om2 dt^2 (1 + 2^-20) <= X_MAX
 // keeps every attempt of the solve inside the fitted range; the 2^-20 also covers the rounding of om2 and x.  Faster
 // spins (om2 dt^2 > X_MAX ~ |w| dt > 0.35 rad) take the stagewise attempt for the whole solve, out of line.
+// Measured (B200): 9.72 -> 9.30 us per step (20-step launches), 8.86 -> 8.65 (250-step).
 // ---------------------------------------------------------------------------------
-#ifndef RDV_PLANE_POLY
-#define RDV_PLANE_POLY 1         /* measured (B200): 9.72 -> 9.30 us per step (20-step launches), 8.86 -> 8.65 (250-step) */
-#endif
 constexpr int PP_P1 = 0, PP_Q1 = PP_P1 + RDV_PP_N_P1, PP_R = PP_Q1 + RDV_PP_N_Q1, PP_I = PP_R + RDV_PP_N_R;
 __constant__ double c_pp[PP_I + RDV_PP_N_I] = {RDV_PP_P1, RDV_PP_Q1, RDV_PP_R, RDV_PP_I};
 
@@ -673,7 +530,7 @@ RDV_DEV void plane_attempt(const double a, const double b, const double g, const
     }
 }
 
-// What the controller sees of one attempted step, in float32 (RDV_CTRL_F32 rationale above): the candidate state
+// What the controller sees of one attempted step, in float32 (rationale at rk45_attitude): the candidate state
 // y_new = a_new q0 + b_new p and the error estimate e = ea q0 + eb p in quaternion components, and
 // err^2 = mean((e_i / (atol + rtol max(|y_i|, |y_new,i|)))^2) over the reference's seven components (the three
 // rate components contribute 0).  q0 is orthogonal to p, so sum e_i^2 = ea^2 |q0|^2 + eb^2 |p|^2 and cancellation
@@ -708,17 +565,15 @@ RDV_DEV double plane_err2_f64(const double ea, const double eb, const double a, 
 }
 // select_initial_step (scipy common.py:68-134, order 4).  The first slope at (a, b) = (1, 0) is (0, 1) exactly:
 // f0 = M q0 / |q0| = p.
-#ifndef RDV_INIT_LAZY_D0
-#define RDV_INIT_LAZY_D0 1      /* measured: 10.12 -> 9.93 us per step (20-step launches), 9.33 -> 9.12 (250-step) */
-#endif
-#ifndef RDV_INIT_NOSQRT
-#define RDV_INIT_NOSQRT 1       /* measured: 9.94 -> 9.76 us per step (20-step launches), 9.13 -> 8.94 (250-step) */
-#endif
-#if RDV_INIT_LAZY_D0
-// Same result, less work in the common case.  The returned value is min(100 h0, h1, dt) with 100 h0 = d0 / d1, and
-// d0 only grows when the three rate components join its norm: whenever the quaternion part alone already puts
-// 100 h0 above min(h1, dt) -- always, unless a body spins at several rad/s -- the rate part of d0 is never formed.
-// The bound that lets the second slope go (below) is taken with h0 <= dt instead of h0 itself, which needs d0 too.
+// d2 = rms((f(y0 + h0 f0) - f0) / scale) / h0 only enters through max(d1, d2).  In plane coordinates
+// f1 - f0 = da q0 + db p with |da| <= om2 h0 and |db| <= om2 h0^2 / 2, hence d2 <= om2 (rms(q0 / scale) + h0 d1 / 2):
+// of the order omega d1, i.e. below d1 unless the body spins at ~1 rad/s.  When this bound (with 5 % slack for the
+// float32 arithmetic) is below d1 the second slope is not evaluated at all; otherwise d2 is formed exactly as scipy does.
+// The returned value is min(100 h0, h1, dt) with 100 h0 = d0 / d1, and d0 only grows when the three rate components
+// join its norm: whenever the quaternion part alone already puts 100 h0 above min(h1, dt) -- always, unless a body
+// spins at several rad/s -- the rate part of d0 is never formed.  The bound that lets the second slope go is then
+// taken with h0 <= dt instead of h0 itself, which needs d0 too (measured against forming d0 first: 10.12 -> 9.93 us
+// per step in 20-step launches, 9.33 -> 9.12 in 250-step ones).
 RDV_DEV double plane_initial_step(const double (&y)[7], const float (&q0f)[4], const float (&pf)[4], const double om2,
                                   const double dt)
 {
@@ -733,15 +588,11 @@ RDV_DEV double plane_initial_step(const double (&y)[7], const float (&q0f)[4], c
     const float d0q = d0r * (1.0f / 7.0f);                                       // the quaternion part of d0^2
     d1s *= (1.0f / 7.0f);
     const float dtf = (float)dt;
-#if RDV_INIT_NOSQRT
     // d2 <= om2 (sqrt(d0q) + dt sqrt(d1s) / 2) with h0 <= dt; "bound^2 * 1.05 <= d1s" without a square root:
     // om2 sqrt(d0q) <= sqrt(d1s) (0.975 - om2 dt / 2), both sides non-negative, squared
+    // (measured against the two square roots: 9.94 -> 9.76 us per step in 20-step launches, 9.13 -> 8.94 in 250-step)
     const float om2f = (float)om2, room = fmaf(-0.5f * dtf, om2f, 0.975f);
     const bool d2_small = room > 0.0f && om2f * om2f * d0q <= d1s * room * room;
-#else
-    const float ub = (float)om2 * fmaf(0.5f * dtf, sqrtf(d1s), sqrtf(d0q));      // bound on d2 with h0 <= dt
-    const bool d2_small = ub * ub * 1.05f <= d1s;
-#endif
     if (d0q >= 1e-10f && d1s >= 1e-10f && d2_small) {
         // common case: d2 <= d1, so h1 = (0.01 / d1)^(1/5); and 100 h0 >= sqrt(d0q / d1s) (or 100 dt)
         const float h1 = pow_neg_tenth_f32(fminf(d1s, 1e30f) * 1e4f);
@@ -783,59 +634,6 @@ RDV_DEV double plane_initial_step(const double (&y)[7], const float (&q0f)[4], c
     else h1 = pow_neg_tenth_f32(fminf(dmax, 1e30f) * 1e4f);  // (0.01/max(d1,d2))**(1/5)
     return fmin(fmin(100.0 * h0, (double)h1), dt);
 }
-#else
-RDV_DEV double plane_initial_step(const double (&y)[7], const float (&q0f)[4], const float (&pf)[4], const double om2,
-                                  const double dt)
-{
-    float inv_sc[4], d0s = 0.0f, d1s = 0.0f;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        inv_sc[i] = rcp_f32(fmaf(fabsf(q0f[i]), (float)RK_RTOL, (float)RK_ATOL));
-        const float v = q0f[i] * inv_sc[i], f = pf[i] * inv_sc[i];               // y0 / scale, f0 / scale
-        d0s = fmaf(v, v, d0s);
-        d1s = fmaf(f, f, d1s);
-    }
-    const float d0q = d0s * (1.0f / 7.0f);                                       // the quaternion part of d0^2
-#pragma unroll
-    for (int i = 4; i < 7; ++i) {                                                // the rate components: f0 = 0
-        const float yi = (float)y[i];
-        const float v = yi * rcp_f32(fmaf(fabsf(yi), (float)RK_RTOL, (float)RK_ATOL));
-        d0s = fmaf(v, v, d0s);
-    }
-    d0s *= (1.0f / 7.0f);
-    d1s *= (1.0f / 7.0f);                                    // squares of the rms norms d0, d1
-    float h0f;
-    if (d0s < 1e-10f || d1s < 1e-10f) h0f = 1e-6f;
-    else h0f = 0.01f * sqrtf(d0s * rcp_f32(d1s));
-    const double h0 = fmin((double)h0f, dt);
-    // d2 = rms((f(y0 + h0 f0) - f0) / scale) / h0 only enters through max(d1, d2).  In plane coordinates
-    // f1 - f0 = da q0 + db p with |da| <= om2 h0 and |db| <= om2 h0^2 / 2, hence
-    // d2 <= om2 (rms(q0 / scale) + h0 d1 / 2): of the order omega d1, i.e. below d1 unless the body
-    // spins at ~1 rad/s.  When this bound (with 5 % slack for the float32 arithmetic) is below d1 the second slope
-    // is not evaluated at all; otherwise d2 is formed exactly as scipy does.
-    const float h0c = (float)h0;
-    const float ub = (float)om2 * fmaf(0.5f * h0c, sqrtf(d1s), sqrtf(d0q));
-    float dmax = d1s;
-    if (!(ub * ub * 1.05f <= d1s)) {
-        double ka1, kb1;
-        rhs_plane(1.0, h0, om2, ka1, kb1);                       // y1 = y0 + h0 f0
-        const float daf = (float)ka1, dbf = (float)(kb1 - 1.0);  // f1 - f0 in plane coordinates
-        float d2s = 0.0f;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const float v = fmaf(dbf, pf[i], daf * q0f[i]) * inv_sc[i];
-            d2s = fmaf(v, v, d2s);
-        }
-        const float inv_h0 = rcp_f32(h0c);
-        d2s = d2s * (1.0f / 7.0f) * inv_h0 * inv_h0;
-        dmax = fmaxf(d1s, d2s);
-    }
-    float h1;
-    if (dmax <= 1e-30f) h1 = fmaxf(1e-6f, h0c * 1e-3f);     // d1 <= 1e-15 and d2 <= 1e-15
-    else h1 = pow_neg_tenth_f32(fminf(dmax, 1e30f) * 1e4f);  // (0.01/max(d1,d2))**(1/5)
-    return fmin(fmin(100.0 * h0, (double)h1), dt);
-}
-#endif
 
 // basis of the invariant plane of one body: q0, p = (0.5 Omega(w) / |q0|) q0 (dynamics.py:137-150), om2 = |0.5 w|^2 / |q0|^2
 RDV_DEV void plane_basis(const double (&y)[7], double (&q0)[4], double (&p)[4], double &om2)
@@ -857,73 +655,33 @@ RDV_DEV void plane_basis(const double (&y)[7], double (&q0)[4], double (&p)[4], 
 struct PlanePoint { double a, b, g, t; float yf[4]; };
 
 // One solver.step() of scipy's RungeKutta._step_impl (rk.py:111-179): attempts from `s` until one is accepted; the
-// accepted point goes to `n` (`s` is left untouched, so the caller alternates two points and no copy is made).
-// Returns false on TOO_SMALL_STEP / a non-finite error norm.
-// RDV_RK_PINGPONG 1: two copies of the step alternate between two points so that an accepted candidate is never
-// copied.  Measured slower on B200 (12.1 vs 11.3 us per step at 65,536 envs: the second copy costs more spills than
-// the ~30 moves per accepted step it saves), so the single-copy form is the default.
-#ifndef RDV_RK_PINGPONG
-#define RDV_RK_PINGPONG 0
-#endif
-#ifndef RDV_MERGE_RARE
-#define RDV_MERGE_RARE 1        /* measured: 10.20 -> 10.13 us per step (20-step launches), 9.415 -> 9.37 (250-step) */
-#endif
-// RDV_LATE_MINSTEP: the TOO_SMALL_STEP test sits behind a rejection, the only place h_abs can have shrunk below
-// min_step (on entry it is clamped up to it).  RDV_LAZY_MINSTEP: min_step = 10 ulp(t) <= 4.4e-15 dt for t in [0, dt],
-// so while h_abs >= 1e-13 dt neither the clamp nor the test can fire and min_step is not formed at all.
-// RDV_LAST_FLAG: whether t has reached dt is known when t_new is clipped; plane_step returns it (2) instead of the
-// caller re-deriving it from t.
-#ifndef RDV_LATE_MINSTEP
-#define RDV_LATE_MINSTEP 0
-#endif
-#ifndef RDV_LAZY_MINSTEP
-#define RDV_LAZY_MINSTEP 0
-#endif
-#ifndef RDV_LAST_FLAG
-#define RDV_LAST_FLAG 0
-#endif
-// RDV_LAST_SHORTCUT: the attempt that is clipped to t = dt ends the solve when it is accepted -- the step factor and
-// the float32 copy of the new point are never used again -- so all it needs from the controller is the accept
-// decision.  With scale_i >= atol,  err^2 <= sum e_i^2 / (7 atol^2) <= 2 (ea^2 |q0|^2 + eb^2 |p|^2) / (7 atol^2)
-// (q0 is orthogonal to p; the factor 2 covers the rounding of that): below 0.99 the attempt is accepted without
-// forming the per-component norm, anything else takes the full path.
-#ifndef RDV_LAST_SHORTCUT
-#define RDV_LAST_SHORTCUT 1     /* measured: 9.76 -> 9.74 us per step (20-step launches), 8.94 -> 8.91 (250-step) */
-#endif
+// accepted point goes to `n` (`s` is left untouched).  Returns 0 on TOO_SMALL_STEP / a non-finite error norm, 2 when
+// the accepted step reaches t = dt (known when t_new is clipped, so the caller need not re-derive it from t), else 1.
+// The attempt that is clipped to t = dt ends the solve when it is accepted -- the step factor and the float32 copy of
+// the new point are never used again -- so all it needs from the controller is the accept decision.  With
+// scale_i >= atol,  err^2 <= sum e_i^2 / (7 atol^2) <= 2 (ea^2 |q0|^2 + eb^2 |p|^2) / (7 atol^2) (q0 is orthogonal to
+// p; the factor 2 covers the rounding of that): below 0.99 the attempt is accepted without forming the per-component
+// norm, anything else takes the full path (measured: 9.76 -> 9.74 us per step in 20-step launches, 8.94 -> 8.91 in
+// 250-step ones).
 template <bool POLY>
 RDV_DEV int plane_step(const PlanePoint &s, PlanePoint &n, double &h_abs, int &n_rejected, const double om2, const double dt,
                         const double (&q0)[4], const double (&p)[4], const float (&q0f)[4], const float (&pf)[4])
 {
     const double a = s.a, b = s.b, t = s.t;
-#if RDV_LAZY_MINSTEP
-    const double lazy_thr = dt * 1e-13;
-    if (h_abs < lazy_thr) {
-        const double min_step = 10.0 * (__longlong_as_double(__double_as_longlong(t) + 1) - t);
-        if (h_abs < min_step) h_abs = min_step;
-    }
-#else
     const double min_step = 10.0 * (__longlong_as_double(__double_as_longlong(t) + 1) - t);
     if (h_abs < min_step) h_abs = min_step;
-#endif
     bool rejected = false;
     for (;;) {
-#if !RDV_LATE_MINSTEP && !RDV_LAZY_MINSTEP
         if (h_abs < min_step) return 0;
-#endif
         double t_new = t + h_abs;
-#if RDV_LAST_FLAG || RDV_LAST_SHORTCUT
         const double over = t_new - dt;
         if (over > 0.0) t_new = dt;
         const bool last = over >= 0.0;
-#else
-        if (t_new - dt > 0.0) t_new = dt;
-#endif
         const double h = t_new - t;
         h_abs = fabs(h);
         // ---- rk_step and the error estimate (K^T E) h in the plane; the controller's norm in quaternion components ----
         double a_new, b_new, ea, eb;
         plane_attempt<POLY>(a, b, s.g, om2, h, a_new, b_new, ea, eb);
-#if RDV_LAST_SHORTCUT
         if (last) {
             const float eaf = (float)ea, ebf = (float)eb;
             float nq = 0.0f, np = 0.0f;
@@ -935,22 +693,15 @@ RDV_DEV int plane_step(const PlanePoint &s, PlanePoint &n, double &h_abs, int &n
                 return 2;
             }
         }
-#endif
         const float esf = plane_err2_f32(ea, eb, a_new, b_new, q0f, pf, s.yf, n.yf);
-#if RDV_MERGE_RARE
         // one branch for both rare cases: a non-finite norm (the reference shrinks h to failure) and the threshold
-        // region, where the accept decision is taken with the fp64 norm
+        // region, where the accept decision is taken with the fp64 norm (measured against two branches: 10.20 -> 10.13
+        // us per step in 20-step launches, 9.415 -> 9.37 in 250-step ones)
         bool accept = esf < 1.0f;
         if (!(fabsf(esf - 1.0f) >= 1.0e-3f && esf < 1.0e30f)) {
             if (!(esf < 1.0e30f)) return 0;
             accept = plane_err2_f64(ea, eb, a, b, a_new, b_new, q0, p) < 1.0;
         }
-#else
-        if (!(esf < 1.0e30f)) return 0;            // NaN / inf: the reference shrinks h to failure
-        bool accept = esf < 1.0f;
-        if (fabsf(esf - 1.0f) < 1.0e-3f)           // threshold region: decide with the fp64 norm
-            accept = plane_err2_f64(ea, eb, a, b, a_new, b_new, q0, p) < 1.0;
-#endif
         // 0.9 err^-0.2, clamped where the controller's min / max saturate anyway
         const float pw = 0.9f * pow_neg_tenth_f32(fminf(fmaxf(esf, 1e-12f), 1e8f));
         if (accept) {
@@ -958,37 +709,18 @@ RDV_DEV int plane_step(const PlanePoint &s, PlanePoint &n, double &h_abs, int &n
             if (rejected) factor = fminf(1.0f, factor);
             h_abs *= (double)factor;
             n.a = a_new; n.b = b_new; n.g = plane_g(a_new, b_new, om2); n.t = t_new;
-#if RDV_LAST_FLAG || RDV_LAST_SHORTCUT
             return last ? 2 : 1;
-#else
-            return 1;
-#endif
         }
         h_abs *= (double)fmaxf(0.2f, pw);
         rejected = true;
         ++n_rejected;
-#if RDV_LAZY_MINSTEP
-        if (h_abs < lazy_thr) {
-            const double min_step = 10.0 * (__longlong_as_double(__double_as_longlong(t) + 1) - t);
-            if (h_abs < min_step) return 0;
-        }
-#elif RDV_LATE_MINSTEP
-        if (h_abs < min_step) return 0;
-#endif
     }
 }
 
 // The float32 copies of the basis are used by every attempted step.  Left alone, the compiler re-converts them from
 // the fp64 values inside the loop (8 F2F per attempt on the 16-lane XU pipe) rather than keep eight more registers;
-// the empty asm makes the converted value opaque, so it is kept (or spilled as 4 bytes) instead.
-#ifndef RDV_NO_REMAT
-#define RDV_NO_REMAT 1          /* measured: 11.29 -> 10.93 us per step at 65,536 envs */
-#endif
-#if RDV_NO_REMAT
-#define RDV_KEEP_F32(x) asm volatile("" : "+f"(x))
-#else
-#define RDV_KEEP_F32(x)
-#endif
+// the empty asm makes the converted value opaque, so it is kept (or spilled as 4 bytes) instead (measured: 11.29 ->
+// 10.93 us per step at 65,536 envs).
 template <bool POLY>
 RDV_DEV int rk45_iso_plane_solve(double (&y)[7], const double dt, int &n_rejected)
 {
@@ -999,35 +731,22 @@ RDV_DEV int rk45_iso_plane_solve(double (&y)[7], const double dt, int &n_rejecte
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         q0f[i] = (float)q0[i]; pf[i] = (float)p[i];
-        RDV_KEEP_F32(q0f[i]); RDV_KEEP_F32(pf[i]);
+        asm volatile("" : "+f"(q0f[i])); asm volatile("" : "+f"(pf[i]));
         X.yf[i] = q0f[i];
     }
     X.a = 1.0; X.b = 0.0; X.g = 1.0; X.t = 0.0;                 // y = a q0 + b p; slope there = p
     double h_abs = plane_initial_step(y, q0f, pf, om2, dt);
     int accepted = 0;
-#if RDV_RK_PINGPONG
-    // two copies of the step that read one point and write the other: the accepted candidate is never copied
-    for (;;) {
-        if (!plane_step<POLY>(X, Y, h_abs, n_rejected, om2, dt, q0, p, q0f, pf)) return -1;
-        ++accepted;
-        if (Y.t - dt >= 0.0) { X.a = Y.a; X.b = Y.b; break; }
-        if (!plane_step<POLY>(Y, X, h_abs, n_rejected, om2, dt, q0, p, q0f, pf)) return -1;
-        ++accepted;
-        if (X.t - dt >= 0.0) break;
-    }
-#else
+    // One copy of the step, and the accepted point is copied back.  Two copies that alternate between X and Y, so that
+    // nothing is copied, measured slower on B200 (12.1 vs 11.3 us per step at 65,536 envs: the second copy costs more
+    // spills than the ~30 moves per accepted step it saves).
     for (;;) {
         const int r = plane_step<POLY>(X, Y, h_abs, n_rejected, om2, dt, q0, p, q0f, pf);
         if (!r) return -1;
         ++accepted;
         X = Y;
-#if RDV_LAST_FLAG || RDV_LAST_SHORTCUT
         if (r == 2) break;
-#else
-        if (X.t - dt >= 0.0) break;
-#endif
     }
-#endif
 #pragma unroll
     for (int i = 0; i < 4; ++i) y[i] = fma(X.b, p[i], X.a * q0[i]);
     return accepted;
@@ -1037,14 +756,10 @@ __device__ __noinline__ int rk45_iso_plane_stagewise(double (&y)[7], const doubl
 {
     return rk45_iso_plane_solve<false>(y, dt, n_rejected);
 }
-RDV_RK_FN int rk45_iso_plane(double (&y)[7], const double dt, int &n_rejected)
+RDV_DEV int rk45_iso_plane(double (&y)[7], const double dt, int &n_rejected)
 {
-#if RDV_PLANE_POLY
     if (!plane_poly_covers(y, dt)) return rk45_iso_plane_stagewise(y, dt, n_rejected);
     return rk45_iso_plane_solve<true>(y, dt, n_rejected);
-#else
-    return rk45_iso_plane_solve<false>(y, dt, n_rejected);
-#endif
 }
 
 // Lock-step form of rk45_iso_plane for TWO bodies in one thread (chaser and target of one env): the control flow of
@@ -1053,7 +768,6 @@ RDV_RK_FN int rk45_iso_plane(double (&y)[7], const double dt, int &n_rejected)
 // the two bodies are interleaved stage by stage in the source, so that two independent slope chains (norm ->
 // rsqrt -> scale) sit next to each other in every basic block.  Arithmetic per body is that of rk45_iso_plane,
 // operation for operation (tests/test_gpu_rollout.py compares the bits).
-template <bool POLY>
 RDV_DEV int rk45_iso_plane_pair_solve(double (&ya)[7], double (&yb)[7], const double dt, int &n_rejected)
 {
     double q0[2][4], p[2][4], om2[2], a[2], b[2], g[2], h_abs[2], t[2];
@@ -1086,7 +800,7 @@ RDV_DEV int rk45_iso_plane_pair_solve(double (&ya)[7], double (&yb)[7], const do
             ha[c] = fabs(h[c]);
         }
 #pragma unroll
-        for (int c = 0; c < 2; ++c) plane_attempt<POLY>(a[c], b[c], g[c], om2[c], h[c], as[c], bs[c], ea[c], eb[c]);
+        for (int c = 0; c < 2; ++c) plane_attempt<true>(a[c], b[c], g[c], om2[c], h[c], as[c], bs[c], ea[c], eb[c]);
 #pragma unroll
         for (int c = 0; c < 2; ++c) {
             // as / bs hold (a_new, b_new) of the attempted step
@@ -1134,12 +848,8 @@ __device__ __noinline__ int rk45_iso_plane_pair_mixed(double (&ya)[7], double (&
 }
 RDV_DEV int rk45_iso_plane_pair(double (&ya)[7], double (&yb)[7], const double dt, int &n_rejected)
 {
-#if RDV_PLANE_POLY
     if (!(plane_poly_covers(ya, dt) && plane_poly_covers(yb, dt))) return rk45_iso_plane_pair_mixed(ya, yb, dt, n_rejected);
-    return rk45_iso_plane_pair_solve<true>(ya, yb, dt, n_rejected);
-#else
-    return rk45_iso_plane_pair_solve<false>(ya, yb, dt, n_rejected);
-#endif
+    return rk45_iso_plane_pair_solve(ya, yb, dt, n_rejected);
 }
 
 // Closed-form alternative (opt-in, RDV_INTEGRATOR_CLOSED_FORM; only valid for ISO bodies):

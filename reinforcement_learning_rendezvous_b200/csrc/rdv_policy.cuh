@@ -1,7 +1,7 @@
 // rdv_policy.cuh -- small pieces shared by the actor kernels (the SB3 MlpPolicy actor 17 -> 64 -> 64 -> 6, tanh;
-// main.py:39-48): the TF32 rounding of a float (TF32 build of the actor) and the Gaussian head's Philox / Box-Muller noise.  The tensor-core
-// forward itself (tcgen05 / TMEM, stand-alone and inside the rollout kernel) lives in rdv_policy_tc.cuh, the
-// plain fp32-FMA numerics reference in rdv_b200.cu (policy_kernel).
+// main.py:39-48): the Gaussian head's Philox / Box-Muller noise.  The tensor-core forward itself (tcgen05 / TMEM,
+// stand-alone and inside the rollout kernel) lives in rdv_policy_tc.cuh, the plain fp32-FMA numerics reference in
+// rdv_b200.cu (policy_kernel).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -11,14 +11,6 @@
 namespace rdv {
 
 constexpr int PI_H = 64;             // hidden width (SB3 default net_arch [64, 64])
-
-// x rounded to TF32 (10 mantissa bits, round to nearest); x - tf32_hi(x) is exact in fp32
-__device__ __forceinline__ float tf32_hi(float x)
-{
-    uint32_t r;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-    return __uint_as_float(r);
-}
 
 // Six N(0,1) float32 draws for (noise seed; env id, step index): Philox blocks 0x20000000 | {0,1,2}, one
 // Box-Muller pair per block (the Gaussian head of SB3's DiagGaussianDistribution.sample()).

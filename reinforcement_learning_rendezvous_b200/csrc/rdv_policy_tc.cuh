@@ -20,8 +20,8 @@
 // Every product is three MMAs of halves (a_lo b_hi + a_hi b_lo + a_hi b_hi, fp32 accumulation) so the result has
 // fp32-level accuracy, like the reference's torch policy: 11 + 11 significant bits per operand.  The halves are
 // fp16 (kind::f16, K = 16 per MMA): observations, tanh outputs and weights are O(1), far inside the fp16 range, lo
-// is exact down to 2^-24 in absolute terms, and a layer costs half the MMAs of the TF32 split (kind::tf32, K = 8;
-// RDV_ACTOR_F16 = 0 builds it) -- the small-N MMAs of this MLP are issue-rate bound, so that is half the tensor time:
+// is exact down to 2^-24 in absolute terms, and a layer costs half the MMAs of a TF32 split (kind::tf32, K = 8) --
+// the small-N MMAs of this MLP are issue-rate bound, so that is half the tensor time:
 // [B200] 19.5 us against 23.2 for 131,072 rows, worst deviation from an fp64 evaluation 2.7e-6 against 5.0e-6 (the
 // MMA truncates the TF32 lo half; the fp16 halves are rounded to nearest).  The hi part of the activations never
 // leaves the tensor-memory: the two products that use it are issued in the "TS" form of tcgen05.mma (A from TMEM,
@@ -36,8 +36,8 @@
 //
 // Shared-memory operands use the canonical no-swizzle K-major UMMA layout: 8-row x 16-byte core matrices, rows of
 // a core matrix 16 B apart, 8-row groups SBO = 128 B apart, the two 16-byte K-chunks of a K-step
-// LBO = rows*16 B apart, i.e. with CHUNK = 8 fp16 (4 TF32) elements per 16 bytes element (r, k) lives at
-// ((k / CHUNK) * rows + r) * 16 + (k % CHUNK) * sizeof(element) bytes.
+// LBO = rows*16 B apart, i.e. with CHUNK = 8 fp16 elements per 16 bytes element (r, k) lives at
+// ((k / CHUNK) * rows + r) * 16 + (k % CHUNK) * 2 bytes.
 // (Descriptor bit layouts: CUTLASS cute/arch/mma_sm100_desc.hpp; instruction forms: cute/arch/mma_sm100_umma.hpp.)
 #pragma once
 #include <cuda_runtime.h>
@@ -46,24 +46,14 @@
 #include "rdv_b200.h"
 #include "rdv_policy.cuh"
 
-#ifndef RDV_ACTOR_F16
-#define RDV_ACTOR_F16 1      /* 1: operands split into two fp16 halves (kind::f16, K = 16); 0: TF32 halves (kind::tf32, K = 8) */
-#endif
-
 namespace rdv {
 namespace tc {
 
 constexpr int TM = 128;                 // envs per tile = UMMA M = threads per group
 constexpr int H = 64;                   // hidden width
-#if RDV_ACTOR_F16
 typedef uint16_t elem_t;                // operand element in shared memory: fp16 bits
 constexpr int KSTEP = 16, CHUNK = 8;    // K of one MMA; elements of one 16-byte chunk of a core-matrix row
 constexpr int K0 = 32;                  // 17 inputs + 1 bias column, padded to 2 K-steps of 16
-#else
-typedef float elem_t;
-constexpr int KSTEP = 8, CHUNK = 4;
-constexpr int K0 = 24;                  // 17 inputs + 1 bias column, padded to 3 K-steps of 8
-#endif
 constexpr int N3 = 16;                  // 6 outputs padded to the smallest legal UMMA N for M = 128
 constexpr int GROUPS = 4;               // independent 128-thread tile pipelines per CTA
 constexpr uint32_t GROUP_COLS = 128;    // TMEM columns per group: D @ +0..63 (D3 @ +0..15), A hi @ +64..127
@@ -109,22 +99,17 @@ __device__ __forceinline__ uint64_t umma_desc(const void *p, uint32_t lbo_bytes,
     d |= (uint64_t)1 << 46;                                        // descriptor version of sm_100
     return d;
 }
-// 32-bit instruction descriptor: D = F32, A = B = TF32 (format 2) or F16 (format 0), both K-major, M = 128, N = n.
+// 32-bit instruction descriptor: D = F32, A = B = F16 (format 0 in bits 7 and 10), both K-major, M = 128, N = n.
 __device__ __forceinline__ uint32_t umma_idesc(int n)
 {
-    const uint32_t fmt = RDV_ACTOR_F16 ? 0u : 2u;
-    return (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(TM >> 4) << 24);
+    return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(TM >> 4) << 24);
 }
 // D += A B with A described in shared memory ("SS")
 __device__ __forceinline__ void umma_ss(uint32_t tmem_d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t accumulate)
 {
     asm volatile(
         "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-#if RDV_ACTOR_F16
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-#else
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-#endif
         :: "r"(tmem_d), "l"(a), "l"(b), "r"(idesc), "r"(accumulate) : "memory");
 }
 // D += A B with A read from tensor memory ("TS"): 128 lanes x 8 columns at tmem_a
@@ -132,11 +117,7 @@ __device__ __forceinline__ void umma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64
 {
     asm volatile(
         "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-#if RDV_ACTOR_F16
         "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-#else
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
-#endif
         :: "r"(tmem_d), "r"(tmem_a), "l"(b), "r"(idesc), "r"(accumulate) : "memory");
 }
 __device__ __forceinline__ void umma_commit(uint64_t *bar)
@@ -186,9 +167,8 @@ __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.a
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-// the two halves of a float: hi = the value rounded to the operand format, lo = what is left, rounded likewise
-// (fp16: 11 + 11 significant bits, lo exact down to 2^-24 in absolute terms; TF32: 11 + 11 bits, lo truncated by the MMA)
-#if RDV_ACTOR_F16
+// the two halves of a float: hi = the value rounded to fp16, lo = what is left, rounded likewise (11 + 11 significant
+// bits, lo exact down to 2^-24 in absolute terms)
 __device__ __forceinline__ void split2(float a, float b, uint32_t &hi, uint32_t &lo)
 {
     const __half2 h = __floats2half2_rn(a, b);
@@ -197,7 +177,6 @@ __device__ __forceinline__ void split2(float a, float b, uint32_t &hi, uint32_t 
     hi = *reinterpret_cast<const uint32_t *>(&h);
     lo = *reinterpret_cast<const uint32_t *>(&l);
 }
-#endif
 
 // bulk copy global -> shared, completion counted in bytes on an mbarrier (one thread issues both)
 __device__ __forceinline__ void bulk_load(void *dst, const void *src, uint32_t bytes, uint64_t *bar)
@@ -237,23 +216,17 @@ struct WeightTile {
                 const int nn = idx / K_PAD, k = idx % K_PAD;
                 const int o = ((k / CHUNK) * N_PAD + nn) * CHUNK + (k % CHUNK);
                 const float v = x[i] * scale;
-#if RDV_ACTOR_F16
                 const __half hi = __float2half_rn(v);
                 wh[o] = __half_as_ushort(hi);
                 wl[o] = __half_as_ushort(__float2half_rn(v - __half2float(hi)));
-#else
-                const float hi = tf32_hi(v);
-                wh[o] = hi;
-                wl[o] = v - hi;
-#endif
             }
         }
     }
 };
 
 // one layer: D[128 x n] (TMEM column d_col) = A[128 x KSTEP*ksteps] W^T, three products of halves, issued by the
-// calling thread.  A hi: TMEM columns a_hi + 8 kk .. + 7 (one 32-bit column per TF32 element / per pair of fp16
-// elements); A lo: shared memory.  A K-step is two 16-byte chunks per row whatever the element size.
+// calling thread.  A hi: TMEM columns a_hi + 8 kk .. + 7 (one 32-bit column per pair of fp16 elements); A lo: shared
+// memory.  A K-step is two 16-byte chunks per row.
 __device__ __forceinline__ void issue_layer(uint32_t a_hi, const elem_t *al, uint32_t tmem_d, const elem_t *wh,
                                             const elem_t *wl, int n, int ksteps, uint64_t *bar)
 {
@@ -323,7 +296,6 @@ __device__ __forceinline__ void hidden_epilogue(uint32_t lane_addr, const float 
             }
             tanh_scaled4(z, reinterpret_cast<float (&)[4]>(t[4 * c]));
         }
-#if RDV_ACTOR_F16
         // 16 activations = 8 packed TMEM columns (hi) and two 16-byte chunks of this row (lo)
         uint32_t hi[8], lo[8];
 #pragma unroll
@@ -331,20 +303,6 @@ __device__ __forceinline__ void hidden_epilogue(uint32_t lane_addr, const float 
         reinterpret_cast<uint4 *>(al)[(2 * q) * TM + r] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
         reinterpret_cast<uint4 *>(al)[(2 * q + 1) * TM + r] = make_uint4(lo[4], lo[5], lo[6], lo[7]);
         tmem_st8(lane_addr + A_COL + 8 * q, hi);
-#else
-        uint32_t hi[16];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-            float lo[4];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                hi[4 * c + j] = __float_as_uint(t[4 * c + j]) & 0xffffe000u;
-                lo[j] = t[4 * c + j] - __uint_as_float(hi[4 * c + j]);
-            }
-            reinterpret_cast<float4 *>(al)[(4 * q + c) * TM + r] = make_float4(lo[0], lo[1], lo[2], lo[3]);
-        }
-        tmem_st16(lane_addr + A_COL + 16 * q, hi);
-#endif
         if (q < 3) tmem_ld_wait(nxt);
     }
     tmem_st_wait();
@@ -433,7 +391,6 @@ __device__ __forceinline__ void tile_forward(elem_t *al, uint64_t *bar, const We
 {
     const uint32_t lane_addr = tmem + ((uint32_t)(r & ~31) << 16);         // this warp's 32 TMEM lanes
     // ---- A0: the observation row and the constant 1 of the bias column, hi -> TMEM, lo -> shared ----
-#if RDV_ACTOR_F16
     {
         // (values beyond the fp16 range are clamped: the first layer's tanh is saturated long before)
         uint32_t hi[K0 / 2], lo[K0 / 2];
@@ -454,31 +411,6 @@ __device__ __forceinline__ void tile_forward(elem_t *al, uint64_t *bar, const We
         tmem_st16(lane_addr + A_COL, hi);
         tmem_st_wait();
     }
-#else
-    {
-        uint32_t hi[K0];
-#pragma unroll
-        for (int c = 0; c < K0 / 4; ++c) {
-            float lo[4];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const int k = 4 * c + j;
-                const float v = k < RDV_OBS_DIM ? x[k < RDV_OBS_DIM ? k : 0] : (k == RDV_OBS_DIM ? 1.0f : 0.0f);
-                hi[k] = __float_as_uint(v) & 0xffffe000u;
-                lo[j] = v - __uint_as_float(hi[k]);
-            }
-            reinterpret_cast<float4 *>(al)[c * TM + r] = make_float4(lo[0], lo[1], lo[2], lo[3]);
-        }
-        uint32_t h0[16], h1[8];
-#pragma unroll
-        for (int j = 0; j < 16; ++j) h0[j] = hi[j];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) h1[j] = hi[16 + j];
-        tmem_st16(lane_addr + A_COL, h0);
-        tmem_st8(lane_addr + A_COL + 16, h1);
-        tmem_st_wait();
-    }
-#endif
     fence_async_smem();
     tc_fence_before();
     group_sync(g, threads);

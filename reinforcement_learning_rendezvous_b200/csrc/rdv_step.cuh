@@ -53,12 +53,8 @@ RDV_DEV void ingest_action_f32(const RdvParams &P, const float (&a)[6], EnvCount
 RDV_DEV void env_translate(const RdvParams &P, EnvRegs &e, const ActionTerms &t)
 {
     double dv[3];
-#if RDV_QUAT_ROTATE
-    quat_rotate(e.qc, t.dvb, dv);                  // one vector: no matrix
-#else
     const Rot Rc_old = rot_from_quat(e.qc);
     rot_apply(Rc_old, t.dvb, dv);
-#endif
     const double r0 = e.rc[0], r1 = e.rc[1], r2 = e.rc[2];
     const double v0 = e.vc[0] + dv[0], v1 = e.vc[1] + dv[1], v2 = e.vc[2] + dv[2];
     const double *c = P.cw;
@@ -116,12 +112,6 @@ RDV_DEV void env_advance(const RdvParams &P, EnvRegs &e, const ActionTerms &t, i
 }
 
 struct StepResult { double rew; int done, reason; };
-#ifndef RDV_EVAL_UNIT_Q
-#define RDV_EVAL_UNIT_Q 1       /* measured: 9.74 -> 9.70 us per step (20-step launches), 8.90 -> 8.87 (250-step) */
-#endif
-#ifndef RDV_NEAR_HOIST
-#define RDV_NEAR_HOIST 0
-#endif
 
 // gym 0.21 Box.contains on the float32 observation (rendezvous_env.py:367) WITHOUT forming the observation: a double
 // x rounds to a float in [-1, 1] iff |x| <= 1 + 2^-24.  Fast path on the high words of the raw state: a scaled entry
@@ -154,34 +144,11 @@ RDV_DEV StepResult env_evaluate(const RdvParams &P, const EnvRegs &e, const doub
                                 float (&ov)[RDV_OBS_DIM], EvalDetail *detail = nullptr)
 {
     const double rc_sq = dot3(e.rc, e.rc);
-#if RDV_QUAT_ROTATE
-    // far from the target only the capture axis is rotated by the chaser's attitude (one vector: no matrix)
-    const bool near = DETAIL || rc_sq < P.near_sq;
-    Rot Rc;
-    double att;
-    if (near) {
-        Rc = rot_from_quat(e.qc);
-        att = attitude_error(P, e, Rc, rc_sq);
-    } else {
-        double cap[3];
-        quat_rotate(e.qc, P.capture_axis, cap);
-        att = rounded_angle_from(-dot3(e.rc, cap), rc_sq, dot3(cap, cap));
-    }
-#else
-#if RDV_EVAL_UNIT_Q
     // the chaser's quaternion was normalised by env_attitude a moment ago: quat2mat's re-normalisation (a factor
-    // within 1 ulp of 1) is skipped outside the evaluator's own form
+    // within 1 ulp of 1) is skipped outside the evaluator's own form (measured: 9.74 -> 9.70 us per step in 20-step
+    // launches, 8.90 -> 8.87 in 250-step ones)
     const Rot Rc = DETAIL ? rot_from_quat(e.qc) : rot_from_unit_quat(e.qc);
-#else
-    const Rot Rc = rot_from_quat(e.qc);
-#endif
     const double att = attitude_error(P, e, Rc, rc_sq);
-#if RDV_NEAR_HOIST
-    const bool near = DETAIL || rc_sq < P.near_sq;
-#else
-#define near (DETAIL || rc_sq < P.near_sq)
-#endif
-#endif
     // The target-relative quantities (corridor angle, position / velocity / rate errors) only matter near the
     // target: a collision needs |rc| < koz, and success (:406-422) or the reward bonus (:348-351) need a position
     // error <= max_rd_error, impossible unless | |rc| - |rd| | <= max_rd_error (|R(qt) rd| = |rd|).  Far away
@@ -189,7 +156,7 @@ RDV_DEV StepResult env_evaluate(const RdvParams &P, const EnvRegs &e, const doub
     bool col_now = false;
     ErrSq es;
     es.pos = es.vel = es.rot = 1.0e300;
-    if (near) {
+    if (DETAIL || rc_sq < P.near_sq) {
         const Rot Rt = rot_from_quat(e.qt);
         if (DETAIL) {
             // the evaluator's own forms (errors_kernel): IEEE square roots, the corridor angle at any distance
@@ -237,9 +204,6 @@ RDV_DEV StepResult env_evaluate(const RdvParams &P, const EnvRegs &e, const doub
     c.ep_ret += rew;
     return r;
 }
-#ifdef near
-#undef near
-#endif
 
 // Per-episode accumulators of monte_carlo.evaluate (monte_carlo.py:94-207), one sample per visited state.
 // Terminal errors (:159-189): the constraint sets are nested (all four < limits  =>  pos, vel and att-or-rot  =>

@@ -1,6 +1,6 @@
-"""CPU: the bounds behind the three controller shortcuts of csrc/rdv_math.cuh (RDV_INIT_LAZY_D0, RDV_INIT_NOSQRT,
-RDV_LAST_SHORTCUT), checked against SciPy's own ``select_initial_step`` / ``rk_step`` on the reference's right-hand
-side -- no GPU involved.  What the kernel skips when a bound holds must be what SciPy would have computed anyway:
+"""CPU: the bounds behind the three controller shortcuts of csrc/rdv_math.cuh (plane_initial_step, plane_step),
+checked against SciPy's own ``select_initial_step`` / ``rk_step`` on the reference's right-hand side -- no GPU
+involved.  What the kernel skips when a bound holds must be what SciPy would have computed anyway:
 
 * ``select_initial_step`` returns min(100 h0, h1, dt); with the kernel's conditions satisfied it equals
   min((0.01 / d1)^(1/5), dt) with d1 from the quaternion components alone (d2 <= d1, and 100 h0 is not the minimum);

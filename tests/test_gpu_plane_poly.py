@@ -1,4 +1,4 @@
-"""GPU: the polynomial form of the attempted plane step (csrc/rdv_math.cuh, RDV_PLANE_POLY) -- the device polynomials
+"""GPU: the polynomial form of the attempted plane step (csrc/rdv_math.cuh, rk45_iso_plane) -- the device polynomials
 against the stagewise attempt, bodies on both sides of the polynomials' range against the C oracle, and launch shapes."""
 import ctypes as C
 

@@ -213,7 +213,7 @@ def test_plane_solver_edge_states_vs_c_oracle():
 @pytest.mark.parametrize("dt", [0.25, 1.0, 4.0])
 def test_fast_spins_take_the_general_controller_paths(dt):
     """select_initial_step and the last attempt of a solve are shortened by bounds that hold for every body the
-    reference's ranges produce (csrc/rdv_math.cuh: RDV_INIT_LAZY_D0, RDV_INIT_NOSQRT, RDV_LAST_SHORTCUT).  Bodies that
+    reference's ranges produce (csrc/rdv_math.cuh: plane_initial_step, plane_step).  Bodies that
     spin at up to several rad/s break those bounds -- 100 h0 becomes the smallest candidate, d2 exceeds d1, steps are
     rejected, the clipped last attempt is not trivially acceptable -- and must then follow the C oracle through the
     general path, at every dt of the sensitivity grid, through both kernels."""
