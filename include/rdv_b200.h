@@ -258,6 +258,23 @@ enum { RDV_MC_EP_LEN = 0, RDV_MC_NUM_COLLISIONS, RDV_MC_COLLIDED, RDV_MC_TOTAL_R
 int rdv_rollout(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, int64_t n, uint64_t seed,
                 int64_t env_offset, void *cuda_stream);
 
+/* Columns of the trajectory record of rdv_rollout_trajectory.  Columns 0 .. RDV_NF64 - 1 are the rows of RdvState.f64
+ * in their order (state, totals, episode return); then the RdvState.i32 rows as doubles; then what rdv_errors returns
+ * for that state: get_errors (position [m], velocity [m/s], attitude [rad], rate [rad/s]), dist_from_koz, and
+ * check_collision / check_success (with the sticky collided flag) as 0 / 1. */
+enum { RDV_TR_I_STEP = RDV_NF64, RDV_TR_I_SUCCESS, RDV_TR_I_COLLIDED, RDV_TR_I_EPISODE,
+       RDV_TR_POS_ERR, RDV_TR_VEL_ERR, RDV_TR_ATT_ERR, RDV_TR_ROT_ERR, RDV_TR_KOZ, RDV_TR_COLLISION, RDV_TR_SUCCESS,
+       RDV_TR_NCOL };
+/* rdv_rollout that also records the fp64 trajectory: traj [K][RDV_TR_NCOL][n] (8-byte aligned, 272 bytes per
+ * env-step), element (k, col, i) at traj[(k * RDV_TR_NCOL + col) * n + i].  Row k is env i after step k's propagation
+ * and evaluation and BEFORE an auto-reset (for an env that finished at step k: its terminal state); columns
+ * 0 .. RDV_TR_I_EPISODE hold what RdvState would hold there, the rest what rdv_errors returns on that state, bit for
+ * bit.  In the evaluator mode a finished env stops stepping, and its later rows repeat its last one.  Every other
+ * output is the same as rdv_rollout's for the same arguments (which it accepts and checks in the same way);
+ * traj NULL: RDV_ERR_NULL. */
+int rdv_rollout_trajectory(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, double *traj, int64_t n,
+                           uint64_t seed, int64_t env_offset, void *cuda_stream);
+
 /* RendezvousEnv.reset (rendezvous_env.py:223-270) for the envs selected by mask (NULL = all).
  * The 24 uniform draws come from Philox4x32-10 keyed by (seed; env_offset+i, episode index),
  * or from `uniforms` ([n][24], in [0,1)) when it is not NULL (test hook that pins the

@@ -123,6 +123,9 @@ POLICY_TILE = 128               # envs per entry of RdvRolloutIO.policy_tile
 (MC_EP_LEN, MC_NUM_COLLISIONS, MC_COLLIDED, MC_TOTAL_REWARD, MC_TOTAL_DELTA_V, MC_NUM_SUCCESSES, MC_SUCCEEDED,
  MC_MIN_KOZ, MC_POS_ERR, MC_VEL_ERR, MC_ATT_ERR, MC_ROT_ERR, MC_LEVEL, MC_TAIL_COUNT, MC_END_REASON,
  MC_TOTAL_DELTA_W, MC_NCOL) = range(17)
+# columns of the trajectory record of rdv_rollout_trajectory: 0 .. NF64 - 1 are the RdvState.f64 rows (RCX .. EPRET)
+(TR_I_STEP, TR_I_SUCCESS, TR_I_COLLIDED, TR_I_EPISODE, TR_POS_ERR, TR_VEL_ERR, TR_ATT_ERR, TR_ROT_ERR, TR_KOZ,
+ TR_COLLISION, TR_SUCCESS, TR_NCOL) = range(NF64, NF64 + 12)
 TUNE_ROLLOUT_TPB, TUNE_RESET_REFILL, TUNE_ROLLOUT_PDL, TUNE_ROLLOUT_HELPERS = 0, 1, 2, 3
 
 
@@ -142,6 +145,8 @@ PROTOTYPES = {
                            C.c_uint64, C.c_int64, C.c_void_p]),
     "rdv_rollout": (C.c_int, [C.POINTER(RdvParams), C.POINTER(RdvState), C.POINTER(RdvRolloutIO), C.c_int64,
                               C.c_uint64, C.c_int64, C.c_void_p]),
+    "rdv_rollout_trajectory": (C.c_int, [C.POINTER(RdvParams), C.POINTER(RdvState), C.POINTER(RdvRolloutIO),
+                                         C.c_void_p, C.c_int64, C.c_uint64, C.c_int64, C.c_void_p]),
     "rdv_reset": (C.c_int, [C.POINTER(RdvParams), C.POINTER(RdvState), C.c_void_p, C.c_void_p, C.c_void_p,
                             C.c_int64, C.c_uint64, C.c_int64, C.c_int, C.c_void_p]),
     "rdv_observe": (C.c_int, [C.POINTER(RdvParams), C.POINTER(RdvState), C.c_void_p, C.c_int64, C.c_void_p]),

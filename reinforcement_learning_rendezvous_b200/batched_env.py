@@ -247,7 +247,7 @@ class BatchedRendezvousEnv:
                 step_base: int = 0, record_rewards: bool = False, record_dones: bool = False,
                 record_obs: bool = False, record_actions: bool = False, policy=None,
                 stochastic: bool = False, carry_reset_rows: bool = True, monte_carlo: bool = False,
-                policy_tiles=None) -> dict:
+                policy_tiles=None, record_trajectory: bool = False) -> dict:
         """``steps`` consecutive env steps in ONE kernel launch (state stays in registers, finished envs restart
         in place when ``auto_reset``).  Actions come from ``actions`` ([steps, N, 6] float32/float64 on the device) or,
         when it is None, from the device Philox stream ``(action_seed; global env id, step_base + k)`` as U(-1,1) fp64
@@ -265,7 +265,12 @@ class BatchedRendezvousEnv:
         tile of 128 envs) names the entry that acts for envs ``128 t .. 128 t + 127``, all in the same launch; every
         tile gives the bits a separate env of its envs (same seed, ``env_offset`` = tile start) rolled with that entry
         would give.  Asynchronous on the current stream (the tile map is checked on the host: a device tensor given as
-        ``policy_tiles`` is read back for that, which waits for the stream; a host sequence does not)."""
+        ``policy_tiles`` is read back for that, which waits for the stream; a host sequence does not).
+        ``record_trajectory``: the launch also records the fp64 trajectory (``rdv_rollout_trajectory``) and returns it
+        as ``trajectory`` f64 [steps, TR_NCOL, N] on the device -- 272 B per env-step.  Row k is every env after step k
+        and before an auto-reset (a finished env's terminal state): columns 0 .. NF64 - 1 the ``f64`` state rows,
+        ``TR_I_STEP`` .. ``TR_I_EPISODE`` the ``i32`` rows, ``TR_POS_ERR`` .. ``TR_SUCCESS`` what :meth:`errors`
+        returns for that state.  Every other output is the same as without the record."""
         steps = int(steps)
         n, dev = self.num_envs, self.device
         if steps < 0:
@@ -311,8 +316,9 @@ class BatchedRendezvousEnv:
             if self.auto_reset:
                 raise ValueError("monte_carlo mode needs an env with auto_reset=False")
             mc_out = torch.empty((n, N.MC_NCOL), dtype=torch.float64, device=dev)
+        traj = torch.empty((steps, N.TR_NCOL, n), dtype=torch.float64, device=dev) if record_trajectory else None
         if len(self._units) > 1 and (rew is not None or don is not None or obs_steps is not None or act_out is not None
-                                     or actions is not None):
+                                     or actions is not None or traj is not None):
             raise NotImplementedError("per-step records / tensor actions with param_batches of general-inertia or "
                                       "closed-form groups (one launch per group): use step()")
         stream = _stream_ptr(dev)
@@ -333,8 +339,13 @@ class BatchedRendezvousEnv:
                     policy.table.data_ptr() if table is not None else None,
                     table.data_ptr() if table is not None else None, len(policy) if table is not None else 0, 0)
                 st = self._state_of(g)
-                N.check(self.lib.rdv_rollout(C.byref(g.params), C.byref(st), C.byref(io), g.n, self.seed,
-                                             self.env_offset + g.lo, stream), "rdv_rollout")
+                if traj is None:
+                    N.check(self.lib.rdv_rollout(C.byref(g.params), C.byref(st), C.byref(io), g.n, self.seed,
+                                                 self.env_offset + g.lo, stream), "rdv_rollout")
+                else:
+                    N.check(self.lib.rdv_rollout_trajectory(C.byref(g.params), C.byref(st), C.byref(io),
+                                                            traj.data_ptr(), g.n, self.seed, self.env_offset + g.lo,
+                                                            stream), "rdv_rollout_trajectory")
         self._keepalive = (actions, policy, table)
         if rew is not None:
             out["rewards"] = rew
@@ -346,6 +357,8 @@ class BatchedRendezvousEnv:
             out["actions"] = act_out
         if mc_out is not None:
             out["mc"] = mc_out
+        if traj is not None:
+            out["trajectory"] = traj
         return out
 
     def _policy_tile_map(self, tiles: np.ndarray) -> torch.Tensor:

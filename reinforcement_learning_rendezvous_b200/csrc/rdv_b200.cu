@@ -9,7 +9,8 @@
 // Kernels (DESIGN.md section 4):
 //   step_kernel     rdv_step     one launch per step, two lanes per env, team-of-8 auto-reset fused in
 //   rollout_kernel  rdv_rollout  K steps per launch, state in registers, one CTA per SM, prefetched in-warp
-//                                resets, actions from a tensor / Philox / the actor on the tensor cores (tcgen05)
+//                                resets, actions from a tensor / Philox / the actor on the tensor cores (tcgen05);
+//                                rdv_rollout_trajectory: the same launch, recording every env's fp64 state each step
 //   reset_kernel, observe_kernel, errors_kernel, frame_kernel, policy_kernel, fp64_peak_kernel
 #include <cuda_runtime.h>
 #include <math.h>
@@ -482,11 +483,14 @@ RDV_DEV void take_reset_row(const double *rw, const int64_t rs, EnvRegs &e, EnvC
 // time.  The helper warps land on those two (warp id mod 4) and take the one piece of the step that does not depend on
 // the trajectory off the workers: recomputing the reset rows that were used.  Workers post (lane, episode) requests in
 // shared memory and never wait -- a row that is not ready when its lane finishes is computed on the spot, as before.
+// TRAJ: every step writes one row of RDV_TR_NCOL doubles per env to `traj` ([K][RDV_TR_NCOL][n], rdv_b200.h): the
+// state and counters after the step's evaluation, before an auto-reset, and the evaluator quantities of that state in
+// the forms of errors_kernel.  Only the TRAJ variants read `traj`.
 template <bool ISO, bool CLOSED, int TPB_, bool POLICY = false, bool MC = false, bool TABLE = false, bool OBS = POLICY,
-          bool HELP = false, bool PTAB = false>
+          bool HELP = false, bool PTAB = false, bool TRAJ = false>
 __global__ void __launch_bounds__(TPB_ + (HELP ? 64 : 0), 1)
 rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __grid_constant__ RdvRolloutIO io,
-               const int64_t n, const uint64_t seed, const int64_t env_offset)
+               const int64_t n, const uint64_t seed, const int64_t env_offset, double *const traj)
 {
     static_assert(!HELP || (!POLICY && !MC && !TABLE && !OBS), "helper warps: plain variant only");
     static_assert(!PTAB || (POLICY && TPB_ == 256), "policy tables: the fused actor with two 128-thread groups");
@@ -737,11 +741,13 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
         McAcc mc;
         bool alive = true;
         int mc_reason = -1;
+        EvalDetail d_last;                                     // TRAJ + MC: the detail of the env's last state
         if constexpr (MC) {
             mc_init(mc);
             EvalDetail d;
             eval_detail_of_state(P, e, d);
             mc_sample(P, d, c.collided, mc);
+            if constexpr (TRAJ) d_last = d;
         }
 
         // One env step = an action phase (actor on the tensor cores, or a tensor / Philox action) and a step phase
@@ -799,6 +805,7 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
                     EvalDetail d;
                     r = env_evaluate<true, true>(P, e, t.fuel, c, ov, &d);
                     mc_sample(P, d, c.collided, mc);                          // monte_carlo.py:140-149
+                    if constexpr (TRAJ) d_last = d;
                     mc.total_reward += r.rew;
                     mc.len += 1;
                     if (r.done) { alive = false; mc_reason = r.reason; }
@@ -873,6 +880,18 @@ rollout_kernel(const __grid_constant__ RdvParams Pc, const RdvState S, const __g
                     st.end0 += r.reason == 0; st.end1 += r.reason == 1; st.end2 += r.reason == 2;
                     st.end3 += r.reason == 3;
                     st.ep_return += c.ep_ret; st.ep_length += (double)c.step; st.delta_v += c.tdv; st.delta_w += c.tdw;
+                }
+            }
+            // ---- trajectory record: the state this step left, before an auto-reset replaces it ----
+            if constexpr (TRAJ) {
+                if (active) {
+                    // The step's own evaluation skips quat2mat's re-normalisation and, far from the target, the
+                    // errors, so the record's quantities are formed here as errors_kernel forms them; the evaluator
+                    // mode has them already (a finished env repeats its last row).
+                    EvalDetail d;
+                    if constexpr (MC) d = d_last;
+                    else eval_detail_of_state(P, e, d);
+                    store_traj_row(traj + (int64_t)k * RDV_TR_NCOL * n + i, n, e, c, d);
                 }
             }
             // ---- auto-reset inside the warp ----
@@ -1526,8 +1545,9 @@ int rdv_step(const RdvParams *p, const RdvState *s, const RdvStepIO *io, int64_t
     return launch_status();
 }
 
-int rdv_rollout(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, int64_t n, uint64_t seed,
-                int64_t env_offset, void *cuda_stream)
+// rdv_rollout (traj NULL) and rdv_rollout_trajectory (traj checked by the caller)
+static int rollout_launch(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, double *traj, int64_t n,
+                          uint64_t seed, int64_t env_offset, void *cuda_stream)
 {
     if (!p || !io || !io->obs) return RDV_ERR_NULL;
     int rc = check_state(s, n);
@@ -1588,12 +1608,12 @@ int rdv_rollout(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, i
             at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;                                        \
             at[0].val.programmaticStreamSerializationAllowed = 1;                                                 \
             cfg.attrs = at; cfg.numAttrs = 1;                                                                     \
-            if (cudaLaunchKernelEx(&cfg, KERNEL, *p, *s, io_k, n, seed, env_offset) != cudaSuccess) {             \
+            if (cudaLaunchKernelEx(&cfg, KERNEL, *p, *s, io_k, n, seed, env_offset, traj) != cudaSuccess) {       \
                 cudaGetLastError();                                                                               \
                 return RDV_ERR_CUDA;                                                                              \
             }                                                                                                     \
         } else {                                                                                                  \
-            KERNEL<<<(unsigned)grid, T_, SMEM, st>>>(*p, *s, io_k, n, seed, env_offset);                          \
+            KERNEL<<<(unsigned)grid, T_, SMEM, st>>>(*p, *s, io_k, n, seed, env_offset, traj);                    \
         }                                                                                                         \
     }
 #define RDV_ROWS_SMEM(T_) ((size_t)(T_ / 32) * 32 * RDV_NEXT_ROW * sizeof(double))
@@ -1616,9 +1636,14 @@ int rdv_rollout(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, i
 #define RDV_LAUNCH_P(T_) RDV_LAUNCH_K((rollout_kernel<true, false, T_, true, false>), T_, sizeof(tc::TileSmem))
 #define RDV_LAUNCH_PT(MC_, TABLE_) \
     RDV_LAUNCH_K((rollout_kernel<true, false, 256, true, MC_, TABLE_, true, false, true>), 256, sizeof(tc::TableSmem))
-    // the policy-table variants are instantiated after all others: ptxas handles a module's kernels in that order, and
-    // with them first the register allocation of an existing variant (POLICY + TABLE) came out differently
-    if (!ptab) {
+    // trajectory records: one CTA shape per configuration, with the observation formed every step (as for obs_steps)
+#define RDV_LAUNCH_T(ISO_, CL_, POLICY_, MC_, TABLE_, PTAB_)                                                       \
+    RDV_LAUNCH_K((rollout_kernel<ISO_, CL_, 256, POLICY_, MC_, TABLE_, true, false, PTAB_, true>), 256,            \
+                 PTAB_ ? sizeof(tc::TableSmem) : POLICY_ ? sizeof(tc::TileSmem) : RDV_ROWS_SMEM(256))
+    // the policy-table variants are instantiated after all others, and the trajectory variants after those: ptxas
+    // handles a module's kernels in that order, and with them first the register allocation of an existing variant
+    // (POLICY + TABLE) came out differently
+    if (!ptab && !traj) {
         if (table) {
             if (!iso || closed) return RDV_ERR_UNSUPPORTED;      // parameter tables: the reference's bodies, RK45
             if (mc && policy) RDV_LAUNCH_K((rollout_kernel<true, false, 256, true, true, true>), 256, sizeof(tc::TileSmem))
@@ -1641,12 +1666,34 @@ int rdv_rollout(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, i
         else if (closed) { RDV_PICK_R(true, true) }
         else if (iso) { RDV_PICK_R(true, false) }
         else RDV_LAUNCH_OBS(false, false)                          // general inertia / held torque: one shape
-    } else {                                                    // (bodies and integrator checked above)
+    } else if (!traj) {                                         // (bodies and integrator checked above)
         if (mc && table) RDV_LAUNCH_PT(true, true)
         else if (mc) RDV_LAUNCH_PT(true, false)
         else if (table) RDV_LAUNCH_PT(false, true)
         else RDV_LAUNCH_PT(false, false)
+    } else {
+        // the configurations rdv_rollout accepts, each in its one trajectory variant
+        if ((table || mc || policy) && (!iso || closed)) return RDV_ERR_UNSUPPORTED;
+        if (ptab) {
+            if (mc && table) RDV_LAUNCH_T(true, false, true, true, true, true)
+            else if (mc) RDV_LAUNCH_T(true, false, true, true, false, true)
+            else if (table) RDV_LAUNCH_T(true, false, true, false, true, true)
+            else RDV_LAUNCH_T(true, false, true, false, false, true)
+        } else if (table) {
+            if (mc && policy) RDV_LAUNCH_T(true, false, true, true, true, false)
+            else if (mc) RDV_LAUNCH_T(true, false, false, true, true, false)
+            else if (policy) RDV_LAUNCH_T(true, false, true, false, true, false)
+            else RDV_LAUNCH_T(true, false, false, false, true, false)
+        } else if (mc) {
+            if (policy) RDV_LAUNCH_T(true, false, true, true, false, false)
+            else RDV_LAUNCH_T(true, false, false, true, false, false)
+        }
+        else if (policy) RDV_LAUNCH_T(true, false, true, false, false, false)
+        else if (closed) RDV_LAUNCH_T(true, true, false, false, false, false)
+        else if (iso) RDV_LAUNCH_T(true, false, false, false, false, false)
+        else RDV_LAUNCH_T(false, false, false, false, false, false)
     }
+#undef RDV_LAUNCH_T
 #undef RDV_LAUNCH_OBS
 #undef RDV_LAUNCH_P
 #undef RDV_LAUNCH_PT
@@ -1656,6 +1703,20 @@ int rdv_rollout(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, i
 #undef RDV_ROWS_SMEM
 #undef RDV_LAUNCH_K
     return launch_status();
+}
+
+int rdv_rollout(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, int64_t n, uint64_t seed,
+                int64_t env_offset, void *cuda_stream)
+{
+    return rollout_launch(p, s, io, nullptr, n, seed, env_offset, cuda_stream);
+}
+
+int rdv_rollout_trajectory(const RdvParams *p, const RdvState *s, const RdvRolloutIO *io, double *traj, int64_t n,
+                           uint64_t seed, int64_t env_offset, void *cuda_stream)
+{
+    if (!traj) return RDV_ERR_NULL;
+    if ((uintptr_t)traj & 7) return RDV_ERR_ALIGN;
+    return rollout_launch(p, s, io, traj, n, seed, env_offset, cuda_stream);
 }
 
 int rdv_reset(const RdvParams *p, const RdvState *s, const uint8_t *mask, const double *uniforms, float *obs,

@@ -253,6 +253,25 @@ RDV_DEV void eval_detail_of_state(const RdvParams &P, const EnvRegs &e, EvalDeta
                d.err[3] <= P.max_wd_error;
 }
 
+// one row of the trajectory record (rdv_rollout_trajectory): `row` points at column 0 of this env, columns are n apart
+RDV_DEV void store_traj_row(double *row, const int64_t n, const EnvRegs &e, const EnvCounters &c, const EvalDetail &d)
+{
+#pragma unroll
+    for (int k = 0; k < 3; ++k) { row[(RDV_RCX + k) * n] = e.rc[k]; row[(RDV_VCX + k) * n] = e.vc[k]; }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) { row[(RDV_QCW + k) * n] = e.qc[k]; row[(RDV_QTW + k) * n] = e.qt[k]; }
+#pragma unroll
+    for (int k = 0; k < 3; ++k) { row[(RDV_WCX + k) * n] = e.wc[k]; row[(RDV_WTX + k) * n] = e.wt[k]; }
+    row[RDV_TDV * n] = c.tdv; row[RDV_TDW * n] = c.tdw; row[RDV_EPRET * n] = c.ep_ret;
+    row[RDV_TR_I_STEP * n] = (double)c.step; row[RDV_TR_I_SUCCESS * n] = (double)c.success;
+    row[RDV_TR_I_COLLIDED * n] = (double)c.collided; row[RDV_TR_I_EPISODE * n] = (double)c.episode;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) row[(RDV_TR_POS_ERR + k) * n] = d.err[k];
+    row[RDV_TR_KOZ * n] = d.koz;
+    row[RDV_TR_COLLISION * n] = d.col_now ? 1.0 : 0.0;
+    row[RDV_TR_SUCCESS * n] = (!c.collided && d.within) ? 1.0 : 0.0;       // check_success with the sticky flag
+}
+
 RDV_DEV void load_counters(const RdvState &S, int64_t i, EnvCounters &c)
 {
     const int64_t ld = S.ld;

@@ -103,7 +103,7 @@ def evaluate(model, env, initial_state):
 
 
 def evaluate_batch(policy, initial_states, config=None, reward_kwargs=None, device="cuda", normalize_quaternions=True,
-                   return_raw=False, **extra) -> dict:
+                   return_raw=False, trajectories=False, **extra) -> dict:
     """All rows of ``initial_states`` ([M,20]: rc vc qc wc qt wt) as one GPU batch: ONE kernel launch and ONE
     device-to-host copy.  The launch is the policy-fused rollout in evaluator mode (``RdvRolloutIO.mc_out``): the actor
     runs on the tensor cores inside the kernel, and per-episode collision / success counts, the running minimum of
@@ -115,7 +115,12 @@ def evaluate_batch(policy, initial_states, config=None, reward_kwargs=None, devi
     ``policy`` may be a list or tuple of :class:`~.policy.MlpPolicy` (e.g. the checkpoints of a training run, or the models
     of a sweep): every model then runs all M initial conditions in its own block of envs, padded to a multiple of 128
     (one tile of the policy table; the padding rows are discarded), still in ONE launch with ONE read-back, and a list
-    with one result dict per model is returned.  Each dict equals what ``evaluate_batch(model, ...)`` returns."""
+    with one result dict per model is returned.  Each dict equals what ``evaluate_batch(model, ...)`` returns.
+
+    ``trajectories``: the same launch also records every env's fp64 trajectory (``rdv_rollout_trajectory``), and each
+    result dict gains ``trajectory``: the reference evaluator's per-step ``errors`` and ``times`` lists (and the state
+    behind them) for every episode at once, over L + 1 samples (L = ``done_steps``; sample 0 is the state at launch,
+    whose errors come from one :meth:`~.BatchedRendezvousEnv.errors` call before it).  See :func:`trajectory_fields`."""
     ics = np.array(initial_states, dtype=np.float64, copy=True).reshape(-1, 20)
     if normalize_quaternions:                                   # monte_carlo.py:66-67
         ics[:, 6:10] /= np.linalg.norm(ics[:, 6:10], axis=1, keepdims=True)
@@ -136,16 +141,50 @@ def evaluate_batch(policy, initial_states, config=None, reward_kwargs=None, devi
     env.reset()
     env.set_state(ics, reset_counters=False)        # flags stay as reset() left them (monte_carlo.py:106-112)
     tiles = None if models is None else np.repeat(np.arange(len(models)), block // N.POLICY_TILE)
-    out = env.rollout(int(p.done_steps), policy=policy, monte_carlo=True, policy_tiles=tiles)
+    row0 = _record_row_of_state(env) if trajectories else None
+    out = env.rollout(int(p.done_steps), policy=policy, monte_carlo=True, policy_tiles=tiles,
+                      record_trajectory=trajectories)
     mc = out["mc"].cpu().numpy()                    # the one read-back: [M, MC_NCOL] (models x block with a list)
+    rec = torch.cat([row0[None], out["trajectory"]]).cpu().numpy() if trajectories else None
     results = []
     for b in range(1 if models is None else len(models)):
         raw = mc[b * block:b * block + m]
         res = mc_columns(raw, p.dt)
         if return_raw:
             res["raw"] = raw
+        if trajectories:
+            res["trajectory"] = trajectory_fields(rec[:, :, b * block:b * block + m], p.dt)
         results.append(res)
     return results[0] if models is None else results
+
+
+def _record_row_of_state(env) -> torch.Tensor:
+    """The current state of every env as one row of the trajectory record, [TR_NCOL, N] on the device."""
+    n = env.num_envs
+    err, col, suc, koz = env.errors()
+    return torch.cat([env.f64[:N.NF64, :n], env.i32[:N.NI32, :n].double(), err.t(), koz[None], col[None].double(),
+                      suc[None].double()])
+
+
+def trajectory_fields(record: np.ndarray, dt: float) -> dict:
+    """[L + 1, TR_NCOL, M] trajectory record (sample 0 = the state at launch, then one row per step of an evaluator
+    launch) -> per-episode series, every array [M, L + 1, ...]: ``t`` (s, round(step * dt, 3) as RendezvousEnv.t),
+    ``rc vc wc wt`` [.., 3] and ``qc qt`` [.., 4] (the state), ``errors`` [.., 4] (get_errors: m, m/s, rad, rad/s),
+    ``dist_from_koz``, ``collision`` (check_collision), ``total_delta_v``, ``total_reward`` (the return so far);
+    ``length`` [M] is the episode length in steps.  Samples after ``length`` repeat the last one (a finished env stops
+    stepping)."""
+    rec = np.asarray(record, dtype=np.float64).transpose(2, 0, 1)          # [M, L + 1, TR_NCOL]
+    out = dict(t=np.round(rec[:, :, N.TR_I_STEP] * dt, 3))
+    for name, (row, k) in (("rc", (N.RCX, 3)), ("vc", (N.VCX, 3)), ("wc", (N.WCX, 3)), ("wt", (N.WTX, 3)),
+                           ("qc", (N.QCW, 4)), ("qt", (N.QTW, 4))):
+        out[name] = rec[:, :, row:row + k].copy()
+    out["errors"] = rec[:, :, N.TR_POS_ERR:N.TR_ROT_ERR + 1].copy()
+    out["dist_from_koz"] = rec[:, :, N.TR_KOZ].copy()
+    out["collision"] = rec[:, :, N.TR_COLLISION] != 0
+    out["total_delta_v"] = rec[:, :, N.TDV].copy()
+    out["total_reward"] = rec[:, :, N.EPRET].copy()
+    out["length"] = (rec[:, -1, N.TR_I_STEP] - rec[:, 0, N.TR_I_STEP]).astype(np.int64)
+    return out
 
 
 def mc_columns(mc: np.ndarray, dt: float) -> dict:
