@@ -45,7 +45,20 @@ enum {
  * max(bubble0 - step*rate, bubble_min) are derived from RDV_I_STEP (:193-198). */
 enum { RDV_I_STEP = 0, RDV_I_SUCCESS, RDV_I_COLLIDED, RDV_I_EPISODE, RDV_NI32 };
 
-/* Slots of the device statistics vector (double[RDV_NSTATS], accumulated with atomics). */
+/* Slots of the device statistics vector (double[RDV_NSTATS], accumulated with atomics).  Every entry point that
+ * takes `stats` adds to it by the same rules, whatever the kernel, launch shape or integrator:
+ *   STEPS, REWARD        every env-step taken, and its reward.  In the evaluator mode (RdvRolloutIO.mc_out) only the
+ *                        steps up to and including the env's first done.
+ *   EPISODES, END_*      env-steps that returned done, split by end reason.  Without auto-reset an env that keeps
+ *                        stepping past its end counts again at every such step.
+ *   RETURN, LENGTH,      at each such step: the episode return (RDV_EPRET), the step counter (RDV_I_STEP) and
+ *   DELTA_V, DELTA_W     total_delta_v / total_delta_w (RDV_TDV / RDV_TDW)
+ *   SUCCEEDED, COLLIDED  at each such step: success counter > 0, and the sticky collided flag
+ *   RK_ACCEPTED          accepted RK45 steps of every attitude solve that completed (a failed solve adds none)
+ *   RK_REJECTED          rejected RK45 attempts of every solve, failed or not; both RK slots stay 0 for
+ *                        RDV_INTEGRATOR_CLOSED_FORM
+ *   FAILURES             one per env-step in which any solve failed (non-finite error norm or TOO_SMALL_STEP), plus
+ *                        one per env-step of a policy-table tile that cannot be run */
 enum {
     RDV_S_STEPS = 0, RDV_S_EPISODES, RDV_S_RETURN, RDV_S_LENGTH, RDV_S_SUCCEEDED, RDV_S_COLLIDED,
     RDV_S_DELTA_V, RDV_S_DELTA_W,

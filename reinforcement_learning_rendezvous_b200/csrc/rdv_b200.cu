@@ -258,6 +258,7 @@ __global__ void __launch_bounds__(TPB, STEP_MIN_CTAS) step_kernel(const __grid_c
     const double pos_sq = pair_swap(part0), vel_sq = pair_swap(part1), rot_sq = pair_swap(part2);
     const double fuel_t = pair_swap(fuel), total_t = pair_swap(total);
     const int col_t = pair_swap(col_now);
+    const int fail_t = pair_swap(fail);
 
     // ---- observation (:205): each lane writes the slots it owns into the shared staging row ----
     float *o = s_obs + (threadIdx.x >> 1) * RDV_OBS_DIM;
@@ -306,7 +307,8 @@ __global__ void __launch_bounds__(TPB, STEP_MIN_CTAS) step_kernel(const __grid_c
             for (int k = 0; k < 3; ++k) { fw[(RDV_RCX + k) * ld] = rc[k]; fw[(RDV_VCX + k) * ld] = vc[k]; }
         }
     }
-    st.rk_acc = active ? rk_acc : 0; st.rk_rej = active ? rk_rej : 0; st.fail = active ? fail : 0;
+    // each lane counts its own body's RK steps; the chaser lane counts one failure for the env-step
+    st.rk_acc = active ? rk_acc : 0; st.rk_rej = active ? rk_rej : 0; st.fail = (active && !body) ? (fail | fail_t) : 0;
 
     // ---- chaser lane: latch, time, bubble, done, reward, outputs ----
     int done = 0, fin_pos = 0;

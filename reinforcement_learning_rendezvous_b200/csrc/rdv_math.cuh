@@ -836,7 +836,8 @@ RDV_DEV int rk45_iso_plane_pair_solve(double (&ya)[7], double (&yb)[7], const do
         ya[i] = fma(b[0], p[0][i], a[0] * q0[0][i]);
         yb[i] = fma(b[1], p[1][i], a[1] * q0[1][i]);
     }
-    return (failed[0] || failed[1]) ? -1 : accepted[0] + accepted[1];
+    return (failed[0] || failed[1]) ? -1 - (failed[0] ? 0 : accepted[0]) - (failed[1] ? 0 : accepted[1])
+                                    : accepted[0] + accepted[1];
 }
 // a pair with a body outside the polynomials' range: the two solves one after the other, each in its own form (the
 // same bits as in the lock-step form), out of line
@@ -844,8 +845,10 @@ __device__ __noinline__ int rk45_iso_plane_pair_mixed(double (&ya)[7], double (&
 {
     const int ka = rk45_iso_plane(ya, dt, n_rejected);
     const int kb = rk45_iso_plane(yb, dt, n_rejected);
-    return (ka < 0 || kb < 0) ? -1 : ka + kb;
+    return (ka < 0 || kb < 0) ? -1 - max(ka, 0) - max(kb, 0) : ka + kb;
 }
+// Both solves of an env: the accepted steps of both, or, when either failed, -1 - the accepted steps of the solve that
+// completed (a failed solve counts none).  Rejected attempts of both go to n_rejected, as one solve after the other.
 RDV_DEV int rk45_iso_plane_pair(double (&ya)[7], double (&yb)[7], const double dt, int &n_rejected)
 {
     if (!(plane_poly_covers(ya, dt) && plane_poly_covers(yb, dt))) return rk45_iso_plane_pair_mixed(ya, yb, dt, n_rejected);

@@ -81,7 +81,7 @@ RDV_DEV void env_attitude(const RdvParams &P, EnvRegs &e, const ActionTerms &t, 
         bt.I = P.inertia_t; bt.Iinv = P.inv_inertia_t; bt.tau = c_zero3;
         if (ISO && LOCKSTEP) {
             const int k = rk45_iso_plane_pair(y, z, P.dt, rk_rej);
-            if (k < 0) fail = 1; else rk_acc += k;
+            if (k < 0) { fail = 1; rk_acc += -1 - k; } else rk_acc += k;
         } else if (ISO) {
             // one solve after the other through a single copy of the solver code (bounded registers)
 #pragma unroll 1
@@ -94,7 +94,8 @@ RDV_DEV void env_attitude(const RdvParams &P, EnvRegs &e, const ActionTerms &t, 
         } else {
             const int kc = rk45_attitude<false>(y, P.dt, bc, rk_rej);
             const int kt = rk45_attitude<false>(z, P.dt, bt, rk_rej);
-            if (kc < 0 || kt < 0) fail = 1; else rk_acc += kc + kt;
+            if (kc < 0) fail = 1; else rk_acc += kc;
+            if (kt < 0) fail = 1; else rk_acc += kt;
         }
     }
     const double ry = fast_rsqrt(dot4(y, y)), rz = fast_rsqrt(dot4(z, z));       // q / |q|  (:574-575, :601-602)
