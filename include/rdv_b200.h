@@ -179,7 +179,8 @@ typedef struct RdvFinishedRow {
 int  rdv_abi_version(void);
 int  rdv_sizeof_params(void);
 /* sizeof of the ABI structs as this build sees them (a binding checks its own mirrors against these):
- * 0 RdvParams, 1 RdvState, 2 RdvStepIO, 3 RdvRolloutIO, 4 RdvPolicy, 5 RdvFinishedRow; -1 for anything else. */
+ * 0 RdvParams, 1 RdvState, 2 RdvStepIO, 3 RdvRolloutIO, 4 RdvPolicy, 5 RdvFinishedRow, 6 RdvLstmPolicy; -1 for
+ * anything else. */
 int  rdv_sizeof(int which);
 const char *rdv_strerror(int status);
 
@@ -322,6 +323,31 @@ int rdv_frame_transform(const double *q, const double *v, double *out, int64_t n
  * rdv_policy_forward_ffma: the same op as plain fp32 FMAs, one thread per env (numerics reference). */
 int rdv_policy_forward(const RdvPolicy *pi, const float *obs, float *actions, int64_t n, void *cuda_stream);
 int rdv_policy_forward_ffma(const RdvPolicy *pi, const float *obs, float *actions, int64_t n, void *cuda_stream);
+
+/* -- recurrent actor (sb3_contrib RecurrentPPO "MlpLstmPolicy", main_rnn.py) ---------------------------------------
+ * Weights of the actor of a RecurrentActorCriticPolicy with one 256-wide LSTM layer and the default pi = [64, 64] Tanh
+ * head.  Row-major [out][in] as in torch; the gate rows of the LSTM are in torch's order i, f, g, o. */
+typedef struct RdvLstmPolicy {
+    const float *weight_ih, *weight_hh;   /* lstm_actor.weight_ih_l0 [4H][17], weight_hh_l0 [4H][H]            */
+    const float *bias_ih, *bias_hh;       /* lstm_actor.bias_ih_l0 [4H], bias_hh_l0 [4H]                        */
+    const float *w0, *b0;                 /* mlp_extractor.policy_net.0: [64][H], [64]                          */
+    const float *w1, *b1;                 /* mlp_extractor.policy_net.2: [64][64], [64]                         */
+    const float *w2, *b2;                 /* action_net: [6][64], [6]                                           */
+    int32_t hidden;                       /* H, must be 256                                                     */
+    int32_t reserved;
+} RdvLstmPolicy;
+/* One deterministic actor step of RecurrentActorCriticPolicy.predict for n envs:
+ *   h, c = 0 where episode_start[i] != 0 (sb3_contrib multiplies the state by 1 - episode_start)
+ *   z = W_ih obs + b_ih + W_hh h + b_hh;  c' = sigmoid(f) c + sigmoid(i) tanh(g);  h' = sigmoid(o) tanh(c')
+ *   actions = clip(W2 tanh(W1 tanh(W0 h' + b0) + b1) + b2, -1, 1)
+ * obs [n][17], actions [n][6] float32; h_in, c_in, h_out, c_out float32 [H][ld] (structure of arrays like RdvState,
+ * element (j, i) at [j * ld + i]); episode_start nullable [n] (NULL: no env starts an episode).  The outputs are
+ * separate buffers from the inputs.  Every product runs on the tensor cores as three MMAs of fp16 halves with fp32
+ * accumulation (fp32-level accuracy); the weights are staged times 2^10, so every weight and bias must be below 64 in
+ * magnitude (not checked here).  Only H = 256 with the 64-64 head is supported (RDV_ERR_UNSUPPORTED). */
+int rdv_lstm_policy_step(const RdvLstmPolicy *pi, const float *obs, const uint8_t *episode_start,
+                         const float *h_in, const float *c_in, float *h_out, float *c_out, float *actions,
+                         int64_t n, int64_t ld, void *cuda_stream);
 
 /* Development / test knobs that used to be environment variables (read once at load as defaults); every setting gives
  * the same bits.  Returns the previous value, or RDV_ERR_SIZE for an unknown key.

@@ -8,6 +8,7 @@ Public surface (mirrors the reference, see INTEGRATION.md):
 * ``make_env`` / ``copy_env`` factory with the reference signature (utils/environment_utils.py)
 * ``MlpPolicy``               fused fp32 policy forward (model.predict, monte_carlo.py:128-133)
 * ``PolicyTable``             several MlpPolicy actors in one fused rollout (one per 128-env tile)
+* ``LstmPolicy``              RecurrentPPO MlpLstmPolicy actor on the tensor cores (main_rnn.py; predict with state)
 * ``evaluate`` / ``evaluate_batch``  Monte-Carlo evaluator (monte_carlo.py:94-207)
 * ``ppo.PPO``                 device-tensor PPO loop with main.py's hyper-parameters (main.py:39-48, :114-118)
 
@@ -33,7 +34,7 @@ def __getattr__(name):
     if name in ("make_env", "make_vec_env", "copy_env"):
         from . import environment_utils
         return getattr(environment_utils, name)
-    if name in ("MlpPolicy", "PolicyTable"):
+    if name in ("MlpPolicy", "PolicyTable", "LstmPolicy"):
         from . import policy
         return getattr(policy, name)
     if name in ("evaluate", "evaluate_batch", "evaluate_sweep", "sensitivity_grid"):
@@ -43,4 +44,4 @@ def __getattr__(name):
 
 
 __all__ = ["BatchedRendezvousEnv", "RendezvousEnv", "RendezvousVecEnv", "make_env", "make_vec_env", "copy_env",
-           "MlpPolicy", "PolicyTable", "evaluate", "evaluate_batch", "evaluate_sweep", "sensitivity_grid", "make_params", "build_native"]
+           "MlpPolicy", "PolicyTable", "LstmPolicy", "evaluate", "evaluate_batch", "evaluate_sweep", "sensitivity_grid", "make_params", "build_native"]

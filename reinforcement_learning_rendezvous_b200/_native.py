@@ -25,7 +25,8 @@ LIB_PATH = os.environ.get("RDV_B200_LIB") or os.path.join(CSRC_DIR, "librdv_b200
 HOST_SRC = os.path.join(CSRC_DIR, "rdv_host.c")                 # CPython helper of RendezvousVecEnv (gcc, no CUDA)
 HOST_LIB = os.path.join(PKG_DIR, "_rdv_host" + (sysconfig.get_config_var("EXT_SUFFIX") or ".so"))
 SOURCES = ("rdv_b200.cu",)
-HEADERS = ("rdv_math.cuh", "rdv_plane_poly.h", "rdv_env.cuh", "rdv_step.cuh", "rdv_policy.cuh", "rdv_policy_tc.cuh")
+HEADERS = ("rdv_math.cuh", "rdv_plane_poly.h", "rdv_env.cuh", "rdv_step.cuh", "rdv_policy.cuh", "rdv_policy_tc.cuh",
+           "rdv_lstm.cuh")
 
 ABI_VERSION = 16
 OBS_DIM, ACT_DIM, N_UNIFORMS = 17, 6, 24
@@ -106,6 +107,17 @@ class RdvPolicy(C.Structure):
     ]
 
 
+class RdvLstmPolicy(C.Structure):
+    _fields_ = [
+        ("weight_ih", C.c_void_p), ("weight_hh", C.c_void_p), ("bias_ih", C.c_void_p), ("bias_hh", C.c_void_p),
+        ("w0", C.c_void_p), ("b0", C.c_void_p), ("w1", C.c_void_p), ("b1", C.c_void_p),
+        ("w2", C.c_void_p), ("b2", C.c_void_p), ("hidden", C.c_int32), ("reserved", C.c_int32),
+    ]
+
+
+LSTM_HIDDEN = 256               # the only LSTM width rdv_lstm_policy_step supports
+
+
 class RdvRolloutIO(C.Structure):
     _fields_ = [
         ("steps", C.c_int32), ("action_source", C.c_int32), ("auto_reset", C.c_int32), ("reserved", C.c_int32),
@@ -156,6 +168,8 @@ PROTOTYPES = {
     "rdv_frame_transform": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "rdv_policy_forward": (C.c_int, [C.POINTER(RdvPolicy), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "rdv_policy_forward_ffma": (C.c_int, [C.POINTER(RdvPolicy), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "rdv_lstm_policy_step": (C.c_int, [C.POINTER(RdvLstmPolicy), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]),
     "rdv_math_probe": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "rdv_fp64_peak_probe": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
 }
@@ -234,7 +248,8 @@ def lib():
             fn.restype, fn.argtypes = res, args
         if L.rdv_abi_version() != ABI_VERSION:
             raise RuntimeError(f"librdv_b200.so ABI {L.rdv_abi_version()} != binding ABI {ABI_VERSION}; rebuild")
-        for which, mirror in enumerate((RdvParams, RdvState, RdvStepIO, RdvRolloutIO, RdvPolicy, RdvFinishedRow)):
+        for which, mirror in enumerate((RdvParams, RdvState, RdvStepIO, RdvRolloutIO, RdvPolicy, RdvFinishedRow,
+                                         RdvLstmPolicy)):
             if L.rdv_sizeof(which) != C.sizeof(mirror):
                 raise RuntimeError(f"{mirror.__name__} layout mismatch between include/rdv_b200.h "
                                    f"({L.rdv_sizeof(which)} B) and _native.py ({C.sizeof(mirror)} B)")

@@ -285,7 +285,10 @@ class BatchedRendezvousEnv:
             source = N.ACTIONS_F64 if actions.dtype == torch.float64 else N.ACTIONS_F32
             esz = 8 if actions.dtype == torch.float64 else 4
         elif policy is not None:
-            from .policy import PolicyTable
+            from .policy import LstmPolicy, PolicyTable
+            if isinstance(policy, LstmPolicy):
+                raise TypeError("the fused rollout runs MlpPolicy actors only; evaluate an LstmPolicy with "
+                                "monte_carlo.evaluate_batch or step it with LstmPolicy.forward")
             if policy.device != dev:
                 raise ValueError("policy and env live on different devices")
             if isinstance(policy, PolicyTable):

@@ -22,6 +22,7 @@
 #include "rdv_step.cuh"
 #include "rdv_policy.cuh"
 #include "rdv_policy_tc.cuh"
+#include "rdv_lstm.cuh"
 
 namespace rdv {
 
@@ -1379,6 +1380,7 @@ int rdv_sizeof(int which)
         case 3: return (int)sizeof(RdvRolloutIO);
         case 4: return (int)sizeof(RdvPolicy);
         case 5: return (int)sizeof(RdvFinishedRow);
+        case 6: return (int)sizeof(RdvLstmPolicy);
         default: return -1;
     }
 }
@@ -1822,6 +1824,35 @@ int rdv_policy_forward_ffma(const RdvPolicy *pi, const float *obs, float *action
     static std::atomic<uint64_t> attr_mask{0};
     if (!ensure_smem(policy_kernel, attr_mask, dev, smem)) return RDV_ERR_CUDA;
     policy_kernel<<<(unsigned)((n + PTPB - 1) / PTPB), PTPB, smem, (cudaStream_t)cuda_stream>>>(*pi, obs, actions, n);
+    return launch_status();
+}
+
+int rdv_lstm_policy_step(const RdvLstmPolicy *pi, const float *obs, const uint8_t *episode_start,
+                         const float *h_in, const float *c_in, float *h_out, float *c_out, float *actions,
+                         int64_t n, int64_t ld, void *cuda_stream)
+{
+    if (!pi || !obs || !h_in || !c_in || !h_out || !c_out || !actions) return RDV_ERR_NULL;
+    const float *w[] = {pi->weight_ih, pi->weight_hh, pi->bias_ih, pi->bias_hh, pi->w0, pi->b0, pi->w1, pi->b1,
+                        pi->w2, pi->b2};
+    for (const float *p : w)
+        if (!p) return RDV_ERR_NULL;
+    if (n < 0 || ld < n) return RDV_ERR_SIZE;
+    const void *f[] = {obs, h_in, c_in, h_out, c_out, actions};
+    for (const void *p : f)
+        if ((uintptr_t)p & 3) return RDV_ERR_ALIGN;
+    for (const float *p : w)
+        if ((uintptr_t)p & 3) return RDV_ERR_ALIGN;
+    if (pi->hidden != tc::LH) return RDV_ERR_UNSUPPORTED;
+    if (n == 0) return RDV_OK;
+    int sm_count = 0;
+    const int dev = current_device(&sm_count);
+    if (dev < 0) return RDV_ERR_CUDA;
+    static std::atomic<uint64_t> attr_mask{0};
+    if (!ensure_smem(tc::lstm_step_kernel, attr_mask, dev, sizeof(tc::LstmSmem))) return RDV_ERR_CUDA;
+    const int64_t pairs = ((n + tc::TM - 1) / tc::TM + tc::LSTM_TILES - 1) / tc::LSTM_TILES;
+    const unsigned grid = (unsigned)(pairs < sm_count ? pairs : sm_count);
+    tc::lstm_step_kernel<<<grid, tc::LSTM_THREADS, sizeof(tc::LstmSmem), (cudaStream_t)cuda_stream>>>(
+        *pi, obs, episode_start, h_in, c_in, h_out, c_out, actions, n, ld);
     return launch_status();
 }
 

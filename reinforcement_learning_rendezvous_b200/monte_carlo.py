@@ -14,7 +14,7 @@ import torch
 from . import _native as N
 from .batched_env import BatchedRendezvousEnv
 from .environment_utils import config_to_kwargs
-from .policy import PolicyTable
+from .policy import LstmPolicy, PolicyTable
 
 MC_COLS = ("ep_len", "num_collisions", "collided", "total_reward", "total_delta_v", "num_successes", "succeeded",
            "min_dist_from_koz", "pos_error", "vel_error", "att_error", "rot_error")
@@ -117,6 +117,12 @@ def evaluate_batch(policy, initial_states, config=None, reward_kwargs=None, devi
     (one tile of the policy table; the padding rows are discarded), still in ONE launch with ONE read-back, and a list
     with one result dict per model is returned.  Each dict equals what ``evaluate_batch(model, ...)`` returns.
 
+    ``policy`` may also be a recurrent :class:`~.policy.LstmPolicy` (RecurrentPPO's MlpLstmPolicy): the same columns and
+    arguments, computed with one actor-step and one one-step rollout launch per step (see ``_evaluate_batch_lstm``)
+    and still one read-back.  A list of them is not supported.  With ``return_raw`` its ``raw`` array has the
+    evaluator mode's [M, MC_NCOL] layout, but the reduction runs on the host from the trajectory record, which carries
+    no end reason: ``MC_LEVEL``, ``MC_TAIL_COUNT`` and ``MC_END_REASON`` are NaN there; every other column is filled.
+
     ``trajectories``: the same launch also records every env's fp64 trajectory (``rdv_rollout_trajectory``), and each
     result dict gains ``trajectory``: the reference evaluator's per-step ``errors`` and ``times`` lists (and the state
     behind them) for every episode at once, over L + 1 samples (L = ``done_steps``; sample 0 is the state at launch,
@@ -126,6 +132,8 @@ def evaluate_batch(policy, initial_states, config=None, reward_kwargs=None, devi
         ics[:, 6:10] /= np.linalg.norm(ics[:, 6:10], axis=1, keepdims=True)
         ics[:, 13:17] /= np.linalg.norm(ics[:, 13:17], axis=1, keepdims=True)
     m = ics.shape[0]
+    if isinstance(policy, LstmPolicy):
+        return _evaluate_batch_lstm(policy, ics, config, reward_kwargs, device, return_raw, trajectories, extra)
     models = list(policy) if isinstance(policy, (list, tuple)) else None
     block = m
     if models is not None:
@@ -156,6 +164,72 @@ def evaluate_batch(policy, initial_states, config=None, reward_kwargs=None, devi
             res["trajectory"] = trajectory_fields(rec[:, :, b * block:b * block + m], p.dt)
         results.append(res)
     return results[0] if models is None else results
+
+
+def _evaluate_batch_lstm(policy, ics, config, reward_kwargs, device, return_raw, trajectories, extra) -> dict:
+    """``evaluate_batch`` with a recurrent :class:`~.policy.LstmPolicy`, by ``evaluate``'s rules (monte_carlo.py:94-207
+    with RecurrentPPO's predict): the state is injected after ``reset()`` without refreshing the flags, the LSTM state
+    starts at zero (``episode_start`` True), then ``episode_start`` is the last ``done``, and the episode ends at the
+    first ``done``.  Each of the ``done_steps`` steps is one ``rdv_lstm_policy_step`` and one ``rdv_rollout_trajectory``
+    launch of one step (float32 actions, no auto-reset) that records the state and its errors; envs keep stepping past
+    their first done, and the per-episode columns are reduced from the record up to it after ONE read-back."""
+    m = ics.shape[0]
+    kw = config_to_kwargs(dict(dt=1, t_max=60) if config is None else config, stochastic=False)
+    env = BatchedRendezvousEnv(m, device=device, auto_reset=False, track_stats=False, reward_kwargs=reward_kwargs,
+                               **kw, **extra)
+    p = env.params
+    if policy.device != env.device:
+        raise ValueError("policy and env live on different devices")
+    env.reset()
+    env.set_state(ics, reset_counters=False)        # flags stay as reset() left them (monte_carlo.py:106-112)
+    steps, dev = int(p.done_steps), env.device
+    rec = torch.empty((steps + 1, N.TR_NCOL, m), dtype=torch.float64, device=dev)
+    dones = torch.empty((steps, m), dtype=torch.float64, device=dev)
+    rec[0] = _record_row_of_state(env)
+    obs = env.observe()
+    (h, c), (h_next, c_next) = policy.initial_state(m), policy.initial_state(m)
+    act = torch.empty((1, m, N.ACT_DIM), dtype=torch.float32, device=dev)
+    start = torch.ones(m, dtype=torch.uint8, device=dev)
+    for k in range(steps):
+        policy.forward(obs, h, c, start, out=(act[0], h_next, c_next))
+        out = env.rollout(1, actions=act, record_dones=True, record_trajectory=True)
+        rec[k + 1] = out["trajectory"][0]
+        start = out["dones"][0]
+        dones[k] = start
+        obs = out["obs"]
+        h, c, h_next, c_next = h_next, c_next, h, c
+    host = torch.cat([rec.reshape(-1), dones.reshape(-1)]).cpu().numpy()     # the one read-back
+    rec = host[:rec.numel()].reshape(steps + 1, N.TR_NCOL, m)
+    done = host[rec.size:].reshape(steps, m) != 0
+    length = np.where(done.any(axis=0), done.argmax(axis=0) + 1, steps)     # steps up to the first done
+    # freeze every env at its first done, as the evaluator mode of the fused rollout does
+    rec = rec[np.minimum(np.arange(steps + 1)[:, None], length[None, :]), :, np.arange(m)[None, :]].transpose(0, 2, 1)
+    cols = rec.transpose(2, 1, 0)                                             # [M, TR_NCOL, L + 1]
+    valid = np.arange(steps + 1)[None, :] <= length[:, None]                  # samples 0 .. length
+    last = rec[-1].T                                                          # [M, TR_NCOL]: the state at the end
+    n_col = ((cols[:, N.TR_COLLISION] != 0) & valid).sum(axis=1)
+    n_suc = ((cols[:, N.TR_SUCCESS] != 0) & valid).sum(axis=1)               # success honours the collided flag
+    limits = (p.max_rd_error, p.max_vd_error, p.max_qd_error, p.max_wd_error)
+    te = _terminal_errors_batch(rec[:, N.TR_POS_ERR:N.TR_ROT_ERR + 1].transpose(0, 2, 1), length, limits)
+    res = dict(ep_len=np.round(length * p.dt, 3), num_collisions=n_col, collided=(n_col > 0).astype(np.int64),
+               total_reward=last[:, N.EPRET].copy(), total_delta_v=last[:, N.TDV].copy(), num_successes=n_suc,
+               succeeded=(n_suc > 0).astype(np.int64),
+               min_dist_from_koz=np.where(valid, cols[:, N.TR_KOZ], np.inf).min(axis=1),
+               pos_error=te[:, 0], vel_error=te[:, 1], att_error=te[:, 2], rot_error=te[:, 3])
+    if return_raw:
+        # the [M, MC_NCOL] layout of the evaluator mode; LEVEL, TAIL_COUNT and END_REASON are not reduced here (NaN)
+        raw = np.full((m, N.MC_NCOL), np.nan)
+        for col, v in ((N.MC_EP_LEN, length), (N.MC_NUM_COLLISIONS, n_col), (N.MC_COLLIDED, res["collided"]),
+                       (N.MC_TOTAL_REWARD, res["total_reward"]), (N.MC_TOTAL_DELTA_V, res["total_delta_v"]),
+                       (N.MC_NUM_SUCCESSES, n_suc), (N.MC_SUCCEEDED, res["succeeded"]),
+                       (N.MC_MIN_KOZ, res["min_dist_from_koz"]), (N.MC_POS_ERR, te[:, 0]), (N.MC_VEL_ERR, te[:, 1]),
+                       (N.MC_ATT_ERR, np.radians(te[:, 2])), (N.MC_ROT_ERR, np.radians(te[:, 3])),
+                       (N.MC_TOTAL_DELTA_W, last[:, N.TDW])):
+            raw[:, col] = v
+        res["raw"] = raw
+    if trajectories:
+        res["trajectory"] = trajectory_fields(rec, p.dt)
+    return res
 
 
 def _record_row_of_state(env) -> torch.Tensor:
