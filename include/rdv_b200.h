@@ -355,9 +355,10 @@ int rdv_lstm_policy_step(const RdvLstmPolicy *pi, const float *obs, const uint8_
  *   RDV_TUNE_RESET_REFILL     reset prefetch period in steps (0 = reset on demand only; default 12)
  *   RDV_TUNE_ROLLOUT_PDL      1 (default): rdv_rollout launches with programmatic stream serialisation, so the
  *                             prologue of a launch overlaps the tail of the previous kernel; 0: plain launch
- *   RDV_TUNE_ROLLOUT_HELPERS  1 (default): launches of 385..448 envs per SM in one pass (65,536 envs on a B200) run
- *                             with two helper warps per CTA that recompute the used reset rows beside the 14 worker
- *                             warps; 0: the workers refill their rows themselves every RESET_REFILL steps */
+ *   RDV_TUNE_ROLLOUT_HELPERS  1: launches of 385..448 envs per SM in one pass (65,536 envs on a B200) run with two
+ *                             helper warps per CTA that recompute the used reset rows beside the 14 worker warps;
+ *                             0 (default, the faster one on B200): the workers refill their rows themselves every
+ *                             RESET_REFILL steps */
 enum { RDV_TUNE_ROLLOUT_TPB = 0, RDV_TUNE_RESET_REFILL = 1, RDV_TUNE_ROLLOUT_PDL = 2, RDV_TUNE_ROLLOUT_HELPERS = 3 };
 int rdv_tune(int key, int value);
 

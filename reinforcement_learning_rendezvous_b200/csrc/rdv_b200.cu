@@ -462,7 +462,11 @@ __global__ void __launch_bounds__(TPB, STEP_MIN_CTAS) step_kernel(const __grid_c
 constexpr int SYNC_PERIOD = 8;            // steps between the CTA barriers that keep the warps in one code region
 constexpr int HELP_POST_PERIOD = 3;       // helper-warp variant: steps between the workers' request posts (1: 12 % slower, 2-4 alike)
 constexpr int HELP_IDLE_NS = 500;         // helper-warp variant: sleep of an idle helper between polls
-constexpr int LOCKSTEP_MAX_TPB = 256;     // CTAs up to this size interleave the two attitude solves (rk45_iso_plane_pair)
+// CTAs up to this size interleave the two attitude solves (rk45_iso_plane_pair).  Measured on B200 with every
+// variant above it in lock-step (profiles/r08_lockstep_timing.txt, 250-step launches): 448 + helpers 8.69 -> 9.06 us
+// per step, plain 448 7.62 -> 8.37, 512 8.11 -> 9.41, 384 6.00 -> 6.06, fused policy at 448 / 512 16.9 -> 19.2 / 17.6,
+// at 384 12.34 -> 12.27 (within noise, so 384 keeps the sequential form with the other big CTAs).
+constexpr int LOCKSTEP_MAX_TPB = 256;
 constexpr int RDV_NEXT_ROW = 22;          // doubles per prefetched reset row: state[20], collided, success
 constexpr int RDV_ROW_TAG = 22;           // row of RdvRolloutIO.reset_rows holding the episode index a row belongs to
 
@@ -1356,7 +1360,7 @@ static int env_int(const char *name, int fallback)
 static std::atomic<int> g_tune_tpb{env_int("RDV_ROLLOUT_TPB", 0)};
 static std::atomic<int> g_tune_refill{env_int("RDV_RESET_REFILL", 12)};
 static std::atomic<int> g_tune_pdl{env_int("RDV_ROLLOUT_PDL", 1)};
-static std::atomic<int> g_tune_helpers{env_int("RDV_ROLLOUT_HELPERS", 1)};
+static std::atomic<int> g_tune_helpers{env_int("RDV_ROLLOUT_HELPERS", 0)};   // off: DESIGN 4.3, "Helper warps"
 
 extern "C" {
 

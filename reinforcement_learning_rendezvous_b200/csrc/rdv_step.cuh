@@ -48,7 +48,8 @@ RDV_DEV void ingest_action_f32(const RdvParams &P, const float (&a)[6], EnvCount
 // two attitude propagations (:552-604).  LOCKSTEP: the two isotropic solves advance interleaved stage by stage
 // (rk45_iso_plane_pair, 2x ILP) -- the right choice with <= 2 warps per SM sub-partition; otherwise one solve after
 // the other through a single copy of the solver (rk45_iso_plane, 128 registers), which wins once 3-4 warps per
-// sub-partition hide the latency instead.
+// sub-partition hide the latency instead.  This still holds with the closed-form attempt: the pair fits 128 registers
+// at 448 and 512 threads and is 4-16 % slower there (DESIGN 4.3, profiles/r08_lockstep_timing.txt).
 // first half of env_advance: the impulse rotated by the OLD chaser attitude, then the CW transition
 RDV_DEV void env_translate(const RdvParams &P, EnvRegs &e, const ActionTerms &t)
 {
