@@ -179,8 +179,8 @@ typedef struct RdvFinishedRow {
 int  rdv_abi_version(void);
 int  rdv_sizeof_params(void);
 /* sizeof of the ABI structs as this build sees them (a binding checks its own mirrors against these):
- * 0 RdvParams, 1 RdvState, 2 RdvStepIO, 3 RdvRolloutIO, 4 RdvPolicy, 5 RdvFinishedRow, 6 RdvLstmPolicy; -1 for
- * anything else. */
+ * 0 RdvParams, 1 RdvState, 2 RdvStepIO, 3 RdvRolloutIO, 4 RdvPolicy, 5 RdvFinishedRow, 6 RdvLstmPolicy,
+ * 7 RdvLstmActorCritic, 8 RdvLstmStepIO; -1 for anything else. */
 int  rdv_sizeof(int which);
 const char *rdv_strerror(int status);
 
@@ -348,6 +348,43 @@ typedef struct RdvLstmPolicy {
 int rdv_lstm_policy_step(const RdvLstmPolicy *pi, const float *obs, const uint8_t *episode_start,
                          const float *h_in, const float *c_in, float *h_out, float *c_out, float *actions,
                          int64_t n, int64_t ld, void *cuda_stream);
+
+/* Weights of a whole RecurrentActorCriticPolicy (sb3_contrib's MlpLstmPolicy with its default separate critic LSTM):
+ * the actor as above, the Gaussian head's log_std, and the critic in the same layout -- lstm_critic.*, then
+ * mlp_extractor.value_net.0 / .2 in w0, b0 / w1, b1 and value_net in w2 [1][64], b2 [1]. */
+typedef struct RdvLstmActorCritic {
+    RdvLstmPolicy actor;                  /* lstm_actor, mlp_extractor.policy_net, action_net                      */
+    const float *log_std;                 /* [6]                                                                   */
+    RdvLstmPolicy critic;                 /* lstm_critic, mlp_extractor.value_net, value_net (w2 [1][64], b2 [1])  */
+} RdvLstmActorCritic;
+/* Buffers of one collection step (rdv_lstm_actor_critic_step).  State buffers are float32 [H][ld] like those of
+ * rdv_lstm_policy_step; every *_out is a separate buffer from every input. */
+typedef struct RdvLstmStepIO {
+    const float *obs;                     /* [n][17]                                                               */
+    const uint8_t *episode_start;         /* nullable [n]: zero both networks' state of these envs first           */
+    const float *h_pi, *c_pi;             /* actor state in                                                        */
+    float *h_pi_out, *c_pi_out;           /* actor state out                                                       */
+    const float *h_vf, *c_vf;             /* critic state in                                                       */
+    float *h_vf_out, *c_vf_out;           /* critic state out                                                      */
+    float *actions;                       /* [n][6] the unclipped draw (what the rollout buffer stores)            */
+    float *env_actions;                   /* nullable [n][6] clip(actions, -1, 1) (what env.step gets)             */
+    float *log_prob;                      /* [n] log-density of the draw                                           */
+    float *values;                        /* [n] critic value                                                      */
+    uint64_t action_seed;                 /* Philox key of the Gaussian noise                                      */
+    int64_t step_index;                   /* noise counter of this step                                            */
+    int64_t env_offset;                   /* global index of env 0 (noise counter)                                 */
+    int64_t ld;                           /* leading dimension of the eight state buffers, >= n                    */
+} RdvLstmStepIO;
+/* One step of RecurrentActorCriticPolicy.forward for n envs, what sb3_contrib's collect_rollouts calls per step, in ONE
+ * launch: CTAs [0, G) run the actor, CTAs [G, 2G) the critic, both with the episode-start zeroing and the LSTM step of
+ * rdv_lstm_policy_step (the actor's h', c' are bit-identical to it).  Actor: mean = action_net(tanh(W1 tanh(W0 h'))),
+ * unclipped; z = the six N(0,1) draws of (action_seed; env_offset + i, step_index) -- the stream and counter layout of
+ * RDV_ACTIONS_POLICY_SAMPLE --; actions = mean + exp(log_std) z, env_actions = clip(actions, -1, 1),
+ * log_prob = sum_j (-z_j^2 / 2 - log_std_j) - 3 ln(2 pi).  Critic: values = value_net(tanh(W1 tanh(W0 h_vf'))), no
+ * clip.  The same precision and weight limit (below 64 in magnitude, not checked here) as rdv_lstm_policy_step.
+ * Returns RDV_ERR_NULL / SIZE (n < 0, ld < n) / ALIGN (a float pointer not 4-byte aligned) / UNSUPPORTED (hidden of
+ * either network != 256); allocates nothing. */
+int rdv_lstm_actor_critic_step(const RdvLstmActorCritic *w, const RdvLstmStepIO *io, int64_t n, void *cuda_stream);
 
 /* Development / test knobs that used to be environment variables (read once at load as defaults); every setting gives
  * the same bits.  Returns the previous value, or RDV_ERR_SIZE for an unknown key.

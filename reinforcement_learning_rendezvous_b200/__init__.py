@@ -11,6 +11,7 @@ Public surface (mirrors the reference, see INTEGRATION.md):
 * ``LstmPolicy``              RecurrentPPO MlpLstmPolicy actor on the tensor cores (main_rnn.py; predict with state)
 * ``evaluate`` / ``evaluate_batch``  Monte-Carlo evaluator (monte_carlo.py:94-207)
 * ``ppo.PPO``                 device-tensor PPO loop with main.py's hyper-parameters (main.py:39-48, :114-118)
+* ``RecurrentPPO``            device-tensor RecurrentPPO loop for main_rnn.py's MlpLstmPolicy (sb3_contrib's update)
 
 Importing the package needs neither a GPU nor the built library; using it does.  There is
 no CPU fallback.
@@ -37,6 +38,9 @@ def __getattr__(name):
     if name in ("MlpPolicy", "PolicyTable", "LstmPolicy"):
         from . import policy
         return getattr(policy, name)
+    if name in ("RecurrentPPO", "RecurrentPPOConfig", "RecurrentActorCritic"):
+        from . import recurrent_ppo
+        return getattr(recurrent_ppo, name)
     if name in ("evaluate", "evaluate_batch", "evaluate_sweep", "sensitivity_grid"):
         from . import monte_carlo
         return getattr(monte_carlo, name)
@@ -44,4 +48,4 @@ def __getattr__(name):
 
 
 __all__ = ["BatchedRendezvousEnv", "RendezvousEnv", "RendezvousVecEnv", "make_env", "make_vec_env", "copy_env",
-           "MlpPolicy", "PolicyTable", "LstmPolicy", "evaluate", "evaluate_batch", "evaluate_sweep", "sensitivity_grid", "make_params", "build_native"]
+           "MlpPolicy", "PolicyTable", "LstmPolicy", "RecurrentPPO", "RecurrentPPOConfig", "RecurrentActorCritic", "evaluate", "evaluate_batch", "evaluate_sweep", "sensitivity_grid", "make_params", "build_native"]

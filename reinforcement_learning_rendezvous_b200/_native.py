@@ -118,6 +118,20 @@ class RdvLstmPolicy(C.Structure):
 LSTM_HIDDEN = 256               # the only LSTM width rdv_lstm_policy_step supports
 
 
+class RdvLstmActorCritic(C.Structure):
+    _fields_ = [("actor", RdvLstmPolicy), ("log_std", C.c_void_p), ("critic", RdvLstmPolicy)]
+
+
+class RdvLstmStepIO(C.Structure):
+    _fields_ = [
+        ("obs", C.c_void_p), ("episode_start", C.c_void_p),
+        ("h_pi", C.c_void_p), ("c_pi", C.c_void_p), ("h_pi_out", C.c_void_p), ("c_pi_out", C.c_void_p),
+        ("h_vf", C.c_void_p), ("c_vf", C.c_void_p), ("h_vf_out", C.c_void_p), ("c_vf_out", C.c_void_p),
+        ("actions", C.c_void_p), ("env_actions", C.c_void_p), ("log_prob", C.c_void_p), ("values", C.c_void_p),
+        ("action_seed", C.c_uint64), ("step_index", C.c_int64), ("env_offset", C.c_int64), ("ld", C.c_int64),
+    ]
+
+
 class RdvRolloutIO(C.Structure):
     _fields_ = [
         ("steps", C.c_int32), ("action_source", C.c_int32), ("auto_reset", C.c_int32), ("reserved", C.c_int32),
@@ -170,6 +184,8 @@ PROTOTYPES = {
     "rdv_policy_forward_ffma": (C.c_int, [C.POINTER(RdvPolicy), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "rdv_lstm_policy_step": (C.c_int, [C.POINTER(RdvLstmPolicy), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]),
+    "rdv_lstm_actor_critic_step": (C.c_int, [C.POINTER(RdvLstmActorCritic), C.POINTER(RdvLstmStepIO), C.c_int64,
+                                             C.c_void_p]),
     "rdv_math_probe": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "rdv_fp64_peak_probe": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
 }
@@ -249,7 +265,7 @@ def lib():
         if L.rdv_abi_version() != ABI_VERSION:
             raise RuntimeError(f"librdv_b200.so ABI {L.rdv_abi_version()} != binding ABI {ABI_VERSION}; rebuild")
         for which, mirror in enumerate((RdvParams, RdvState, RdvStepIO, RdvRolloutIO, RdvPolicy, RdvFinishedRow,
-                                         RdvLstmPolicy)):
+                                         RdvLstmPolicy, RdvLstmActorCritic, RdvLstmStepIO)):
             if L.rdv_sizeof(which) != C.sizeof(mirror):
                 raise RuntimeError(f"{mirror.__name__} layout mismatch between include/rdv_b200.h "
                                    f"({L.rdv_sizeof(which)} B) and _native.py ({C.sizeof(mirror)} B)")

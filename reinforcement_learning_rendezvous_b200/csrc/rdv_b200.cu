@@ -1385,6 +1385,8 @@ int rdv_sizeof(int which)
         case 4: return (int)sizeof(RdvPolicy);
         case 5: return (int)sizeof(RdvFinishedRow);
         case 6: return (int)sizeof(RdvLstmPolicy);
+        case 7: return (int)sizeof(RdvLstmActorCritic);
+        case 8: return (int)sizeof(RdvLstmStepIO);
         default: return -1;
     }
 }
@@ -1852,11 +1854,49 @@ int rdv_lstm_policy_step(const RdvLstmPolicy *pi, const float *obs, const uint8_
     const int dev = current_device(&sm_count);
     if (dev < 0) return RDV_ERR_CUDA;
     static std::atomic<uint64_t> attr_mask{0};
-    if (!ensure_smem(tc::lstm_step_kernel, attr_mask, dev, sizeof(tc::LstmSmem))) return RDV_ERR_CUDA;
+    if (!ensure_smem(tc::lstm_step_kernel<tc::LSTM_HEAD_MEAN>, attr_mask, dev, sizeof(tc::LstmSmem))) return RDV_ERR_CUDA;
     const int64_t pairs = ((n + tc::TM - 1) / tc::TM + tc::LSTM_TILES - 1) / tc::LSTM_TILES;
     const unsigned grid = (unsigned)(pairs < sm_count ? pairs : sm_count);
-    tc::lstm_step_kernel<<<grid, tc::LSTM_THREADS, sizeof(tc::LstmSmem), (cudaStream_t)cuda_stream>>>(
-        *pi, obs, episode_start, h_in, c_in, h_out, c_out, actions, n, ld);
+    tc::lstm_step_kernel<tc::LSTM_HEAD_MEAN><<<grid, tc::LSTM_THREADS, sizeof(tc::LstmSmem), (cudaStream_t)cuda_stream>>>(
+        *pi, obs, episode_start, h_in, c_in, h_out, c_out, actions, n, ld, {});
+    return launch_status();
+}
+
+int rdv_lstm_actor_critic_step(const RdvLstmActorCritic *w, const RdvLstmStepIO *io, int64_t n, void *cuda_stream)
+{
+    if (!w || !io) return RDV_ERR_NULL;
+    const RdvLstmPolicy &a = w->actor, &v = w->critic;
+    const float *wp[] = {w->log_std,
+                         a.weight_ih, a.weight_hh, a.bias_ih, a.bias_hh, a.w0, a.b0, a.w1, a.b1, a.w2, a.b2,
+                         v.weight_ih, v.weight_hh, v.bias_ih, v.bias_hh, v.w0, v.b0, v.w1, v.b1, v.w2, v.b2};
+    for (const float *p : wp)
+        if (!p) return RDV_ERR_NULL;
+    const void *f[] = {io->obs, io->h_pi, io->c_pi, io->h_pi_out, io->c_pi_out, io->h_vf, io->c_vf, io->h_vf_out,
+                       io->c_vf_out, io->actions, io->log_prob, io->values};
+    for (const void *p : f)
+        if (!p) return RDV_ERR_NULL;
+    if (n < 0 || io->ld < n) return RDV_ERR_SIZE;
+    for (const void *p : f)
+        if ((uintptr_t)p & 3) return RDV_ERR_ALIGN;
+    if ((uintptr_t)io->env_actions & 3) return RDV_ERR_ALIGN;
+    for (const float *p : wp)
+        if ((uintptr_t)p & 3) return RDV_ERR_ALIGN;
+    if (w->actor.hidden != tc::LH || w->critic.hidden != tc::LH) return RDV_ERR_UNSUPPORTED;
+    if (n == 0) return RDV_OK;
+    int sm_count = 0;
+    const int dev = current_device(&sm_count);
+    if (dev < 0) return RDV_ERR_CUDA;
+    constexpr int AC = tc::LSTM_HEAD_ACTOR_CRITIC;
+    static std::atomic<uint64_t> attr_mask{0};
+    if (!ensure_smem(tc::lstm_step_kernel<AC>, attr_mask, dev, sizeof(tc::LstmSmem))) return RDV_ERR_CUDA;
+    // one CTA per SM (shared memory, TMEM): half of the SMs for each network
+    const int64_t pairs = ((n + tc::TM - 1) / tc::TM + tc::LSTM_TILES - 1) / tc::LSTM_TILES;
+    const int64_t per_net = sm_count / 2 > 1 ? sm_count / 2 : 1;
+    const int64_t half = pairs < per_net ? pairs : per_net;
+    const tc::LstmExtra<AC> x{w->critic, io->h_vf, io->c_vf, io->h_vf_out, io->c_vf_out, io->env_actions, io->log_prob,
+                              io->values, w->log_std, io->action_seed, io->step_index, io->env_offset, half};
+    tc::lstm_step_kernel<AC><<<(unsigned)(2 * half), tc::LSTM_THREADS, sizeof(tc::LstmSmem), (cudaStream_t)cuda_stream>>>(
+        w->actor, io->obs, io->episode_start, io->h_pi, io->c_pi, io->h_pi_out, io->c_pi_out, io->actions, n, io->ld, x);
     return launch_status();
 }
 

@@ -1,6 +1,8 @@
-// rdv_lstm.cuh -- one deterministic step of the actor of sb3_contrib's RecurrentPPO "MlpLstmPolicy" (main_rnn.py:
-// one 256-wide LSTM layer, then the default pi = [64, 64] Tanh head) on the 5th-generation tensor cores, built from the
-// primitives of rdv_policy_tc.cuh (UMMA descriptors, TS/SS MMAs, TMEM loads/stores, mbarriers, fp16 hi/lo split).
+// rdv_lstm.cuh -- one step of sb3_contrib's RecurrentPPO "MlpLstmPolicy" (main_rnn.py: one 256-wide LSTM layer, then
+// the default [64, 64] Tanh heads) on the 5th-generation tensor cores, built from the primitives of rdv_policy_tc.cuh
+// (UMMA descriptors, TS/SS MMAs, TMEM loads/stores, mbarriers, fp16 hi/lo split).  One kernel body, templated on what
+// follows the LSTM (LstmHead): the deterministic actor (rdv_lstm_policy_step), or the collection step's actor with
+// the sampled Gaussian head and critic with the value head in one grid (rdv_lstm_actor_critic_step).
 //
 // A CTA of 256 threads holds TWO tiles of 128 envs (one group per tile, thread = env = TMEM lane, UMMA M = 128):
 //
@@ -132,9 +134,38 @@ __device__ __forceinline__ void cta_sync_for_mma()
     tc_fence_after();
 }
 
+// What the step does after the LSTM: LSTM_HEAD_MEAN is the deterministic clipped actor of rdv_lstm_policy_step;
+// LSTM_HEAD_ACTOR_CRITIC is the collection step of rdv_lstm_actor_critic_step, where CTAs [0, half) run the actor's
+// tile pairs with the sampled Gaussian head and CTAs [half, 2 half) the critic's (LstmCritic) with the value head.
+enum LstmHead { LSTM_HEAD_MEAN = 0, LSTM_HEAD_ACTOR_CRITIC = 1 };
+
+template <int HEAD> struct LstmExtra {};
+template <> struct LstmExtra<LSTM_HEAD_ACTOR_CRITIC> {
+    RdvLstmPolicy critic;                                // its w2, b2: value_net [1][64], [1]
+    const float *h_in, *c_in;                            // the critic's state in / out
+    float *h_out, *c_out;
+    float *env_actions, *log_prob, *values;              // env_actions nullable
+    const float *log_std;
+    uint64_t seed;                                       // noise of env i: philox_normals(seed; env_offset + i, step)
+    int64_t step_index, env_offset, half;
+};
+
+// W1 and W2 (ROWS outputs) of the head into the weight stage
+template <int ROWS>
+__device__ __forceinline__ void stage_head_w12(const RdvLstmPolicy &pi, LstmSmem &s, int t)
+{
+    WeightTile<LSTM_THREADS, H, H, H, H> w1;
+    WeightTile<LSTM_THREADS, ROWS, H, N3, H> w2;
+    w1.fetch(pi.w1, nullptr, t);
+    w2.fetch(pi.w2, nullptr, t);
+    w1.store(LSTM_WSCALE, s.wh, s.wl, t);
+    w2.store(LSTM_WSCALE, s.wh + H * H, s.wl + H * H, t);
+}
+
+template <int HEAD>
 __global__ void __launch_bounds__(LSTM_THREADS, 1)
-lstm_step_kernel(const RdvLstmPolicy pi, const float *obs, const uint8_t *start, const float *h_in, const float *c_in,
-                 float *h_out, float *c_out, float *actions, int64_t n, int64_t ld)
+lstm_step_kernel(RdvLstmPolicy pi, const float *obs, const uint8_t *start, const float *h_in, const float *c_in,
+                 float *h_out, float *c_out, float *actions, int64_t n, int64_t ld, const LstmExtra<HEAD> x)
 {
     extern __shared__ __align__(128) unsigned char raw[];
     LstmSmem &s = *reinterpret_cast<LstmSmem *>(raw);
@@ -146,8 +177,22 @@ lstm_step_kernel(const RdvLstmPolicy pi, const float *obs, const uint8_t *start,
     uint64_t *bar = &s.mma_bar[g];
     uint32_t phase = 0;
     const int64_t tiles = (n + TM - 1) / TM, pairs = (tiles + LSTM_TILES - 1) / LSTM_TILES;
+    unsigned first = blockIdx.x, stride = gridDim.x;
+    bool critic = false;
+    if constexpr (HEAD == LSTM_HEAD_ACTOR_CRITIC) {
+        stride = (unsigned)x.half;
+        critic = blockIdx.x >= stride;
+        if (critic) {
+            first -= stride;
+            pi = x.critic;
+            h_in = x.h_in;
+            c_in = x.c_in;
+            h_out = x.h_out;
+            c_out = x.c_out;
+        }
+    }
 
-    for (int64_t pair = blockIdx.x; pair < pairs; pair += gridDim.x) {
+    for (int64_t pair = first; pair < pairs; pair += stride) {
         const int64_t env = (pair * LSTM_TILES + g) * TM + r;
         const bool valid = env < n;
         const bool keep = valid && !(start && start[env]);                  // else h = c = 0 (episode start)
@@ -213,7 +258,7 @@ lstm_step_kernel(const RdvLstmPolicy pi, const float *obs, const uint8_t *start,
                 s.b0[t] = __ldg(pi.b0 + t);
                 s.b1[t] = __ldg(pi.b1 + t);
             }
-            if (t < N3) s.b2[t] = t < RDV_ACT_DIM ? __ldg(pi.b2 + t) : 0.0f;
+            if (t < N3) s.b2[t] = t < (critic ? 1 : RDV_ACT_DIM) ? __ldg(pi.b2 + t) : 0.0f;
             w0.store(LSTM_WSCALE, s.wh, s.wl, t);
             float v[32];
 #pragma unroll 1
@@ -231,14 +276,10 @@ lstm_step_kernel(const RdvLstmPolicy pi, const float *obs, const uint8_t *start,
         tc_fence_after();
         lstm_head_epilogue(lane_addr, s.b0, al, r);
         cta_sync_for_mma();                                  // both groups are past their W0 MMAs
-        {
-            WeightTile<LSTM_THREADS, H, H, H, H> w1;
-            WeightTile<LSTM_THREADS, RDV_ACT_DIM, H, N3, H> w2;
-            w1.fetch(pi.w1, nullptr, t);
-            w2.fetch(pi.w2, nullptr, t);
-            w1.store(LSTM_WSCALE, s.wh, s.wl, t);
-            w2.store(LSTM_WSCALE, s.wh + H * H, s.wl + H * H, t);
-        }
+        if (critic)
+            stage_head_w12<1>(pi, s, t);
+        else
+            stage_head_w12<RDV_ACT_DIM>(pi, s, t);
         cta_sync_for_mma();
         if (r == 0) issue_layer(tmem + A_COL, al, tmem, s.wh, s.wl, H, H / KSTEP, bar);
         mbar_wait(bar, phase);
@@ -259,10 +300,28 @@ lstm_step_kernel(const RdvLstmPolicy pi, const float *obs, const uint8_t *start,
             uint32_t v[16];
             tmem_ld16_issue(lane_addr, v);
             tmem_ld_wait(v);
-            if (valid) {
+            if constexpr (HEAD == LSTM_HEAD_MEAN) {
+                if (valid) {
 #pragma unroll
-                for (int j = 0; j < RDV_ACT_DIM; ++j)
-                    actions[env * RDV_ACT_DIM + j] = fminf(1.0f, fmaxf(-1.0f, fmaf(__uint_as_float(v[j]), LSTM_WUNSCALE, s.b2[j])));
+                    for (int j = 0; j < RDV_ACT_DIM; ++j)
+                        actions[env * RDV_ACT_DIM + j] =
+                            fminf(1.0f, fmaxf(-1.0f, fmaf(__uint_as_float(v[j]), LSTM_WUNSCALE, s.b2[j])));
+                }
+            } else if (valid && critic) {
+                x.values[env] = fmaf(__uint_as_float(v[0]), LSTM_WUNSCALE, s.b2[0]);
+            } else if (valid) {                              // a ~ N(mean, exp(log_std)^2), as the fused rollout draws
+                float z[RDV_ACT_DIM];
+                philox_normals(x.seed, x.env_offset + env, x.step_index, z);
+                float lp = 0.0f;
+#pragma unroll
+                for (int j = 0; j < RDV_ACT_DIM; ++j) {
+                    const float ls = __ldg(x.log_std + j);
+                    const float a = fmaf(expf(ls), z[j], fmaf(__uint_as_float(v[j]), LSTM_WUNSCALE, s.b2[j]));
+                    actions[env * RDV_ACT_DIM + j] = a;
+                    if (x.env_actions) x.env_actions[env * RDV_ACT_DIM + j] = fminf(1.0f, fmaxf(-1.0f, a));
+                    lp += fmaf(-0.5f * z[j], z[j], -ls);
+                }
+                x.log_prob[env] = lp - 5.51363120f;         // 3 ln(2 pi)
             }
         }
         // the next pair restages the weights, biases and this group's A
