@@ -343,8 +343,12 @@ typedef struct RdvLstmPolicy {
  * obs [n][17], actions [n][6] float32; h_in, c_in, h_out, c_out float32 [H][ld] (structure of arrays like RdvState,
  * element (j, i) at [j * ld + i]); episode_start nullable [n] (NULL: no env starts an episode).  The outputs are
  * separate buffers from the inputs.  Every product runs on the tensor cores as three MMAs of fp16 halves with fp32
- * accumulation (fp32-level accuracy); the weights are staged times 2^10, so every weight and bias must be below 64 in
- * magnitude (not checked here).  Only H = 256 with the 64-64 head is supported (RDV_ERR_UNSUPPORTED). */
+ * accumulation (fp32-level accuracy); the weights are staged times 2^10, so every weight and bias must be below
+ * 65520 / 1024 = 63.984375 in magnitude (not checked here: from there on fp16 rounds the staged hi half to infinity and
+ * what depends on that weight is NaN for every env).  Each observation component is clamped to [-60000, 60000] before
+ * its split, and a NaN one is taken as -60000.  A NaN or infinite h of an env that does not start an episode makes its
+ * h' and c' NaN and its actions -1 (the clip takes NaN to -1); an infinite c gives an infinite c' in that unit, as the
+ * formula does.  Only H = 256 with the 64-64 head is supported (RDV_ERR_UNSUPPORTED). */
 int rdv_lstm_policy_step(const RdvLstmPolicy *pi, const float *obs, const uint8_t *episode_start,
                          const float *h_in, const float *c_in, float *h_out, float *c_out, float *actions,
                          int64_t n, int64_t ld, void *cuda_stream);
@@ -381,7 +385,9 @@ typedef struct RdvLstmStepIO {
  * unclipped; z = the six N(0,1) draws of (action_seed; env_offset + i, step_index) -- the stream and counter layout of
  * RDV_ACTIONS_POLICY_SAMPLE --; actions = mean + exp(log_std) z, env_actions = clip(actions, -1, 1),
  * log_prob = sum_j (-z_j^2 / 2 - log_std_j) - 3 ln(2 pi).  Critic: values = value_net(tanh(W1 tanh(W0 h_vf'))), no
- * clip.  The same precision and weight limit (below 64 in magnitude, not checked here) as rdv_lstm_policy_step.
+ * clip.  The same precision, weight limit (below 63.984375 in magnitude, not checked here), observation clamp (a NaN
+ * component taken as -60000) and handling of a non-finite state as rdv_lstm_policy_step, per network: a NaN or
+ * infinite h_pi gives NaN actions and env_actions of -1, a NaN or infinite h_vf a NaN value.
  * Returns RDV_ERR_NULL / SIZE (n < 0, ld < n) / ALIGN (a float pointer not 4-byte aligned) / UNSUPPORTED (hidden of
  * either network != 256); allocates nothing. */
 int rdv_lstm_actor_critic_step(const RdvLstmActorCritic *w, const RdvLstmStepIO *io, int64_t n, void *cuda_stream);

@@ -116,6 +116,9 @@ class RdvLstmPolicy(C.Structure):
 
 
 LSTM_HIDDEN = 256               # the only LSTM width rdv_lstm_policy_step supports
+# Every weight and bias of an LSTM network must be below this in magnitude: the kernels stage the weights times 2^10 in
+# fp16 hi / lo halves, and fp16 rounds 65520 (its largest finite value 65504 plus half an ulp) and above to infinity.
+LSTM_WEIGHT_LIMIT = 65520.0 / 1024.0
 
 
 class RdvLstmActorCritic(C.Structure):

@@ -37,7 +37,8 @@ constexpr int GN = 4 * HU;                              // gate rows per chunk (
 constexpr int KA = K0 + LH;                             // [obs | 1 | pad] + h = 288
 // Every weight is staged times 2^10 (exact) and D is scaled back by 2^-10 in fp32: the lo half of a weight of magnitude
 // |w| then stays a normal fp16 number down to |w| = 2.4e-4 instead of 0.25 (below that fp16 rounds it to 2^-24 in
-// absolute terms, which for |w| ~ 0.05 costs ~20x the precision of the fp32 weight).  hi must stay finite: |w| < 64.
+// absolute terms, which for |w| ~ 0.05 costs ~20x the precision of the fp32 weight).  hi must stay finite: fp16 rounds
+// 65520 up to infinity, so |w| < 65520 / 1024 = 63.984375 (LSTM_WEIGHT_LIMIT of _native.py).
 constexpr float LSTM_WSCALE = 1024.0f, LSTM_WUNSCALE = 1.0f / 1024.0f;
 static_assert(LSTM_TILES * LSTM_TILE_COLS <= TMEM_COLS, "TMEM budget");
 static_assert(A_COL + KA / 2 <= LSTM_TILE_COLS, "A hi must fit the group's TMEM columns");

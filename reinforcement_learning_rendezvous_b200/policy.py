@@ -142,9 +142,9 @@ class LstmPolicy:
             if tuple(np.shape(state_dict[name])) != shapes[k]:
                 raise ValueError(f"{name} has shape {tuple(np.shape(state_dict[name]))}, expected {shapes[k]} "
                                  f"(LSTM of {hid} units, 64-64 head)")
-            if not np.all(np.abs(state_dict[name]) < 64):
-                raise ValueError(f"{name} has entries of magnitude >= 64 or non-finite ones; the kernel stages the "
-                                 "weights times 2^10 in fp16 halves")
+            if not np.all(np.abs(state_dict[name]) < N.LSTM_WEIGHT_LIMIT):
+                raise ValueError(f"{name} has entries of magnitude >= {N.LSTM_WEIGHT_LIMIT} (64 - 1/64) or non-finite "
+                                 "ones; the kernel stages the weights times 2^10 in fp16 halves")
         if not torch.cuda.is_available():
             raise RuntimeError("LstmPolicy needs a CUDA device; there is no CPU fallback")
         self.device = torch.device(device)

@@ -34,8 +34,6 @@ from .batched_env import BatchedRendezvousEnv, _stream_ptr
 from .policy import LstmPolicy
 from .ppo import gae
 
-WEIGHT_LIMIT = 64.0             # the LSTM kernels stage weights times 2^10 in fp16 halves: |w| must stay below 64
-
 
 class _Extractor(nn.Module):
     def __init__(self, hidden, net):
@@ -84,13 +82,14 @@ class RecurrentActorCritic(nn.Module):
         return N.RdvLstmActorCritic(net(*pi), self.log_std.data_ptr(), net(*vf))
 
     def check_weights(self):
-        """Raise unless every parameter the kernel reads is finite and below 64 in magnitude (one device reduction and
-        one read-back)."""
+        """Raise unless every parameter the kernel reads is finite and below ``LSTM_WEIGHT_LIMIT`` in magnitude (one
+        device reduction and one read-back)."""
+        limit = N.LSTM_WEIGHT_LIMIT
         worst = float(torch.stack([p.detach().abs().max() for p in self.parameters()]).max())
-        if not worst < WEIGHT_LIMIT:
-            bad = [k for k, p in self.named_parameters() if not float(p.detach().abs().max()) < WEIGHT_LIMIT]
-            raise ValueError(f"parameters {bad} have entries of magnitude >= {WEIGHT_LIMIT:g} or non-finite ones; the LSTM "
-                             "kernel stages the weights times 2^10 in fp16 halves")
+        if not worst < limit:
+            bad = [k for k, p in self.named_parameters() if not float(p.detach().abs().max()) < limit]
+            raise ValueError(f"parameters {bad} have entries of magnitude >= {limit} (64 - 1/64) or non-finite ones; "
+                             "the LSTM kernel stages the weights times 2^10 in fp16 halves")
 
     @staticmethod
     def _sequence(lstm, obs, h0, c0, start0):

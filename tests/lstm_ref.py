@@ -44,17 +44,26 @@ def _mm_split(a, w, scale=2.0 ** 10):
     return ((al @ wh.T + ah @ wl.T + ah @ wh.T) * np.float32(1.0 / scale)).astype(np.float32)
 
 
+def gates_split_emulation(sd, obs, h, episode_start=None, mm=_mm_split):
+    """The gate pre-activations z [n, 4 * 256] (float32, torch's order i, f, g, o) as rdv_lstm_policy_step computes
+    them: ``mm(a, w)`` the product of a = [obs | h] (h zeroed where episode_start is set) and w = [W_ih | W_hh], then
+    b_ih + b_hh added in float32.  ``mm`` defaults to the kernel's three-product split (tests pass altered ones)."""
+    w = {k: np.asarray(v, dtype=np.float32) for k, v in sd.items()}
+    h = np.asarray(h, np.float32)
+    if episode_start is not None:
+        h = np.where(~np.asarray(episode_start, dtype=bool).reshape(-1, 1), h, 0).astype(np.float32)
+    a = np.concatenate([np.asarray(obs, np.float32), h], axis=1)
+    wcat = np.concatenate([w["lstm_actor.weight_ih_l0"], w["lstm_actor.weight_hh_l0"]], axis=1)
+    return mm(a, wcat) + (w["lstm_actor.bias_ih_l0"] + w["lstm_actor.bias_hh_l0"])
+
+
 def lstm_step_split_emulation(sd, obs, h, c, episode_start=None):
     """numpy emulation of rdv_lstm_policy_step's arithmetic (fp16 hi / lo operands, three products, float32
     accumulation and activations; numpy's float32 accumulation order, not the tensor core's), state only: (h', c')."""
-    w = {k: np.asarray(v, dtype=np.float32) for k, v in sd.items()}
-    h, c = np.asarray(h, np.float32), np.asarray(c, np.float32)
+    c = np.asarray(c, np.float32)
     if episode_start is not None:
-        keep = ~np.asarray(episode_start, dtype=bool).reshape(-1, 1)
-        h, c = np.where(keep, h, 0).astype(np.float32), np.where(keep, c, 0).astype(np.float32)
-    a = np.concatenate([np.asarray(obs, np.float32), h], axis=1)
-    wcat = np.concatenate([w["lstm_actor.weight_ih_l0"], w["lstm_actor.weight_hh_l0"]], axis=1)
-    z = _mm_split(a, wcat) + (w["lstm_actor.bias_ih_l0"] + w["lstm_actor.bias_hh_l0"])
+        c = np.where(~np.asarray(episode_start, dtype=bool).reshape(-1, 1), c, 0).astype(np.float32)
+    z = gates_split_emulation(sd, obs, h, episode_start)
     zi, zf, zg, zo = np.split(z, 4, axis=1)
     sig = lambda x: np.float32(1) / (np.float32(1) + np.exp(-x))
     c2 = (sig(zf) * c + sig(zi) * np.tanh(zg)).astype(np.float32)
@@ -105,6 +114,22 @@ def make_state_dict(kind="torch", seed=0, critic=True):
     if critic:
         sd["log_std"] = np.zeros(ACT)
     return {k: np.asarray(v, dtype=np.float32) for k, v in sd.items()}
+
+
+def scale_state_dict(sd, s_lstm, s_head):
+    """sd with every LSTM weight and bias (actor and critic) times s_lstm and every head weight and bias times s_head
+    (float32).  A factor "max" is the largest that keeps that part's largest magnitude at 0.999 of the loaders' limit
+    (``_native.LSTM_WEIGHT_LIMIT``)."""
+    from reinforcement_learning_rendezvous_b200._native import LSTM_WEIGHT_LIMIT
+    out = dict(sd)
+    parts = (("lstm_",), ("mlp_extractor.", "action_net.", "value_net."))
+    for s, prefixes in zip((s_lstm, s_head), parts):
+        keys = [k for k in sd if k.startswith(prefixes)]
+        if s == "max":
+            s = 0.999 * LSTM_WEIGHT_LIMIT / max(float(np.abs(sd[k]).max()) for k in keys)
+        for k in keys:
+            out[k] = (np.asarray(sd[k], dtype=np.float64) * s).astype(np.float32)
+    return out
 
 
 def actor_keys(sd):

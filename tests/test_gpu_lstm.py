@@ -81,7 +81,7 @@ def test_step_matches_fp64_reference(kind):
     print(f"{kind}: kernel |da| {err[0]:.2e} |dh| {err[1]:.2e} |dc|rel {err[2]:.2e};  "
           f"torch fp32 {t32[0]:.2e} {t32[1]:.2e} {t32[2]:.2e}")
     assert max(err) <= 1e-5, err
-    for n in (1, 127, 129, 1000):
+    for n in (1, 127, 129, 1000, NMAX - 77):             # NMAX - 77: CTAs loop over pairs, the last one ragged
         part = _run(pol, obs[:n], h[:n], c[:n], start[:n])
         for a, b in zip(part, full):
             assert np.array_equal(a, b[:n]), n
@@ -135,6 +135,8 @@ def test_episode_start_and_predict_contract():
     obs = _observations(n, rng)
     garbage_h = rng.uniform(-1e30, 1e30, (n, H)).astype(np.float32)
     garbage_c = rng.uniform(-1e30, 1e30, (n, H)).astype(np.float32)
+    for g in (garbage_h, garbage_c):                      # non-finite garbage too: the select clears it, 0 * x would not
+        g[0::3, 0::5], g[1::3, 1::7], g[2::3, 2::11] = np.nan, np.inf, -np.inf
     zeros = np.zeros((n, H), np.float32)
     fresh = _run(pol, obs, zeros, zeros)
     reset = _run(pol, obs, garbage_h, garbage_c, np.ones(n, dtype=bool))

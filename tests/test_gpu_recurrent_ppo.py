@@ -33,12 +33,14 @@ def _module(sd):
     return m
 
 
-def _step(m, obs, start, states, seed=SEED, step=STEP, offset=OFFSET, env_actions=True):
-    """One launch on device inputs; states: four [256, n] tensors.  Returns the outputs as device tensors."""
+def _step(m, obs, start, states, seed=SEED, step=STEP, offset=OFFSET, env_actions=True, ld=None):
+    """One launch on device inputs; states: four [256, n] tensors with leading dimension ld (default n), the output
+    states column slices of NaN-filled [256, ld] buffers.  Returns the outputs as device tensors."""
     from reinforcement_learning_rendezvous_b200 import _native as N
     from reinforcement_learning_rendezvous_b200.batched_env import _stream_ptr
     n, dev = obs.shape[0], obs.device
-    out = dict(states=[torch.full((H, n), np.nan, device=dev) for _ in range(4)],
+    ld = n if ld is None else ld
+    out = dict(states=[torch.full((H, ld), np.nan, device=dev)[:, :n] for _ in range(4)],
                actions=torch.full((n, 6), np.nan, device=dev), env_actions=torch.full((n, 6), np.nan, device=dev),
                log_prob=torch.full((n,), np.nan, device=dev), values=torch.full((n,), np.nan, device=dev))
     w = m.kernel_weights()
@@ -46,7 +48,7 @@ def _step(m, obs, start, states, seed=SEED, step=STEP, offset=OFFSET, env_action
     io = N.RdvLstmStepIO(obs.data_ptr(), start.data_ptr(), s[0].data_ptr(), s[1].data_ptr(), o[0].data_ptr(),
                          o[1].data_ptr(), s[2].data_ptr(), s[3].data_ptr(), o[2].data_ptr(), o[3].data_ptr(),
                          out["actions"].data_ptr(), out["env_actions"].data_ptr() if env_actions else None,
-                         out["log_prob"].data_ptr(), out["values"].data_ptr(), seed, step, offset, n)
+                         out["log_prob"].data_ptr(), out["values"].data_ptr(), seed, step, offset, ld)
     N.check(N.lib().rdv_lstm_actor_critic_step(C.byref(w), C.byref(io), n, _stream_ptr(dev)), "step")
     return out
 
@@ -80,7 +82,9 @@ def _assert_against_ref(got, ref, sd, z, r, what):
 @pytest.mark.parametrize("kind", KINDS)
 def test_actor_critic_step_matches_fp64(kind):
     """One step at n = 65536 from random states with 5 % episode starts against fp64; the actor's state bit-identical
-    to rdv_lstm_policy_step; every env independent of n (1, 127, 129, 1000) and of its position in the batch."""
+    to rdv_lstm_policy_step; every env independent of n (1, 127, 129, 1000, and 65459, where CTAs loop over several
+    tile pairs and the last pair is ragged), of its position in the batch and of the state buffers' leading
+    dimension."""
     from reinforcement_learning_rendezvous_b200 import LstmPolicy
     rng = np.random.default_rng(20)
     sd = make_state_dict(kind, seed=3)
@@ -106,10 +110,20 @@ def test_actor_critic_step_matches_fp64(kind):
     _, h1, c1 = pol.forward(obs_d, st_d[0], st_d[1], start_d)
     assert np.array_equal(h1.t().cpu().numpy(), full["h_pi"]) and np.array_equal(c1.t().cpu().numpy(), full["c_pi"])
     # independent of n and of the position: a prefix, and a slice run with its global env offset
-    for n in (1, 127, 129, 1000):
+    for n in (1, 127, 129, 1000, NMAX - 77):
         part = _np(_step(m, obs_d[:n], start_d[:n], [x[:, :n].contiguous() for x in st_d]))
         for k, v in part.items():
             assert np.array_equal(v, full[k][:n]), (n, k)
+    # column slices of wider buffers (ld > n), NaN past column n: the same bits, nothing written past column n
+    n, ld = 1000, 1333
+    wide = [torch.full((H, ld), np.nan, device=dev) for _ in range(4)]
+    for w_, x in zip(wide, st_d):
+        w_[:, :n] = x[:, :n]
+    out = _step(m, obs_d[:n], start_d[:n], [w_[:, :n] for w_ in wide], ld=ld)
+    for k, v in _np(out).items():
+        assert np.array_equal(v, full[k][:n]), ("ld", k)
+    for o in out["states"]:
+        assert o.stride(0) == ld and bool(o.as_strided((H, ld), (ld, 1))[:, n:].isnan().all())
     lo, n = 3000, 1000
     part = _np(_step(m, obs_d[lo:lo + n], start_d[lo:lo + n], [x[:, lo:lo + n].contiguous() for x in st_d],
                      offset=OFFSET + lo))

@@ -90,6 +90,27 @@ def test_loader_rejects_other_shapes():
         LstmPolicy(missing)
 
 
+def test_loader_weight_limit():
+    """|w| < 65520 / 1024 = 63.984375: the largest float32 below it passes, from it on (where the fp16 hi half of the
+    weight staged times 2^10 rounds to infinity) and non-finite values are rejected -- in every tensor the kernel reads."""
+    assert N.LSTM_WEIGHT_LIMIT == 63.984375
+    largest = np.nextafter(np.float32(N.LSTM_WEIGHT_LIMIT), np.float32(0))
+    sd = make_state_dict("torch", seed=5, critic=False)
+    for name in ("lstm_actor.weight_ih_l0", "lstm_actor.weight_hh_l0", "lstm_actor.bias_hh_l0",
+                 "mlp_extractor.policy_net.2.weight", "action_net.weight"):
+        ok = dict(sd)
+        ok[name] = sd[name].copy()
+        ok[name].flat[3] = largest
+        ok[name].flat[-1] = -largest
+        _construct(ok)
+        for bad in (N.LSTM_WEIGHT_LIMIT, -N.LSTM_WEIGHT_LIMIT, 64.0, np.inf, -np.inf, np.nan):
+            wrong = dict(sd)
+            wrong[name] = sd[name].copy()
+            wrong[name].flat[3] = bad
+            with pytest.raises(ValueError, match="63.984375"):
+                LstmPolicy(wrong)
+
+
 @pytest.fixture(scope="module")
 def lib():
     N.build()

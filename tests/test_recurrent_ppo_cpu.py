@@ -9,6 +9,7 @@ import torch
 from lstm_ref import H, make_state_dict
 from recurrent_ref import process_sequence_loop
 
+from reinforcement_learning_rendezvous_b200 import _native as N
 from reinforcement_learning_rendezvous_b200.recurrent_ppo import (RecurrentActorCritic, RecurrentPPO,
                                                                   RecurrentPPOConfig, plan_minibatches)
 
@@ -125,6 +126,28 @@ def test_module_layout_init_and_defaults():
     assert (c.learning_rate, c.n_steps, c.batch_size, c.n_epochs, c.clip_range, c.gamma, c.gae_lambda, c.ent_coef,
             c.vf_coef, c.max_grad_norm, c.normalize_advantage) == (3e-4, 128, 128, 10, 0.2, 0.99, 0.95, 0.0, 0.5, 0.5,
                                                                    True)
+
+
+def test_check_weights_limit():
+    """The collection step's weight check: the largest float32 below 65520 / 1024 passes, the limit itself, 64 and
+    non-finite values raise, in the actor's and the critic's tensors alike."""
+    assert N.LSTM_WEIGHT_LIMIT == 63.984375
+    largest = float(np.nextafter(np.float32(N.LSTM_WEIGHT_LIMIT), np.float32(0)))
+    m = RecurrentActorCritic()
+    for p in (m.lstm_actor.weight_hh_l0, m.lstm_critic.weight_ih_l0, m.mlp_extractor.value_net[0].weight,
+              m.action_net.weight):
+        keep = p.detach().clone()
+        with torch.no_grad():
+            p[0, 1], p[-1, -1] = largest, -largest
+        m.check_weights()
+        for bad in (N.LSTM_WEIGHT_LIMIT, -N.LSTM_WEIGHT_LIMIT, 64.0, float("inf"), float("nan")):
+            with torch.no_grad():
+                p[0, 1] = bad
+            with pytest.raises(ValueError, match="63.984375"):
+                m.check_weights()
+        with torch.no_grad():
+            p.copy_(keep)
+    m.check_weights()
 
 
 def test_rejects_anything_but_a_batched_env():
